@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus 1 --steps K --warmup W       # the reference's CPU implementation of the path
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W                        # data parallel, one rank per GPU (weak scaling)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR     # + what the last timed step computed, as DIR/*.npy
 
 Workloads (`--workload`, BASELINE.json configs):
   c2-dense128 (default)  configs[1]: toyotagraph-shaped world (60 000 POIs, 300 categories, 995 users), hidden 128 (+64), 8 heads,
@@ -26,6 +27,11 @@ One training step = forward + loss + backward + (NCCL all-reduce) + AdamW over o
 value  = units/s with the inputs already resident in HBM;
 e2e    = units/s through the public API from HOST buffers: raw items -> collator (pack, H2D, K1 APSP + path edges on
          the GPU) -> training step -> loss read back, every step.
+
+--dump-outputs DIR writes, after the timed steps of `value`, what the last of them computed (rank 0): for a training workload
+the loss, and every parameter after the optimizer step and its gradient (`loss.npy`, `param.<name>.npy`, `grad.<name>.npy`);
+for c5-eval the head's top-k values / ids, target ranks and target logits; for c3-preprocess K1's outputs of the last batch of
+graphs.  The inputs are seeded, so two builds run with the same arguments can be compared array for array (see dump_outputs).
 """
 import argparse
 import json
@@ -41,6 +47,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the source tree: without this, importing the package modules that build() did not import
+# (trainer, model, ops, ...) would add their .pyc files under mobgt_b200/__pycache__/
+sys.dont_write_bytecode = True
 
 HP = dict(n_layers=6, num_heads=8, hidden_dim=128, dropout_rate=0.1, intput_dropout_rate=0.1, weight_decay=0.01, ffn_dim=1024,
           warmup_updates=40000, tot_updates=400000, peak_lr=2e-4, end_lr=1e-9, edge_type="multi_hop", multi_hop_max_dist=20,
@@ -54,6 +63,31 @@ def emit(line):
     out = _REAL_STDOUT if _REAL_STDOUT is not None else sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
+
+
+DUMP_SAMPLE = 1 << 15            # values kept per dumped array: at most 256 KB each, a few tens of MB for a whole model
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array of `arrays` (name -> tensor / ndarray; None is skipped) as out_dir/<name>.npy: floating point as
+    float32 (float64 stays float64), integers as float64 (exact).  An array of more than DUMP_SAMPLE values is replaced by the
+    values at DUMP_SAMPLE fixed positions of its flattened form (sorted, drawn with seed 0 from its size alone), so the files of
+    two runs line up value for value."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        if a is None:
+            continue
+        a = (a.detach() if torch.is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a))).reshape(-1)
+        if a.numel() > DUMP_SAMPLE:        # sampled where the array lives: only DUMP_SAMPLE values are converted and copied
+            pos = np.sort(np.random.default_rng(0).choice(a.numel(), DUMP_SAMPLE, replace=False))
+            a = a[torch.from_numpy(pos).to(a.device)]
+        a = (a.float() if a.is_floating_point() and a.dtype != torch.float64 else a.double()).cpu().numpy()
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise RuntimeError(f"--dump-outputs: more than {DUMP_LIMIT >> 20} MB at {name}")
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -463,13 +497,18 @@ def run_ours(args):
     def resident_step():
         b = batches[state["i"] % nbatches]
         state["i"] += 1
-        return tr.train_step(b)
+        state["loss"] = tr.train_step(b)
 
     for _ in range(max(args.warmup, 2 * nbatches)):       # every distinct shape is seen twice: repeated shapes get captured
         resident_step()
     n0, g0 = _C.launch_count(), tr.graph_steps
     sampler = ClockSampler(local) if rank == 0 else None
     ms = _timed(resident_step, args.steps, dev, world_size)
+    if args.dump_outputs and rank == 0:        # now: the next step (a graph replay) overwrites the loss, the gradients, the weights
+        outs = {"loss": state["loss"]}
+        for name, p in model.named_parameters():
+            outs["param." + name], outs["grad." + name] = p, p.grad
+        dump_outputs(args.dump_outputs, outs)
     replays_value = tr.graph_steps - g0
     launches = (_C.launch_count() - n0) / args.steps + tr.graph_launches * replays_value / args.steps
     tokens = int(np.mean([int(b.tok_pos.numel()) for b in batches]))
@@ -527,7 +566,7 @@ def run_ours(args):
         chunk_ms.append(cur)
     if rank == 0:
         print("[bench] e2e warm-up chunks (ms/step): " + " ".join(f"{x:.2f}" for x in chunk_ms), file=sys.stderr)
-    e2e_steps = max(4, args.steps)
+    e2e_steps = args.steps
     eg0, ee0 = tr.graph_steps, tr.eager_steps
     ms_e2e = _timed(e2e_step, e2e_steps, dev, world_size, finalize=e2e_flush)
     clocks = sampler.stop() if sampler else None
@@ -598,6 +637,8 @@ def run_c5(args):
     n0 = _C.launch_count()
     sampler = ClockSampler(local) if rank == 0 else None
     ms = _timed(step, args.steps, dev, world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res["r"])
     launches = (_C.launch_count() - n0) / args.steps
     # e2e: z rows and targets start in pinned HOST memory; top-k ids and ranks are read back to the host every step
     zh, th = z.cpu().pin_memory(), target.cpu().pin_memory()
@@ -729,6 +770,8 @@ def run_c3(args):
     n0 = _C.launch_count()
     sampler = ClockSampler(local) if rank == 0 else None
     ms = _timed(step_resident, args.steps, dev, world_size)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, keep["o"])
     launches = (_C.launch_count() - n0) / args.steps
     step_e2e()
     ms_e2e = _timed(step_e2e, args.steps, dev, world_size, finalize=torch.cuda.synchronize)
@@ -818,7 +861,13 @@ def main():
     ap.add_argument("--no-cuda-graph", dest="cuda_graph", action="store_false", help="run every step eagerly")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernel-report", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(3, args.warmup)
     # stdout carries exactly ONE JSON line: everything libraries print to fd 1 meanwhile (the NCCL version banner, ...) goes to
     # stderr; the line is written to the saved descriptor at the end

@@ -7,7 +7,9 @@
  *
  * Pinned against the really-compiled reference (oracle/_ref, built by
  * oracle/build_ref.py from algos.pyx unmodified) on the KATs in
- * tests/golden/ and on random graphs in tests/test_oracle_algos.py.
+ * tests/golden/, and on seeded random and node-510 hub graphs in
+ * tests/test_oracle_algos.py: there against oracle/_ref when it is built,
+ * else against a Python restatement of algos.pyx pinned to those KATs.
  */
 #include <stdint.h>
 #include <stdlib.h>

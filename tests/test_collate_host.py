@@ -53,12 +53,12 @@ def test_worker_stream_shards_batches_in_order():
 
 
 def test_packed_loader_protocol_without_cuda():
-    """PackedLoader's one-batch-ahead protocol (current / advance / iteration, end of stream) with a host-only collate_fn:
-    the side stream is only created when CUDA is available, so this runs on the CPU."""
+    """PackedLoader's one-batch-ahead protocol (current / advance / iteration, end of stream) with a host-only collate_fn and
+    no side stream (a side-stream batch must be an object that carries its ready event), so it runs alike with or without CUDA."""
     from mobgt_b200 import collator
     batches = [[i, i + 1] for i in range(5)]
     seen = []
-    loader = collator.PackedLoader(iter(batches), collate_fn=lambda items: {"items": list(items)}, num_workers=0)
+    loader = collator.PackedLoader(iter(batches), collate_fn=lambda items: {"items": list(items)}, num_workers=0, side_stream=False)
     assert loader.current()["items"] == [0, 1]
     loader.advance()
     assert loader.current()["items"] == [1, 2]

@@ -16,7 +16,6 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 NPZ = os.path.join(HERE, "golden", "gowalla_nevda_real.npz")
-ARCHIVE = "/root/reference/gowalla_nevda.7z"
 
 
 @pytest.fixture(scope="module")
@@ -67,24 +66,60 @@ def test_generate_queue_orders():
     assert q == exp
 
 
-@pytest.mark.skipif(not os.path.exists(ARCHIVE), reason="the reference's archive only exists in the build container")
-def test_adapter_reads_the_reference_files(real, tmp_path):
-    """load_world / load_items on the files of the archive themselves == the committed fixture (itself == the reference)."""
-    import _gowalla
+def test_adapter_reads_files_in_the_reference_format(real, tmp_path):
+    """load_world / load_items on a small data set written in the reference's on-disk format (Graph_*.csv with one header row,
+    {split}.pickle = {user: {session: dict of torch tensors}}, {split}_idx.pkl = {user: [session, ...]}): the world is known by
+    construction, and the items are real trajectories of the committed fixture, read back field for field."""
+    import pickle
+    import torch
     from mobgt_b200 import owndata
-    z, world, splits = real
     raw = tmp_path / "raw"
     raw.mkdir()
-    for name, blob in _gowalla.unpack().items():
-        if name.endswith((".pickle", ".pkl", ".csv")):
-            (raw / name).write_bytes(blob)
+    P, C = 6, 3
+    cat = np.array([2, 1, 3, 1, 2, 3])
+    poi = [(i + 1, 10 * i + 1, 36.0 + 0.25 * i, -115.5 + 0.125 * i, int(cat[i])) for i in range(P)]
+    rng = np.random.default_rng(4)
+    A_d, A_c = (rng.random((P, P)) < 0.4).astype(np.int64), (rng.random((C, C)) < 0.5).astype(np.int64)
+
+    def write_csv(name, rows, header):
+        (raw / name).write_text(header + "\n" + "".join(",".join(str(v) for v in r) + "\n" for r in rows))
+
+    write_csv("Graph_poi.csv", poi, "POI ID,check_freq,latitude,longitude,cat")
+    write_csv("Graph_dist.csv", A_d, ",".join(str(i) for i in range(P)))
+    write_csv("Graph_cat.csv", A_c, ",".join(str(i) for i in range(C)))
     w = owndata.load_world(str(raw), "gowalla_nevda")
-    assert np.array_equal(w.X, world.X) and w.dist_max == world.dist_max and np.array_equal(w.cat_of_poi, world.cat_of_poi)
-    for a, b in zip(w.D_A + w.C_A, world.D_A + world.C_A):
-        assert np.array_equal(a, b)
-    for split in ("train", "test"):
-        items = owndata.load_items(str(raw), split)
-        assert _gowalla.items_digest(items) == str(z[f"ref_digest_{split}"])
+    assert (w.P, w.C, w.U) == (P, C, 1080) and np.array_equal(w.cat_of_poi, cat)
+    assert np.array_equal(w.check_freq, [r[1] for r in poi])
+    assert np.array_equal(w.latlon, np.array([r[2:4] for r in poi], np.float32))
+    assert np.array_equal(w.X[:, 0], [r[1] for r in poi]) and np.array_equal(w.X[np.arange(P), cat], np.ones(P, np.float32))
+    for (crow, col, val), A in ((w.D_A, A_d), (w.C_A, A_c)):
+        n = len(A)
+        dense = np.zeros((n, n), np.float32)
+        dense[np.repeat(np.arange(n), np.diff(crow)), col] = val
+        hat = ((A + np.eye(n)) / (A.sum(1) + 1)[:, None]).astype(np.float32)        # (D + I)^-1 (A + I)
+        assert np.allclose(dense, hat, rtol=1e-6, atol=0)
+
+    _, _, splits = real
+    src = splits["test"][:7]
+    sessions = {}
+    for k, it in enumerate(src):          # two sessions per user, in the order written
+
+        adj = np.zeros((len(it.x), len(it.x)), np.int64)
+        adj[it.edge_index[0], it.edge_index[1]] = it.edge_attr
+        sessions.setdefault(k // 2, {})[k % 2] = dict(
+            node_name=torch.from_numpy(np.asarray(it.x).reshape(-1)), edge_type=torch.from_numpy(adj),
+            target=torch.from_numpy(np.asarray(it.y)), time=torch.from_numpy(np.asarray(it.time).reshape(-1)),
+            time_normal=torch.from_numpy(np.asarray(it.time_normal).reshape(-1)),
+            user=torch.from_numpy(np.asarray(it.user).reshape(-1)), cat=torch.from_numpy(np.asarray(it.cat).reshape(-1)))
+    with open(raw / "test.pickle", "wb") as f:
+        pickle.dump(sessions, f)
+    with open(raw / "test_idx.pkl", "wb") as f:
+        pickle.dump({u: list(s) for u, s in sessions.items()}, f)
+    got = owndata.load_items(str(raw), "test")                 # 'normal' order: users, then sessions, as written
+    assert len(got) == len(src)
+    for a, b in zip(got, src):
+        for name in ("x", "edge_index", "edge_attr", "y", "time", "time_normal", "user", "cat"):
+            assert np.array_equal(np.asarray(getattr(a, name)), np.asarray(getattr(b, name))), name
 
 
 def test_real_batches_pack_and_match_the_oracle_collator(real):

@@ -681,7 +681,7 @@ def test_entry_cli_main_reference_flags(lib_built, tmp_path, capsys):
     assert r3["steps"] == 2 and np.isfinite(r3["loss"])
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (run with gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_entry_two_ranks_report_the_one_rank_metrics(lib_built, tmp_path):
     """`entry --test` under torch.distributed.run with 2 ranks prints the metrics of the WHOLE test set (every rank evaluates its
     share, the metric sums are all-reduced) — the same numbers as the 1-rank run of the same checkpoint; and a 2-rank training
