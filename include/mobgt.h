@@ -110,6 +110,10 @@ int32_t mobgt_poi_pos(const int32_t *x, const int32_t *n, const int64_t *sq_off,
  *   live hop slots and the clamp of the mean (sp = clamp(M, 1, dk), model_fqandtoyo.py:1168-1174); 1 <= dk <= hops.
  *   forward workspace: mobgt_bias_fwd_workspace_bytes() (the E.W table [hops,128,H] and the rel_pos-keyed table RL [512,H]);
  *   backward workspace: mobgt_bias_bwd_workspace_bytes().
+ * Input domain (not checked on the device; K1 writes only values inside it):
+ *   rel_pos in 0..511 (511: unreachable pair); poi_pos in 0..num_bins-1; edge_in bytes in 0..127, bytes [dk, hops) of
+ *   every row 0; E row 0 (edge_encoder's padding row) zero.  Cells with rel_pos - 1 >= rel_pos_max are -inf in the forward.
+ *   The backward never reads a dBias cell outside a graph's live (n[g]+1)^2 square, in row 0, or masked by rel_pos_max.
  * Backward: dBias -> dR [512,H], dPpos [bins,H], dE [128,H], dW [hops*H*H], dtvd [H]  (all overwritten).
  *   dbias_dtype MOBGT_F32:  one f32 [B,H,T,Tp] buffer holding the sum over layers (n_layers = 1);
  *   dbias_dtype MOBGT_BF16: n_layers bf16 [B,H,T,Tp] planes, layer_stride elements apart (mobgt_attn_bwd mode 2),

@@ -518,7 +518,15 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
             const uint32_t ent = lds_u32(s_dlist + (uint32_t)e * 4u);
             const int b = ent & 0xFFF;
             const float d = lds_f32(s_dsum + (uint32_t)h * pitch4 + (uint32_t)b * 4u);
-            if (ent & (1u << 12)) fx_add(dR64 + min(max((int)c.rel_pos[rowp + b], 0), kRelRows - 1) * kH + h, d);
+            if (ent & (1u << 12)) {
+                // a key outside the plan has no histogram row, so the dRL unfold of the scatter kernel never sees it: its
+                // expected-walk share d / sp for each of the L(rk) hops goes into dEW[k][dom] here (sp = L: rk >= 2 here)
+                const int rk = min(max((int)c.rel_pos[rowp + b], 0), kRelRows - 1);
+                fx_add(dR64 + rk * kH + h, d);
+                const int Lk = expected_walk(rk, c.dk);
+                const float dl = d * invT[max(Lk, 1)];
+                for (int k = 0; k < Lk; ++k) fx_add(sEW + (k * kSmallVocab + kDomEdge) * kH + h, dl);
+            }
             if (!(ent & (1u << 14))) continue;
             const uint32_t cd = lds_u32(s_cdev + (uint32_t)b * 4u);
             const int L = (cd >> 2) & 63, nd = cd & 3;
