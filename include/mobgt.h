@@ -139,9 +139,11 @@ int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *r
 /* ------------------------------------------------------------------------------------------
  * K3 — biased multi-head attention (tcgen05 / TMEM / TMA).  Replaces the core of
  * MultiHeadAttention.forward, model_fqandtoyo.py:1693-1706, for packed var-len graphs:
- * graph g owns token rows tok_off[g]..tok_off[g+1] (row 0 = graph token).  head dim is 24.
- *   q,k,v  bf16 [ntok, H*24] with a common row stride (elements) — usually slices of one fused projection
- *   bias   bf16 [B,H,T,Tp] from mobgt_bias_fwd ;  out bf16 [ntok, H*24] ;  lse f32 [ntok, H]
+ * graph g owns token rows tok_off[g]..tok_off[g+1] (row 0 = graph token).  d = the head dim: 24 for the entry points
+ * without a head_dim argument; the _hd variants take it as head_dim, built for 16 and 24 (any other value returns
+ * MOBGT_ERR_UNSUPPORTED).
+ *   q,k,v  bf16 [ntok, H*d] with a common row stride (elements) — usually slices of one fused projection
+ *   bias   bf16 [B,H,T,Tp] from mobgt_bias_fwd ;  out bf16 [ntok, H*d] ;  lse f32 [ntok, H]
  *   drop_p, seed, seed_dev: the attention dropout of model_fqandtoyo.py:1704 (`x = self.att_dropout(x)` on the softmax
  *          probabilities; training only — pass drop_p = 0 in eval).  The keep mask is a counter-based hash of
  *          (seed, plane, row, column), regenerated by the backward from the SAME seed: nothing is stored.  seed_dev (u64 in
@@ -160,9 +162,13 @@ int32_t mobgt_attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_
                        const int32_t *tok_off, const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp,
                        int32_t t_max_host, int32_t t_min_host, float scale, float drop_p, uint64_t seed, const void *seed_dev,
                        void *out, float *lse, void *stream);
+int32_t mobgt_attn_fwd_hd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                          const int32_t *tok_off, const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok, int32_t T,
+                          int32_t Tp, int32_t t_max_host, int32_t t_min_host, float scale, float drop_p, uint64_t seed,
+                          const void *seed_dev, void *out, float *lse, int32_t head_dim, void *stream);
 
-/* Backward of mobgt_attn_fwd.  o, dout: bf16 [ntok, H*24] contiguous; lse from the forward.
- * dq, dk, dv: bf16 with a common row stride (usually slices of one [ntok, 3*H*24] buffer).
+/* Backward of mobgt_attn_fwd.  o, dout: bf16 [ntok, H*d] contiguous; lse from the forward.
+ * dq, dk, dv: bf16 with a common row stride (usually slices of one [ntok, 3*H*d] buffer).
  * dbias receives dS = d(scores) = d(bias) [B,H,T,Tp]:
  *   mode 0: f32, overwritten ;  mode 1: f32, added to (the bias is shared by all encoder layers) ;
  *   mode 2: bf16, overwritten by ONE TMA store per tile from the MMA operand image — each layer writes its own plane and
@@ -174,6 +180,11 @@ int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_
                        int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host, float scale,
                        void *dq, void *dk, void *dv, int64_t dqkv_row_stride, void *dbias, int32_t mode, float drop_p,
                        uint64_t seed, const void *seed_dev, void *stream);
+int32_t mobgt_attn_bwd_hd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                          const void *o, const void *dout, const float *lse, const int32_t *tok_off, const int32_t *graph_order,
+                          int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host,
+                          float scale, void *dq, void *dk, void *dv, int64_t dqkv_row_stride, void *dbias, int32_t mode,
+                          float drop_p, uint64_t seed, const void *seed_dev, int32_t head_dim, void *stream);
 
 /* K3 in fp32 mode: the same attention core (model_fqandtoyo.py:1693-1706) with fp32 q / k / v / bias / out and fp32 math
  * (IEEE expf / logf, SIMT), for graphs of any size up to 513 tokens — the arithmetic of the reference's `--precision 32`
@@ -181,7 +192,8 @@ int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_
  * tensor-core kernels above round their operands to bf16 by construction.  Same packed layout, same dropout mask (seed, plane,
  * row, column) as mobgt_attn_fwd; lse is the natural-log row normaliser.  dbias f32 [B,H,T,Tp]: mode 0 overwritten, mode 1
  * added to (only the live cells of a graph are touched); feed it to mobgt_bias_bwd with dbias_dtype MOBGT_F32, n_layers 1.
- * Bitwise reproducible (fixed-order shuffle reductions, no atomics). */
+ * Bitwise reproducible (fixed-order shuffle reductions, no atomics).  Head dim 24; the _hd variants take it as head_dim
+ * (built: 16, 24; anything else returns MOBGT_ERR_UNSUPPORTED). */
 int32_t mobgt_attn_f32_fwd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
                            const int32_t *tok_off, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host,
                            float scale, float drop_p, uint64_t seed, const void *seed_dev, float *out, float *lse, void *stream);
@@ -190,6 +202,15 @@ int32_t mobgt_attn_f32_bwd(const float *q, const float *k, const float *v, int64
                            int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, float scale, float *dq, float *dk, float *dv,
                            int64_t dqkv_row_stride, float *dbias, int32_t mode, float drop_p, uint64_t seed, const void *seed_dev,
                            void *stream);
+int32_t mobgt_attn_f32_fwd_hd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
+                              const int32_t *tok_off, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp,
+                              int32_t t_max_host, float scale, float drop_p, uint64_t seed, const void *seed_dev, float *out,
+                              float *lse, int32_t head_dim, void *stream);
+int32_t mobgt_attn_f32_bwd_hd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
+                              const float *o, const float *dout, const float *lse, const int32_t *tok_off, int32_t B, int32_t H,
+                              int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, float scale, float *dq, float *dk, float *dv,
+                              int64_t dqkv_row_stride, float *dbias, int32_t mode, float drop_p, uint64_t seed,
+                              const void *seed_dev, int32_t head_dim, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * K4 — node-embedding gather / sum and the deterministic segmented scatter-add backward.

@@ -41,6 +41,15 @@ SIGNATURES = {
                            c_p, c_p, c_p],
     "mobgt_attn_f32_bwd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_p, c_p, c_p,
                            c_i64, c_p, c_i32, c_f32, ctypes.c_uint64, c_p, c_p],
+    # the same four with an int32 head_dim before the stream (built: 16, 24)
+    "mobgt_attn_fwd_hd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_f32,
+                          ctypes.c_uint64, c_p, c_p, c_p, c_i32, c_p],
+    "mobgt_attn_bwd_hd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_p,
+                          c_p, c_p, c_i64, c_p, c_i32, c_f32, ctypes.c_uint64, c_p, c_i32, c_p],
+    "mobgt_attn_f32_fwd_hd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_f32, ctypes.c_uint64,
+                              c_p, c_p, c_p, c_i32, c_p],
+    "mobgt_attn_f32_bwd_hd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_p, c_p,
+                              c_p, c_i64, c_p, c_i32, c_f32, ctypes.c_uint64, c_p, c_i32, c_p],
     "mobgt_embed_gather_fwd": [c_p, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_p, c_i32, c_p],
     "mobgt_embed_sum_fwd": [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_p, c_i32, c_p],
     "mobgt_segment_sum": [c_p, c_i32, c_i64, c_i32, c_i32, c_p, c_p, c_i32, c_p, c_i32, c_p, c_i64, c_p],

@@ -4,10 +4,11 @@
 //   P  = exp(scale * Q K^T + bias - lse)            recomputed per tile, never stored in HBM
 //   dP = dO V^T ;  D = rowsum(dO * O) ;  dS = P * (dP - D)          (dS is also d(bias))
 //   dV = P^T dO ;  dK = scale * dS^T Q ;  dQ = scale * dS K
-// One CTA per (graph, head).  Five MMAs per (kv block j, query tile i):
-//   S, dP    M=128 (queries) N<=128 K=32           -> TMEM [0,128), [128,256)
-//   dV, dK   M=128 (keys)    N=32   K=128 queries  -> TMEM [256,288), [288,320)   (accumulate over i)
-//   dQ_i     M=128 (queries) N=32   K<=128 keys    -> TMEM [320+32 i, ...)        (accumulate over j)
+// One CTA per (graph, head).  Five MMAs per (kv block j, query tile i), dp = the head dim d rounded up to 16
+// (d = 24: dp = 32, d = 16: dp = 16; k3_small.cuh AttnShape):
+//   S, dP    M=128 (queries) N<=128 K=dp           -> TMEM [0,128), [128,256)
+//   dV, dK   M=128 (keys)    N=dp   K=128 queries  -> TMEM [256,256+dp), [288,288+dp)   (accumulate over i)
+//   dQ_i     M=128 (queries) N=dp   K<=128 keys    -> TMEM [320+32 i, ...)              (accumulate over j)
 // P and dS are written once to shared memory as bf16 in the [chunk][row][8] layout; that single image is the
 // K-major A operand of dQ = dS.K and the MN-major (transposed) A operand of dV = P^T.dO / dK = dS^T.Q.
 // dS is streamed to the fp32 dBias buffer [B,H,T,Tp] (overwrite or accumulate across layers); the table gradients
@@ -22,11 +23,7 @@ namespace mobgt {
 using namespace sm100;
 
 namespace bwd {
-constexpr int kAttD = 24;
-constexpr int kAttChunks = 3;
 constexpr int kTile = 128;
-constexpr int kBoxBytes = 4 * kTile * 16;
-constexpr int kBoxTxBytes = kAttChunks * kTile * 16;
 constexpr int kBiasTileBytes = 2 * kTile * 128;
 constexpr int kPBytes = 16 * kTile * 16;
 constexpr int kMaxTiles = 5;   // T <= 513
@@ -35,8 +32,8 @@ using namespace bwd;
 
 struct AttnBwdParams {
     const int32_t *tok_off;
-    const __nv_bfloat16 *o;    // [ntok, H*24]
-    const __nv_bfloat16 *dout; // [ntok, H*24]
+    const __nv_bfloat16 *o;    // [ntok, H*d]
+    const __nv_bfloat16 *dout; // [ntok, H*d]
     const float *lse;          // [ntok, H]
     __nv_bfloat16 *dq, *dk, *dv;  // [ntok, *] with row stride dqkv_stride (elements)
     int64_t dqkv_stride;
@@ -55,14 +52,39 @@ struct AttnBwdParams {
     const int32_t *order;             // [B] graph ids in launch order (descending size) or NULL
 };
 
-// 24 bf16 (three 16-byte words) -> fp32
-__device__ __forceinline__ void unpack24(const uint4 &a, const uint4 &b, const uint4 &c, float (&f)[24]) {
-    const uint32_t w[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+// the d bf16 of row `row` of a [chunk][row][8] operand box -> fp32
+template <int kD>
+__device__ __forceinline__ void box_row(const uint8_t *box, int row, float (&f)[kD]) {
+    uint4 w[kD / 8];
 #pragma unroll
-    for (int e = 0; e < 12; ++e) {
-        f[2 * e] = __uint_as_float(w[e] << 16);
-        f[2 * e + 1] = __uint_as_float(w[e] & 0xFFFF0000u);
-    }
+    for (int c = 0; c < kD / 8; ++c) w[c] = *reinterpret_cast<const uint4 *>(box + c * (kTile * 16) + row * 16);
+    unpack_words<kD / 8>(w, f);
+}
+// d bf16 at 16-byte aligned global memory -> fp32
+template <int kD>
+__device__ __forceinline__ void global_row(const __nv_bfloat16 *src, float (&f)[kD]) {
+    const uint4 *g = reinterpret_cast<const uint4 *>(src);
+    uint4 w[kD / 8];
+#pragma unroll
+    for (int c = 0; c < kD / 8; ++c) w[c] = g[c];
+    unpack_words<kD / 8>(w, f);
+}
+// the d fp32 of an accumulator row (TMEM columns [0, d)) times sc -> bf16 at dst (16-byte aligned)
+template <int kD>
+__device__ __forceinline__ void store_row(__nv_bfloat16 *dst, const uint32_t *acc, float sc) {
+    uint4 *d = reinterpret_cast<uint4 *>(dst);
+#pragma unroll
+    for (int c = 0; c < kD / 8; ++c)
+        d[c] = make_uint4(pack_bf16(__uint_as_float(acc[8 * c]) * sc, __uint_as_float(acc[8 * c + 1]) * sc),
+                          pack_bf16(__uint_as_float(acc[8 * c + 2]) * sc, __uint_as_float(acc[8 * c + 3]) * sc),
+                          pack_bf16(__uint_as_float(acc[8 * c + 4]) * sc, __uint_as_float(acc[8 * c + 5]) * sc),
+                          pack_bf16(__uint_as_float(acc[8 * c + 6]) * sc, __uint_as_float(acc[8 * c + 7]) * sc));
+}
+// kDPad accumulator columns of this warp's 32 TMEM lanes
+template <int kDPad>
+__device__ __forceinline__ void tmem_ld_acc(uint32_t taddr, uint32_t (&r)[kDPad]) {
+    if constexpr (kDPad == 32) tmem_ld32(taddr, r);
+    else tmem_ld16(taddr, r);
 }
 __device__ __forceinline__ float bf16_at(const __nv_bfloat16 *p) { return __bfloat162float(*p); }
 
@@ -92,7 +114,7 @@ __device__ __forceinline__ void red_add_f32x4(float *addr, float a, float b, flo
 // full tiles only and the last token sp = 128 m is handled by plain SIMT math (lse is known, so every element is independent):
 //   row sp against all keys, all rows against key sp -> dS / P scalars in shared memory, their rank-1 contributions are added
 //   to the dK / dV / dQ accumulators in the epilogues, and dQ[sp], dK[sp], dV[sp] are three small mat-vec reductions.
-template <bool kDrop>
+template <int kAttD, bool kDrop>
 __global__ void __launch_bounds__(256, 1)
 k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                    const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
@@ -105,7 +127,10 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     __shared__ float sA_ds[kMaxTiles * kTile], sA_pd[kMaxTiles * kTile];   // tail: dS / dropped P of (row sp, key c)
     __shared__ float sB_ds[kMaxTiles * kTile], sB_pd[kMaxTiles * kTile];   // tail: dS / dropped P of (row r, key sp)
     __shared__ float sSp[4][kAttD];                                        // q, k, v, dO of token sp
-    __shared__ float sRed[3][10][kAttD];
+    __shared__ float sRed[3][AttnShape<kAttD>::kSegs][kAttD];
+    using Sh = AttnShape<kAttD>;
+    constexpr int kAttChunks = Sh::kChunks, kDPad = Sh::kDPad, kBoxBytes = Sh::kBoxBytes, kBoxTxBytes = Sh::kBoxTxBytes;
+    constexpr int kSegs = Sh::kSegs;
 
     MOBGT_STAMP(p.timeline, 0);
     const int tid = threadIdx.x, warp = tid >> 5, wg = tid >> 7, t128 = tid & 127;
@@ -126,13 +151,13 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     //   this thread's first row of the lse / delta prologue, and (fold) the bias row / column of the tail token.
     const int rows_pro = NB * kTile + (fold ? 1 : 0);
     float lse_pre = 0.f;
-    uint4 o_pre[3], d_pre[3];
+    uint4 o_pre[kAttChunks], d_pre[kAttChunks];
     if (tid < Tg && tid < rows_pro) {
         lse_pre = p.lse[(size_t)(t0 + tid) * p.H + h];
         const uint4 *po = reinterpret_cast<const uint4 *>(p.o + (size_t)(t0 + tid) * HD + h * kAttD);
         const uint4 *pd = reinterpret_cast<const uint4 *>(p.dout + (size_t)(t0 + tid) * HD + h * kAttD);
 #pragma unroll
-        for (int q = 0; q < 3; ++q) {
+        for (int q = 0; q < kAttChunks; ++q) {
             o_pre[q] = po[q];
             d_pre[q] = pd[q];
         }
@@ -184,7 +209,7 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         tma_load_3d(sBias, &tmBias, &bar_bias[0], 0, 0, plane0);
         tma_load_3d(sBias + kTile * 128, &tmBias, &bar_bias[0], 64, 0, plane0);
     }
-    {   // zero the K-padding chunk (d = 24..31) of every operand box: 128 rows x 16 B each
+    if (kDPad != kAttD) {   // zero the K-padding chunk (d = 24..31) of every operand box: 128 rows x 16 B each
         const uint4 z = make_uint4(0, 0, 0, 0);
         uint8_t *qd = wg == 0 ? sQ : sdO;
         *reinterpret_cast<uint4 *>(qd + 3 * kTile * 16 + t128 * 16) = z;
@@ -209,7 +234,7 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             const uint4 *po = reinterpret_cast<const uint4 *>(p.o + (size_t)(t0 + r) * HD + h * kAttD);
             const uint4 *pd = reinterpret_cast<const uint4 *>(p.dout + (size_t)(t0 + r) * HD + h * kAttD);
 #pragma unroll
-            for (int q = 0; q < 3; ++q) {
+            for (int q = 0; q < kAttChunks; ++q) {
                 const uint4 a = pre ? o_pre[q] : po[q], b = pre ? d_pre[q] : pd[q];
                 const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, bw[4] = {b.x, b.y, b.z, b.w};
 #pragma unroll
@@ -258,11 +283,11 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         const uint32_t aq = smem_u32(sQ + b * kBoxBytes), ado = smem_u32(sdO + b * kBoxBytes);
         const uint32_t bk = smem_u32(sK + (size_t)j * kBoxBytes), bv = smem_u32(sV + (size_t)j * kBoxBytes);
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks)
+        for (int ks = 0; ks < kDPad / 16; ++ks)
             umma_bf16(tS, make_smem_desc(aq + ks * 2 * kTile * 16, kTile * 16, 128),
                       make_smem_desc(bk + ks * 2 * kTile * 16, kTile * 16, 128), idesc, ks > 0);
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks)
+        for (int ks = 0; ks < kDPad / 16; ++ks)
             umma_bf16(tdP, make_smem_desc(ado + ks * 2 * kTile * 16, kTile * 16, 128),
                       make_smem_desc(bv + ks * 2 * kTile * 16, kTile * 16, 128), idesc, ks > 0);
         umma_commit(&bar_s);
@@ -293,12 +318,6 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             else if (p.accumulate == 1) atomicAdd(ds32 + o, v);
             else ds32[o] = v;
         };
-        // 24 bf16 of row `row` of a [chunk][row][8] operand box
-        auto box_row = [&](const uint8_t *box, int row, float (&f)[24]) {
-            const uint8_t *b0 = box + row * 16;
-            unpack24(*reinterpret_cast<const uint4 *>(b0), *reinterpret_cast<const uint4 *>(b0 + kTile * 16),
-                     *reinterpret_cast<const uint4 *>(b0 + 2 * kTile * 16), f);
-        };
         mbar_wait(&bar_kv, 0);                      // K / V boxes and the first Q / dO tile have landed
         mbar_wait(&bar_qdo[0], 0);                  // (every thread observes the phases; tile 0 stays put until iteration 1)
         {   // part A: query row sp against every key c (itself included)
@@ -310,9 +329,9 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
                 if (c >= Tg) break;
                 float dot = 0.f, dp = 0.f;
                 if (c < sp) {
-                    float kf[24], vf[24];
-                    box_row(sK + (size_t)(c >> 7) * kBoxBytes, c & 127, kf);
-                    box_row(sV + (size_t)(c >> 7) * kBoxBytes, c & 127, vf);
+                    float kf[kAttD], vf[kAttD];
+                    box_row<kAttD>(sK + (size_t)(c >> 7) * kBoxBytes, c & 127, kf);
+                    box_row<kAttD>(sV + (size_t)(c >> 7) * kBoxBytes, c & 127, vf);
 #pragma unroll
                     for (int e = 0; e < kAttD; ++e) {
                         dot = fmaf(sSp[0][e], kf[e], dot);
@@ -339,15 +358,13 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             for (int u = 0; u < 2; ++u) {
                 const int r = tid + u * 256;
                 if (r >= sp) break;
-                float qf[24], df[24];
+                float qf[kAttD], df[kAttD];
                 if (r < kTile) {
-                    box_row(sQ, r, qf);
-                    box_row(sdO, r, df);
+                    box_row<kAttD>(sQ, r, qf);
+                    box_row<kAttD>(sdO, r, df);
                 } else {
-                    const uint4 *qg = reinterpret_cast<const uint4 *>(p.q + (size_t)(t0 + r) * p.qkv_stride + h * kAttD);
-                    const uint4 *dg = reinterpret_cast<const uint4 *>(p.dout + (size_t)(t0 + r) * HD + h * kAttD);
-                    unpack24(qg[0], qg[1], qg[2], qf);
-                    unpack24(dg[0], dg[1], dg[2], df);
+                    global_row<kAttD>(p.q + (size_t)(t0 + r) * p.qkv_stride + h * kAttD, qf);
+                    global_row<kAttD>(p.dout + (size_t)(t0 + r) * HD + h * kAttD, df);
                 }
                 float dot = 0.f, dp = 0.f;
 #pragma unroll
@@ -372,24 +389,24 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             const int seg = tid / kAttD, e = tid - seg * kAttD;
             const int eo = (e >> 3) * (kTile * 16) + (e & 7) * 2;      // byte offset of element e inside a box row
             float aq = 0.f, ak = 0.f, av = 0.f;
-            for (int c = seg; c < sp; c += 10)                         // keys: every box is resident
+            for (int c = seg; c < sp; c += kSegs)                      // keys: every box is resident
                 aq = fmaf(sA_ds[c], bf16_at(reinterpret_cast<const __nv_bfloat16 *>(
                                         sK + (size_t)(c >> 7) * kBoxBytes + (c & 127) * 16 + eo)), aq);
-            for (int r = seg; r < kTile; r += 10) {                    // query rows of tile 0: shared memory
+            for (int r = seg; r < kTile; r += kSegs) {                 // query rows of tile 0: shared memory
                 ak = fmaf(sB_ds[r], bf16_at(reinterpret_cast<const __nv_bfloat16 *>(sQ + r * 16 + eo)), ak);
                 av = fmaf(sB_pd[r], bf16_at(reinterpret_cast<const __nv_bfloat16 *>(sdO + r * 16 + eo)), av);
             }
-            for (int r0 = kTile + seg; r0 < sp; r0 += 80) {            // further tiles: global, 8 rows in flight
+            for (int r0 = kTile + seg; r0 < sp; r0 += 8 * kSegs) {     // further tiles: global, 8 rows in flight
                 float qv8[8], dv8[8];
 #pragma unroll
                 for (int u = 0; u < 8; ++u) {
-                    const int r = r0 + 10 * u;
+                    const int r = r0 + kSegs * u;
                     qv8[u] = r < sp ? bf16_at(p.q + (size_t)(t0 + r) * p.qkv_stride + h * kAttD + e) : 0.f;
                     dv8[u] = r < sp ? bf16_at(p.dout + (size_t)(t0 + r) * HD + h * kAttD + e) : 0.f;
                 }
 #pragma unroll
                 for (int u = 0; u < 8; ++u) {
-                    const int r = r0 + 10 * u;
+                    const int r = r0 + kSegs * u;
                     if (r < sp) {
                         ak = fmaf(sB_ds[r], qv8[u], ak);
                         av = fmaf(sB_pd[r], dv8[u], av);
@@ -405,7 +422,7 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             const int which = tid / kAttD, e = tid - which * kAttD;
             float a = 0.f;
 #pragma unroll
-            for (int sg = 0; sg < 10; ++sg) a += sRed[which][sg][e];
+            for (int sg = 0; sg < kSegs; ++sg) a += sRed[which][sg][e];
             // the (sp, sp) element: dQ += dS k_sp ; dK += dS q_sp ; dV += P dO_sp
             a += which == 0 ? sA_ds[sp] * sSp[1][e] : which == 1 ? sA_ds[sp] * sSp[0][e] : sA_pd[sp] * sSp[3][e];
             if (which < 2) a *= p.scale;
@@ -554,8 +571,8 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
                 const uint32_t aP = smem_u32(sP), aS = smem_u32(sdS);
                 const uint32_t bQ = smem_u32(sQ + buf * kBoxBytes), bdO = smem_u32(sdO + buf * kBoxBytes);
                 const uint32_t bK = smem_u32(sK + (size_t)j * kBoxBytes);
-                const uint32_t id_t = make_idesc_bf16(kTile, 32, 1, 1);   // A = P^T / dS^T (MN-major), B MN-major
-                const uint32_t id_q = make_idesc_bf16(kTile, 32, 0, 1);   // A = dS (K-major),        B MN-major
+                const uint32_t id_t = make_idesc_bf16(kTile, kDPad, 1, 1);   // A = P^T / dS^T (MN-major), B MN-major
+                const uint32_t id_q = make_idesc_bf16(kTile, kDPad, 0, 1);   // A = dS (K-major),        B MN-major
                 for (int ks = 0; ks < qk / 16; ++ks)      // dV_j += P^T dO_i   (K = query rows)
                     umma_bf16(tdV, make_smem_desc(aP + ks * 256, 128, kTile * 16),
                               make_smem_desc(bdO + ks * 256, 128, kTile * 16), id_t, (i > 0 || ks > 0));
@@ -583,8 +600,8 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         {
             const int krow = j * kTile + t128;
             if (j * kTile + (warp & 3) * 32 < Tg) {
-                uint32_t kvv[32];
-                tmem_ld32((wg == 0 ? tdK : tdV) + lane_off, kvv);
+                uint32_t kvv[kDPad];
+                tmem_ld_acc<kDPad>((wg == 0 ? tdK : tdV) + lane_off, kvv);
                 tmem_ld_wait();
                 if (krow < Tg) {
                     const float sc = wg == 0 ? p.scale : 1.0f;
@@ -594,14 +611,7 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 #pragma unroll
                         for (int e = 0; e < kAttD; ++e) kvv[e] = __float_as_uint(fmaf(a, vec[e], __uint_as_float(kvv[e])));
                     }
-                    uint32_t w[12];
-#pragma unroll
-                    for (int e = 0; e < 12; ++e)
-                        w[e] = pack_bf16(__uint_as_float(kvv[2 * e]) * sc, __uint_as_float(kvv[2 * e + 1]) * sc);
-                    uint4 *dst = reinterpret_cast<uint4 *>((wg == 0 ? p.dk : p.dv) + (size_t)(t0 + krow) * p.dqkv_stride + h * kAttD);
-                    dst[0] = make_uint4(w[0], w[1], w[2], w[3]);
-                    dst[1] = make_uint4(w[4], w[5], w[6], w[7]);
-                    dst[2] = make_uint4(w[8], w[9], w[10], w[11]);
+                    store_row<kAttD>((wg == 0 ? p.dk : p.dv) + (size_t)(t0 + krow) * p.dqkv_stride + h * kAttD, kvv, sc);
                 }
             }
         }
@@ -613,8 +623,8 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     for (int i = wg; i < NB; i += 2) {
         const int row = i * kTile + t128;
         if (i * kTile + (warp & 3) * 32 >= Tg) continue;
-        uint32_t qv[32];
-        tmem_ld32(tdQ + 32 * i + lane_off, qv);
+        uint32_t qv[kDPad];
+        tmem_ld_acc<kDPad>(tdQ + 32 * i + lane_off, qv);
         tmem_ld_wait();
         if (row < Tg) {
             if (fold) {   // + dS[row][sp] k_sp
@@ -622,14 +632,7 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 #pragma unroll
                 for (int e = 0; e < kAttD; ++e) qv[e] = __float_as_uint(fmaf(a, sSp[1][e], __uint_as_float(qv[e])));
             }
-            uint32_t w[12];
-#pragma unroll
-            for (int e = 0; e < 12; ++e)
-                w[e] = pack_bf16(__uint_as_float(qv[2 * e]) * p.scale, __uint_as_float(qv[2 * e + 1]) * p.scale);
-            uint4 *dst = reinterpret_cast<uint4 *>(p.dq + (size_t)(t0 + row) * p.dqkv_stride + h * kAttD);
-            dst[0] = make_uint4(w[0], w[1], w[2], w[3]);
-            dst[1] = make_uint4(w[4], w[5], w[6], w[7]);
-            dst[2] = make_uint4(w[8], w[9], w[10], w[11]);
+            store_row<kAttD>(p.dq + (size_t)(t0 + row) * p.dqkv_stride + h * kAttD, qv, p.scale);
         }
     }
     if (warp0 && p.accumulate == 2) tma_store_wait_all();   // whichever lane of warp 0 was the elected issuer
@@ -650,12 +653,12 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 // (query tile, key block) per CTA none of that buffering buys anything, so this variant is sized for TWO CTAs per SM — one
 // CTA's TMA / MMA / TMEM round trips hide behind the other's softmax-gradient math:
 //   * S and dP are produced one after the other into the SAME 128 TMEM columns (P is taken to registers in between):
-//     128 + 3 x 32 = 224 columns -> a 256-column allocation;
+//     128 + 3 x 32 = 224 columns -> a 256-column allocation (d = 16 uses 16 of each accumulator's 32 columns);
 //   * the bias tile is consumed into P before dS exists, so the dS operand image reuses the bias tile's 32 KB;
 //     no double buffers: 97 KB of dynamic shared memory;
 //   * one score tile (64 fp32 P values) in registers at a time: <= 128 registers / thread.
 // Arithmetic, operand layouts, the dropout mask and the single-token tail are those of the general kernel.
-template <bool kDrop>
+template <int kAttD, bool kDrop>
 __global__ void __launch_bounds__(256, 2)
 k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                     const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
@@ -669,7 +672,10 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
     __shared__ float sA_ds[kRows], sA_pd[kRows];   // tail: dS / dropped P of (row sp, key c)
     __shared__ float sB_ds[kRows], sB_pd[kRows];   // tail: dS / dropped P of (row r, key sp)
     __shared__ float sSp[4][kAttD];                // q, k, v, dO of token sp
-    __shared__ float sRed[3][10][kAttD];
+    __shared__ float sRed[3][AttnShape<kAttD>::kSegs][kAttD];
+    using Sh = AttnShape<kAttD>;
+    constexpr int kAttChunks = Sh::kChunks, kDPad = Sh::kDPad, kBoxBytes = Sh::kBoxBytes, kBoxTxBytes = Sh::kBoxTxBytes;
+    constexpr int kSegs = Sh::kSegs;
 
     const int tid = threadIdx.x, warp = tid >> 5, wg = tid >> 7, t128 = tid & 127;
     const bool warp0 = warp_index_uniform() == 0;
@@ -686,13 +692,13 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 
     // ---- global loads issued at the very top (consumed after the barrier / TMA set-up): one row per thread (Tg <= 129 < 256)
     float lse_pre = 0.f;
-    uint4 o_pre[3], d_pre[3];
+    uint4 o_pre[kAttChunks], d_pre[kAttChunks];
     if (tid < Tg) {
         lse_pre = p.lse[(size_t)(t0 + tid) * p.H + h];
         const uint4 *po = reinterpret_cast<const uint4 *>(p.o + (size_t)(t0 + tid) * HD + h * kAttD);
         const uint4 *pd = reinterpret_cast<const uint4 *>(p.dout + (size_t)(t0 + tid) * HD + h * kAttD);
 #pragma unroll
-        for (int q = 0; q < 3; ++q) {
+        for (int q = 0; q < kAttChunks; ++q) {
             o_pre[q] = po[q];
             d_pre[q] = pd[q];
         }
@@ -738,7 +744,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         tma_load_3d(sBD, &tmBias, &bar_bias, 0, 0, plane);
         tma_load_3d(sBD + kTile * 128, &tmBias, &bar_bias, 64, 0, plane);
     }
-    {   // zero the K-padding chunk (d = 24..31) of the four operand boxes
+    if (kDPad != kAttD) {   // zero the K-padding chunk (d = 24..31) of the four operand boxes
         const uint4 z = make_uint4(0, 0, 0, 0);
         *reinterpret_cast<uint4 *>((wg == 0 ? sQ : sdO) + 3 * kTile * 16 + t128 * 16) = z;
         *reinterpret_cast<uint4 *>((wg == 0 ? sK : sV) + 3 * kTile * 16 + t128 * 16) = z;
@@ -748,7 +754,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         if (tid < Tg) {
             lse2 = lse_pre * 1.4426950408889634f;
 #pragma unroll
-            for (int q = 0; q < 3; ++q) {
+            for (int q = 0; q < kAttChunks; ++q) {
                 const uint32_t aw[4] = {o_pre[q].x, o_pre[q].y, o_pre[q].z, o_pre[q].w};
                 const uint32_t bw[4] = {d_pre[q].x, d_pre[q].y, d_pre[q].z, d_pre[q].w};
 #pragma unroll
@@ -778,7 +784,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         tc_fence_after();
         const uint32_t aq = smem_u32(sQ), bk = smem_u32(sK);
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks)
+        for (int ks = 0; ks < kDPad / 16; ++ks)
             umma_bf16(tS, make_smem_desc(aq + ks * 2 * kTile * 16, kTile * 16, 128),
                       make_smem_desc(bk + ks * 2 * kTile * 16, kTile * 16, 128), id_sn, ks > 0);
         umma_commit(&bar_s);
@@ -793,20 +799,15 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 
     if (fold) {   // ---- the single-token tail, SIMT (overlaps the S MMA)
         __nv_bfloat16 *ds16 = reinterpret_cast<__nv_bfloat16 *>(p.dbias) + (size_t)plane * p.T * p.Tp;
-        auto box_row = [&](const uint8_t *box, int row, float (&f)[24]) {
-            const uint8_t *b0 = box + row * 16;
-            unpack24(*reinterpret_cast<const uint4 *>(b0), *reinterpret_cast<const uint4 *>(b0 + kTile * 16),
-                     *reinterpret_cast<const uint4 *>(b0 + 2 * kTile * 16), f);
-        };
         mbar_wait(&bar_ld, 0);
         if (tid < Tg) {   // part A: query row sp against key c = tid (itself included)
             const int c = tid;
             const uint32_t rk = kDrop ? attn_drop_rowkey((uint32_t)plane, (uint32_t)sp, seed_lo, seed_hi) : 0u;
             float dot = 0.f, dp = 0.f;
             if (c < sp) {
-                float kf[24], vf[24];
-                box_row(sK, c, kf);
-                box_row(sV, c, vf);
+                float kf[kAttD], vf[kAttD];
+                box_row<kAttD>(sK, c, kf);
+                box_row<kAttD>(sV, c, vf);
 #pragma unroll
                 for (int e = 0; e < kAttD; ++e) {
                     dot = fmaf(sSp[0][e], kf[e], dot);
@@ -829,9 +830,9 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         }
         if (tid < sp) {   // part B: query row r = tid against key sp
             const int r = tid;
-            float qf[24], df[24];
-            box_row(sQ, r, qf);
-            box_row(sdO, r, df);
+            float qf[kAttD], df[kAttD];
+            box_row<kAttD>(sQ, r, qf);
+            box_row<kAttD>(sdO, r, df);
             float dot = 0.f, dp = 0.f;
 #pragma unroll
             for (int e = 0; e < kAttD; ++e) {
@@ -854,7 +855,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
             const int seg = tid / kAttD, e = tid - seg * kAttD;
             const int eo = (e >> 3) * (kTile * 16) + (e & 7) * 2;
             float aq = 0.f, ak = 0.f, av = 0.f;
-            for (int c = seg; c < sp; c += 10) {
+            for (int c = seg; c < sp; c += kSegs) {
                 aq = fmaf(sA_ds[c], bf16_at(reinterpret_cast<const __nv_bfloat16 *>(sK + c * 16 + eo)), aq);
                 ak = fmaf(sB_ds[c], bf16_at(reinterpret_cast<const __nv_bfloat16 *>(sQ + c * 16 + eo)), ak);
                 av = fmaf(sB_pd[c], bf16_at(reinterpret_cast<const __nv_bfloat16 *>(sdO + c * 16 + eo)), av);
@@ -868,7 +869,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
             const int which = tid / kAttD, e = tid - which * kAttD;
             float a = 0.f;
 #pragma unroll
-            for (int sg = 0; sg < 10; ++sg) a += sRed[which][sg][e];
+            for (int sg = 0; sg < kSegs; ++sg) a += sRed[which][sg][e];
             a += which == 0 ? sA_ds[sp] * sSp[1][e] : which == 1 ? sA_ds[sp] * sSp[0][e] : sA_pd[sp] * sSp[3][e];
             if (which < 2) a *= p.scale;
             __nv_bfloat16 *dst = (which == 0 ? p.dq : which == 1 ? p.dk : p.dv) + (size_t)(t0 + sp) * p.dqkv_stride + h * kAttD + e;
@@ -931,7 +932,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         tc_fence_after();
         const uint32_t ado = smem_u32(sdO), bv = smem_u32(sV);
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks)
+        for (int ks = 0; ks < kDPad / 16; ++ks)
             umma_bf16(tS, make_smem_desc(ado + ks * 2 * kTile * 16, kTile * 16, 128),
                       make_smem_desc(bv + ks * 2 * kTile * 16, kTile * 16, 128), id_sn, ks > 0);
         umma_commit(&bar_s);
@@ -1002,8 +1003,8 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         tma_store_commit();
         const uint32_t aP = smem_u32(sP), aS = smem_u32(sBD);
         const uint32_t bQ = smem_u32(sQ), bdO = smem_u32(sdO), bK = smem_u32(sK);
-        const uint32_t id_t = make_idesc_bf16(kTile, 32, 1, 1);   // A = P^T / dS^T (MN-major), B MN-major
-        const uint32_t id_q = make_idesc_bf16(kTile, 32, 0, 1);   // A = dS (K-major),        B MN-major
+        const uint32_t id_t = make_idesc_bf16(kTile, kDPad, 1, 1);   // A = P^T / dS^T (MN-major), B MN-major
+        const uint32_t id_q = make_idesc_bf16(kTile, kDPad, 0, 1);   // A = dS (K-major),        B MN-major
         for (int ks = 0; ks < nb / 16; ++ks)      // dV = P^T dO   (K = query rows)
             umma_bf16(tdV, make_smem_desc(aP + ks * 256, 128, kTile * 16), make_smem_desc(bdO + ks * 256, 128, kTile * 16), id_t, ks > 0);
         for (int ks = 0; ks < nb / 16; ++ks)      // dK = dS^T Q
@@ -1017,8 +1018,8 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
     tc_fence_after();
     if (warp_live) {
         {   // dK (warpgroup 0) / dV (warpgroup 1): key row = t128
-            uint32_t kvv[32];
-            tmem_ld32((wg == 0 ? tdK : tdV) + lane_off, kvv);
+            uint32_t kvv[kDPad];
+            tmem_ld_acc<kDPad>((wg == 0 ? tdK : tdV) + lane_off, kvv);
             tmem_ld_wait();
             if (row_ok) {
                 const float sc = wg == 0 ? p.scale : 1.0f;
@@ -1028,17 +1029,10 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 #pragma unroll
                     for (int e = 0; e < kAttD; ++e) kvv[e] = __float_as_uint(fmaf(a, vec[e], __uint_as_float(kvv[e])));
                 }
-                uint32_t w[12];
-#pragma unroll
-                for (int e = 0; e < 12; ++e)
-                    w[e] = pack_bf16(__uint_as_float(kvv[2 * e]) * sc, __uint_as_float(kvv[2 * e + 1]) * sc);
-                uint4 *dst = reinterpret_cast<uint4 *>((wg == 0 ? p.dk : p.dv) + (size_t)(t0 + row) * p.dqkv_stride + h * kAttD);
-                dst[0] = make_uint4(w[0], w[1], w[2], w[3]);
-                dst[1] = make_uint4(w[4], w[5], w[6], w[7]);
-                dst[2] = make_uint4(w[8], w[9], w[10], w[11]);
+                store_row<kAttD>((wg == 0 ? p.dk : p.dv) + (size_t)(t0 + row) * p.dqkv_stride + h * kAttD, kvv, sc);
             }
         }
-        {   // dQ: columns [0,16) by warpgroup 0, [16,24) by warpgroup 1
+        if (kAttD > 16 || wg == 0) {   // dQ: columns [0,16) by warpgroup 0, [16,24) by warpgroup 1 (d = 16: warpgroup 0 alone)
             uint32_t qv[16];
             tmem_ld16(tdQ + lane_off + wg * 16, qv);
             tmem_ld_wait();
@@ -1047,7 +1041,7 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
                     const float a = sB_ds[row];
 #pragma unroll
                     for (int e = 0; e < 16; ++e)
-                        if (wg == 0 || e < 8) qv[e] = __float_as_uint(fmaf(a, sSp[1][wg * 16 + e], __uint_as_float(qv[e])));
+                        if (wg == 0 || e < kAttD - 16) qv[e] = __float_as_uint(fmaf(a, sSp[1][wg * 16 + e], __uint_as_float(qv[e])));
                 }
                 uint32_t w[8];
 #pragma unroll
@@ -1073,15 +1067,19 @@ k3_attn_bwd1_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 
 using namespace mobgt;
 
-// Inputs as mobgt_attn_fwd plus o, dout (bf16 [ntok, H*24], contiguous) and lse.  Outputs dq, dk, dv: bf16 with a common
-// row stride (usually slices of one [ntok, 3*H*24] buffer, so the fused projection's backward gets a single tensor);
+namespace {
+// Inputs as mobgt_attn_fwd plus o, dout (bf16 [ntok, H*d], contiguous) and lse.  Outputs dq, dk, dv: bf16 with a common
+// row stride (usually slices of one [ntok, 3*H*d] buffer, so the fused projection's backward gets a single tensor);
 // dbias f32 [B,H,T,Tp]: overwritten (accumulate = 0) or accumulated into (accumulate = 1).
-extern "C" int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
-                                  const void *o, const void *dout, const float *lse, const int32_t *tok_off,
-                                  const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host,
-                                  float scale, void *dq,
-                                  void *dk, void *dv, int64_t dqkv_row_stride, void *dbias, int32_t accumulate, float drop_p,
-                                  uint64_t seed, const void *seed_dev, void *stream) {
+template <int kAttD>
+int32_t attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                 const void *o, const void *dout, const float *lse, const int32_t *tok_off,
+                 const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host,
+                 float scale, void *dq,
+                 void *dk, void *dv, int64_t dqkv_row_stride, void *dbias, int32_t accumulate, float drop_p,
+                 uint64_t seed, const void *seed_dev, void *stream) {
+    using Sh = AttnShape<kAttD>;
+    constexpr int kAttChunks = Sh::kChunks, kBoxBytes = Sh::kBoxBytes;
     MOBGT_REQUIRE(q && k && v && bias && o && dout && lse && tok_off && dq && dk && dv && dbias, MOBGT_ERR_NULL,
                   "mobgt_attn_bwd: null pointer");
     MOBGT_REQUIRE(qkv_row_stride % 8 == 0 && dqkv_row_stride % 8 == 0 && Tp % 8 == 0 && Tp >= T, MOBGT_ERR_BAD_SHAPE,
@@ -1109,13 +1107,13 @@ extern "C" int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, i
         sp.dq = static_cast<__nv_bfloat16 *>(dq); sp.dk = static_cast<__nv_bfloat16 *>(dk); sp.dv = static_cast<__nv_bfloat16 *>(dv);
         sp.dqkv_stride = dqkv_row_stride;
         sp.dbias = dbias; sp.accumulate = accumulate;
-        if (!any_large) return launch_small_attn_bwd(sp, B, static_cast<cudaStream_t>(stream));
+        if (!any_large) return launch_small_attn_bwd<kAttD>(sp, B, static_cast<cudaStream_t>(stream));
         // both kernels: they work on disjoint graphs, so the SIMT one runs on a side stream next to the tensor-core one
         int32_t rc = get_fork_join(1, &fj);
         if (rc) return rc;
         MOBGT_CUDA_OK(cudaEventRecord(fj.fork, static_cast<cudaStream_t>(stream)));
         MOBGT_CUDA_OK(cudaStreamWaitEvent(fj.side, fj.fork, 0));
-        rc = launch_small_attn_bwd(sp, B, fj.side);
+        rc = launch_small_attn_bwd<kAttD>(sp, B, fj.side);
         MOBGT_CUDA_OK(cudaEventRecord(fj.join, fj.side));
         forked = true;
         if (rc) {
@@ -1156,7 +1154,7 @@ extern "C" int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, i
     const size_t smem = smem_base + (size_t)bias_bufs * kBiasTileBytes;
     MOBGT_REQUIRE(drop_p >= 0.f && drop_p < 1.f, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_bwd: drop_p=%f must be in [0, 1)", drop_p);
     const AttnDrop drop = make_attn_drop(drop_p, seed, seed_dev);
-    auto kern = drop.th16 ? k3_attn_bwd_kernel<true> : k3_attn_bwd_kernel<false>;
+    auto kern = drop.th16 ? k3_attn_bwd_kernel<kAttD, true> : k3_attn_bwd_kernel<kAttD, false>;
     MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     AttnBwdParams p{tok_off,
                     static_cast<const __nv_bfloat16 *>(o),
@@ -1184,7 +1182,7 @@ extern "C" int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, i
                     any_small ? kSmallT : 0, graph_order};
     if (accumulate == 2 && t_max_host <= kTile + 1) {   // every graph fits one (query tile, key block): two CTAs per SM
         const size_t smem1 = (size_t)kBiasTileBytes + kPBytes + 4 * kBoxBytes + 1024;
-        auto kern1 = drop.th16 ? k3_attn_bwd1_kernel<true> : k3_attn_bwd1_kernel<false>;
+        auto kern1 = drop.th16 ? k3_attn_bwd1_kernel<kAttD, true> : k3_attn_bwd1_kernel<kAttD, false>;
         MOBGT_CUDA_OK(cudaFuncSetAttribute(kern1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
         MOBGT_CUDA_OK(cudaFuncSetAttribute(kern1, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
         kern1<<<B * H, 256, smem1, static_cast<cudaStream_t>(stream)>>>(tmQ, tmK, tmV, tmdO, tmB, tmDS, p);
@@ -1198,4 +1196,28 @@ extern "C" int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, i
     const int32_t rc = run_tensor_core();
     if (forked) cudaStreamWaitEvent(static_cast<cudaStream_t>(stream), fj.join, 0);   // join on every path
     return rc;
+}
+}  // namespace
+
+extern "C" int32_t mobgt_attn_bwd_hd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                                     const void *o, const void *dout, const float *lse, const int32_t *tok_off,
+                                     const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp,
+                                     int32_t t_max_host, int32_t t_min_host, float scale, void *dq, void *dk, void *dv,
+                                     int64_t dqkv_row_stride, void *dbias, int32_t accumulate, float drop_p, uint64_t seed,
+                                     const void *seed_dev, int32_t head_dim, void *stream) {
+    MOBGT_REQUIRE(head_dim == 16 || head_dim == 24, MOBGT_ERR_UNSUPPORTED,
+                  "mobgt_attn_bwd_hd: head_dim=%d is not built (head dims 16 and 24)", head_dim);
+    auto f = head_dim == 16 ? attn_bwd<16> : attn_bwd<24>;
+    return f(q, k, v, qkv_row_stride, bias, o, dout, lse, tok_off, graph_order, B, H, ntok, T, Tp, t_max_host, t_min_host, scale,
+             dq, dk, dv, dqkv_row_stride, dbias, accumulate, drop_p, seed, seed_dev, stream);
+}
+
+extern "C" int32_t mobgt_attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                                  const void *o, const void *dout, const float *lse, const int32_t *tok_off,
+                                  const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host,
+                                  float scale, void *dq,
+                                  void *dk, void *dv, int64_t dqkv_row_stride, void *dbias, int32_t accumulate, float drop_p,
+                                  uint64_t seed, const void *seed_dev, void *stream) {
+    return mobgt_attn_bwd_hd(q, k, v, qkv_row_stride, bias, o, dout, lse, tok_off, graph_order, B, H, ntok, T, Tp, t_max_host,
+                             t_min_host, scale, dq, dk, dv, dqkv_row_stride, dbias, accumulate, drop_p, seed, seed_dev, 24, stream);
 }

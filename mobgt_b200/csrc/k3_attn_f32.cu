@@ -8,9 +8,10 @@
 // compare logits, loss and every parameter gradient with the fp32 oracle at 1e-5.  It is a verification / full-precision
 // mode, not the benchmarked one: plain SIMT FFMA, one CTA per (graph, head), IEEE expf / logf.
 //
-// Layout: K and V (backward: Q, K, V, dO) of the (graph, head) are staged in shared memory with a 25-float row pitch (lanes
-// read different rows: conflict-free); a warp owns one query row (forward and the dQ / dS pass) or one key column (the dK / dV
-// pass) at a time, its lanes stride over the other index, and the 24-wide partial sums are merged by shuffles in a fixed
+// Layout: K and V (backward: Q, K, V, dO) of the (graph, head) are staged in shared memory with an odd row pitch of d + 1 floats
+// (25 for head dim 24, 17 for 16: lanes read different rows, conflict-free); a warp owns one query row (forward and the dQ / dS
+// pass) or one key column (the dK / dV pass) at a time, its lanes stride over the other index, and the d-wide partial sums are
+// merged by shuffles in a fixed
 // order — no atomics, bitwise reproducible.  Scores and probabilities are recomputed, never stored.  The dropout mask is the
 // tensor-core path's (common.cuh attn_drop_*: same seed, same mask).
 #include "common.cuh"
@@ -18,8 +19,6 @@
 namespace mobgt {
 
 namespace {
-constexpr int kD = 24;
-constexpr int kPitch = 25;
 constexpr int kWarps = 8;
 constexpr int kThreadsF = kWarps * 32;
 constexpr int kMaxT = 513;
@@ -32,7 +31,7 @@ struct F32AttnParams {
     int H, T, Tp;
     float scale;
     AttnDrop drop;
-    float *out, *lse;             // [ntok, H*24], [ntok, H]  (backward: o / lse are inputs)
+    float *out, *lse;             // [ntok, H*d], [ntok, H]  (backward: o / lse are inputs)
     const float *o, *dout;
     float *dq, *dk, *dv;
     int64_t dqkv_stride;
@@ -50,14 +49,16 @@ __device__ __forceinline__ float warp_max(float x) {
     for (int o = 16; o > 0; o >>= 1) x = fmaxf(x, __shfl_xor_sync(0xFFFFFFFFu, x, o));
     return x;
 }
-// rows [t0, t0 + Tg) x 24 floats of head h of a [ntok, stride] matrix -> dst[row * 25 + e]
+// rows [t0, t0 + Tg) x d floats of head h of a [ntok, stride] matrix -> dst[row * (d + 1) + e]
+template <int kD, int kPitch = kD + 1>
 __device__ __forceinline__ void stage(const float *src, int64_t stride, int t0, int Tg, int h, float *dst) {
     for (int i = threadIdx.x; i < Tg * kD; i += kThreadsF) {
         const int r = i / kD, e = i - r * kD;
         dst[r * kPitch + e] = __ldg(src + (size_t)(t0 + r) * stride + h * kD + e);
     }
 }
-__device__ __forceinline__ float dot24(const float (&a)[kD], const float *b) {
+template <int kD>
+__device__ __forceinline__ float dotd(const float (&a)[kD], const float *b) {
     float s = 0.f;
 #pragma unroll
     for (int e = 0; e < kD; ++e) s = fmaf(a[e], b[e], s);
@@ -70,14 +71,16 @@ __device__ __forceinline__ bool keep_bit(bool on, uint32_t rowkey, int col, uint
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------- forward
+template <int kD>
 __global__ void __launch_bounds__(kThreadsF) k3f_attn_fwd_kernel(const F32AttnParams p) {
+    constexpr int kPitch = kD + 1;
     extern __shared__ __align__(16) float smem[];
     const int g = blockIdx.x / p.H, h = blockIdx.x - g * p.H;
     const int t0 = p.tok_off[g], Tg = p.tok_off[g + 1] - t0;
     if (Tg <= 0) return;
     float *sK = smem, *sV = smem + Tg * kPitch;
-    stage(p.k, p.qkv_stride, t0, Tg, h, sK);
-    stage(p.v, p.qkv_stride, t0, Tg, h, sV);
+    stage<kD>(p.k, p.qkv_stride, t0, Tg, h, sK);
+    stage<kD>(p.v, p.qkv_stride, t0, Tg, h, sV);
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const bool drop = p.drop.th16 != 0;
@@ -92,13 +95,13 @@ __global__ void __launch_bounds__(kThreadsF) k3f_attn_fwd_kernel(const F32AttnPa
         const float *brow = p.bias + ((size_t)plane * p.T + i) * p.Tp;
         const uint32_t rowkey = drop ? attn_drop_rowkey((uint32_t)plane, (uint32_t)i, seed_lo, seed_hi) : 0u;
         float m = -INFINITY;
-        for (int j = lane; j < Tg; j += 32) m = fmaxf(m, fmaf(p.scale, dot24(q, sK + j * kPitch), __ldg(brow + j)));
+        for (int j = lane; j < Tg; j += 32) m = fmaxf(m, fmaf(p.scale, dotd(q, sK + j * kPitch), __ldg(brow + j)));
         m = warp_max(m);
         float l = 0.f, o[kD];
 #pragma unroll
         for (int e = 0; e < kD; ++e) o[e] = 0.f;
         for (int j = lane; j < Tg; j += 32) {
-            const float pe = expf(fmaf(p.scale, dot24(q, sK + j * kPitch), __ldg(brow + j)) - m);
+            const float pe = expf(fmaf(p.scale, dotd(q, sK + j * kPitch), __ldg(brow + j)) - m);
             l += pe;                                          // the denominator is taken before the dropout mask
             if (keep_bit(drop, rowkey, j, p.drop.th16)) {
                 const float *vr = sV + j * kPitch;
@@ -123,7 +126,9 @@ __global__ void __launch_bounds__(kThreadsF) k3f_attn_fwd_kernel(const F32AttnPa
 // pass A, warp = query row i: D_i = dO_i . O_i ; per key j: p = exp(s - lse_i), dP = dO_i . V_j (masked, / keep),
 //         dS = p (dP - D_i) -> dbias, dQ_i = scale * sum_j dS K_j
 // pass B, warp = key column j: the same p / dS recomputed per query row i: dK_j = scale * sum_i dS Q_i, dV_j = sum_i (mask p / keep) dO_i
+template <int kD>
 __global__ void __launch_bounds__(kThreadsF) k3f_attn_bwd_kernel(const F32AttnParams p) {
+    constexpr int kPitch = kD + 1;
     extern __shared__ __align__(16) float smem[];
     const int g = blockIdx.x / p.H, h = blockIdx.x - g * p.H;
     const int t0 = p.tok_off[g], Tg = p.tok_off[g + 1] - t0;
@@ -131,10 +136,10 @@ __global__ void __launch_bounds__(kThreadsF) k3f_attn_bwd_kernel(const F32AttnPa
     const int HD = p.H * kD;
     float *sQ = smem, *sK = sQ + Tg * kPitch, *sV = sK + Tg * kPitch, *sdO = sV + Tg * kPitch;
     float *sLse = sdO + Tg * kPitch, *sDel = sLse + Tg;
-    stage(p.q, p.qkv_stride, t0, Tg, h, sQ);
-    stage(p.k, p.qkv_stride, t0, Tg, h, sK);
-    stage(p.v, p.qkv_stride, t0, Tg, h, sV);
-    stage(p.dout, HD, t0, Tg, h, sdO);
+    stage<kD>(p.q, p.qkv_stride, t0, Tg, h, sQ);
+    stage<kD>(p.k, p.qkv_stride, t0, Tg, h, sK);
+    stage<kD>(p.v, p.qkv_stride, t0, Tg, h, sV);
+    stage<kD>(p.dout, HD, t0, Tg, h, sdO);
     for (int i = threadIdx.x; i < Tg; i += kThreadsF) {
         const float *og = p.o + (size_t)(t0 + i) * HD + h * kD, *dg = p.dout + (size_t)(t0 + i) * HD + h * kD;
         float d = 0.f;
@@ -166,8 +171,8 @@ __global__ void __launch_bounds__(kThreadsF) k3f_attn_bwd_kernel(const F32AttnPa
         float *drow = p.dbias + pl + (size_t)i * p.Tp;
         for (int j = lane; j < Tg; j += 32) {
             const float *kr = sK + j * kPitch;
-            const float pr = expf(fmaf(p.scale, dot24(q, kr), __ldg(brow + j)) - lse);
-            const float dp = keep_bit(drop, rowkey, j, p.drop.th16) ? dot24(dO, sV + j * kPitch) * ik : 0.f;
+            const float pr = expf(fmaf(p.scale, dotd(q, kr), __ldg(brow + j)) - lse);
+            const float dp = keep_bit(drop, rowkey, j, p.drop.th16) ? dotd(dO, sV + j * kPitch) * ik : 0.f;
             const float ds = pr * (dp - del);
             drow[j] = (p.accumulate == 1 ? drow[j] : 0.f) + ds;
 #pragma unroll
@@ -192,11 +197,11 @@ __global__ void __launch_bounds__(kThreadsF) k3f_attn_bwd_kernel(const F32AttnPa
         }
         for (int i = lane; i < Tg; i += 32) {
             const float *qr = sQ + i * kPitch, *dor = sdO + i * kPitch;
-            const float pr = expf(fmaf(p.scale, dot24(k, qr), __ldg(p.bias + pl + (size_t)i * p.Tp + j)) - sLse[i]);
+            const float pr = expf(fmaf(p.scale, dotd(k, qr), __ldg(p.bias + pl + (size_t)i * p.Tp + j)) - sLse[i]);
             bool kp = true;
             if (drop) kp = keep_bit(true, attn_drop_rowkey((uint32_t)plane, (uint32_t)i, seed_lo, seed_hi), j, p.drop.th16);
             const float pd = kp ? pr * ik : 0.f;
-            const float ds = pr * ((kp ? dot24(v, dor) * ik : 0.f) - sDel[i]);
+            const float ds = pr * ((kp ? dotd(v, dor) * ik : 0.f) - sDel[i]);
 #pragma unroll
             for (int e = 0; e < kD; ++e) {
                 dk[e] = fmaf(ds, qr[e], dk[e]);
@@ -233,10 +238,12 @@ int32_t check_common(const void *q, const void *k, const void *v, const void *bi
 
 using namespace mobgt;
 
-extern "C" int32_t mobgt_attn_f32_fwd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
-                                      const int32_t *tok_off, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp,
-                                      int32_t t_max_host, float scale, float drop_p, uint64_t seed, const void *seed_dev, float *out,
-                                      float *lse, void *stream) {
+extern "C" int32_t mobgt_attn_f32_fwd_hd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
+                                         const int32_t *tok_off, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp,
+                                         int32_t t_max_host, float scale, float drop_p, uint64_t seed, const void *seed_dev, float *out,
+                                         float *lse, int32_t head_dim, void *stream) {
+    MOBGT_REQUIRE(head_dim == 16 || head_dim == 24, MOBGT_ERR_UNSUPPORTED,
+                  "mobgt_attn_f32_fwd_hd: head_dim=%d is not built (head dims 16 and 24)", head_dim);
     const int32_t rc = check_common(q, k, v, bias, tok_off, B, H, ntok, T, Tp, t_max_host, drop_p);
     if (rc != MOBGT_OK) return rc;
     MOBGT_REQUIRE(out && lse, MOBGT_ERR_NULL, "mobgt_attn_f32_fwd: null output");
@@ -245,18 +252,21 @@ extern "C" int32_t mobgt_attn_f32_fwd(const float *q, const float *k, const floa
     p.tok_off = tok_off; p.q = q; p.k = k; p.v = v; p.qkv_stride = qkv_row_stride; p.bias = bias;
     p.H = H; p.T = T; p.Tp = Tp; p.scale = scale; p.drop = make_attn_drop(drop_p, seed, seed_dev);
     p.out = out; p.lse = lse;
-    const size_t smem = (size_t)2 * t_max_host * kPitch * sizeof(float);
-    MOBGT_CUDA_OK(cudaFuncSetAttribute(k3f_attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k3f_attn_fwd_kernel<<<B * H, kThreadsF, smem, static_cast<cudaStream_t>(stream)>>>(p);
+    const size_t smem = (size_t)2 * t_max_host * (head_dim + 1) * sizeof(float);    // row pitch d + 1
+    auto kern = head_dim == 16 ? k3f_attn_fwd_kernel<16> : k3f_attn_fwd_kernel<24>;
+    MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<B * H, kThreadsF, smem, static_cast<cudaStream_t>(stream)>>>(p);
     MOBGT_LAUNCH_OK("k3f_attn_fwd_kernel");
     return MOBGT_OK;
 }
 
-extern "C" int32_t mobgt_attn_f32_bwd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
-                                      const float *o, const float *dout, const float *lse, const int32_t *tok_off, int32_t B,
-                                      int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, float scale, float *dq,
-                                      float *dk, float *dv, int64_t dqkv_row_stride, float *dbias, int32_t mode, float drop_p,
-                                      uint64_t seed, const void *seed_dev, void *stream) {
+extern "C" int32_t mobgt_attn_f32_bwd_hd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
+                                         const float *o, const float *dout, const float *lse, const int32_t *tok_off, int32_t B,
+                                         int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, float scale, float *dq,
+                                         float *dk, float *dv, int64_t dqkv_row_stride, float *dbias, int32_t mode, float drop_p,
+                                         uint64_t seed, const void *seed_dev, int32_t head_dim, void *stream) {
+    MOBGT_REQUIRE(head_dim == 16 || head_dim == 24, MOBGT_ERR_UNSUPPORTED,
+                  "mobgt_attn_f32_bwd_hd: head_dim=%d is not built (head dims 16 and 24)", head_dim);
     const int32_t rc = check_common(q, k, v, bias, tok_off, B, H, ntok, T, Tp, t_max_host, drop_p);
     if (rc != MOBGT_OK) return rc;
     MOBGT_REQUIRE(o && dout && lse && dq && dk && dv && dbias, MOBGT_ERR_NULL, "mobgt_attn_f32_bwd: null pointer");
@@ -267,9 +277,27 @@ extern "C" int32_t mobgt_attn_f32_bwd(const float *q, const float *k, const floa
     p.H = H; p.T = T; p.Tp = Tp; p.scale = scale; p.drop = make_attn_drop(drop_p, seed, seed_dev);
     p.lse = const_cast<float *>(lse); p.o = o; p.dout = dout; p.dq = dq; p.dk = dk; p.dv = dv; p.dqkv_stride = dqkv_row_stride;
     p.dbias = dbias; p.accumulate = mode;
-    const size_t smem = ((size_t)4 * t_max_host * kPitch + 2 * (size_t)t_max_host) * sizeof(float);
-    MOBGT_CUDA_OK(cudaFuncSetAttribute(k3f_attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k3f_attn_bwd_kernel<<<B * H, kThreadsF, smem, static_cast<cudaStream_t>(stream)>>>(p);
+    const size_t smem = ((size_t)4 * t_max_host * (head_dim + 1) + 2 * (size_t)t_max_host) * sizeof(float);   // row pitch d + 1
+    auto kern = head_dim == 16 ? k3f_attn_bwd_kernel<16> : k3f_attn_bwd_kernel<24>;
+    MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<B * H, kThreadsF, smem, static_cast<cudaStream_t>(stream)>>>(p);
     MOBGT_LAUNCH_OK("k3f_attn_bwd_kernel");
     return MOBGT_OK;
+}
+
+extern "C" int32_t mobgt_attn_f32_fwd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
+                                      const int32_t *tok_off, int32_t B, int32_t H, int32_t ntok, int32_t T, int32_t Tp,
+                                      int32_t t_max_host, float scale, float drop_p, uint64_t seed, const void *seed_dev, float *out,
+                                      float *lse, void *stream) {
+    return mobgt_attn_f32_fwd_hd(q, k, v, qkv_row_stride, bias, tok_off, B, H, ntok, T, Tp, t_max_host, scale, drop_p, seed, seed_dev,
+                                 out, lse, 24, stream);
+}
+
+extern "C" int32_t mobgt_attn_f32_bwd(const float *q, const float *k, const float *v, int64_t qkv_row_stride, const float *bias,
+                                      const float *o, const float *dout, const float *lse, const int32_t *tok_off, int32_t B,
+                                      int32_t H, int32_t ntok, int32_t T, int32_t Tp, int32_t t_max_host, float scale, float *dq,
+                                      float *dk, float *dv, int64_t dqkv_row_stride, float *dbias, int32_t mode, float drop_p,
+                                      uint64_t seed, const void *seed_dev, void *stream) {
+    return mobgt_attn_f32_bwd_hd(q, k, v, qkv_row_stride, bias, o, dout, lse, tok_off, B, H, ntok, T, Tp, t_max_host, scale, dq, dk,
+                                 dv, dqkv_row_stride, dbias, mode, drop_p, seed, seed_dev, 24, stream);
 }

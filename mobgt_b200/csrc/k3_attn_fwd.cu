@@ -7,10 +7,12 @@
 // streamed by TMA, and the scores never touch HBM.
 //
 // One CTA per (graph, head); K and V of the graph stay resident in shared memory.
-//   S  = Q_i K_j^T      tcgen05.mma  M=128, N<=128, K=32 (d=24 zero-padded)      -> TMEM cols [0,128)
+//   S  = Q_i K_j^T      tcgen05.mma  M=128, N<=128, K=dp                          -> TMEM cols [0,128)
 //   P  = softmax tile   tcgen05.ld -> registers (+ bias tile from smem, online max/sum) -> bf16 -> smem
-//   O += P V_j          tcgen05.mma  M=128, N=32, K=kv                             -> TMEM cols [128,160)
-// Operands use the no-swizzle [chunk][row][8] layout of umma.cuh (3-D TMA boxes {8, 128 rows, 3 chunks});
+//   O += P V_j          tcgen05.mma  M=128, N=dp, K=kv                             -> TMEM cols [128,128+dp)
+// The head dim d is a template parameter, built for 24 (dp = 32: one zero K-padding chunk, two K=16 MMAs for S) and
+// 16 (dp = 16: no padding, one MMA for S); k3_small.cuh AttnShape.
+// Operands use the no-swizzle [chunk][row][8] layout of umma.cuh (3-D TMA boxes {8, 128 rows, d/8 chunks});
 // the bias tile is two {64 x 128} boxes with the 128-byte TMA swizzle.
 #include <cuda_bf16.h>
 
@@ -21,17 +23,13 @@
 namespace mobgt {
 using namespace sm100;
 
-constexpr int kAttD = 24;        // head dim (192 / 8); padded to 32 for the MMA K / N granularity
-constexpr int kAttChunks = 3;    // 24 / 8
 constexpr int kTile = 128;       // query rows per tile == KV rows per box
-constexpr int kBoxBytes = 4 * kTile * 16;        // [4 chunks][128 rows][16 B]; chunk 3 stays zero
-constexpr int kBoxTxBytes = kAttChunks * kTile * 16;
 constexpr int kBiasTileBytes = 2 * kTile * 128;  // two 64-column halves, 128 B per row
 constexpr int kPBytes = 16 * kTile * 16;         // [16 chunks][128 rows][16 B]
 
 struct AttnFwdParams {
     const int32_t *tok_off;  // [B+1]
-    __nv_bfloat16 *out;      // [Ntok, H*24]
+    __nv_bfloat16 *out;      // [Ntok, H*d]
     float *lse;              // [Ntok, H]
     int H;
     float scale;
@@ -47,13 +45,13 @@ struct AttnFwdParams {
     int n_items;                      // B * H work items; CTA b works on items b, b + gridDim.x, ... (persistent CTAs)
 };
 
-__device__ __forceinline__ void fwd_unpack24(const uint4 &a, const uint4 &b, const uint4 &c, float (&f)[24]) {
-    const uint32_t w[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+// the d bf16 of row `row` of a [chunk][row][8] operand box -> fp32
+template <int kD>
+__device__ __forceinline__ void fwd_box_row(const uint8_t *box, int row, float (&f)[kD]) {
+    uint4 w[kD / 8];
 #pragma unroll
-    for (int e = 0; e < 12; ++e) {
-        f[2 * e] = __uint_as_float(w[e] << 16);
-        f[2 * e + 1] = __uint_as_float(w[e] & 0xFFFF0000u);
-    }
+    for (int c = 0; c < kD / 8; ++c) w[c] = *reinterpret_cast<const uint4 *>(box + c * (kTile * 16) + row * 16);
+    unpack_words<kD / 8>(w, f);
 }
 
 __device__ __forceinline__ float fast_exp2(float x) {
@@ -74,7 +72,7 @@ __device__ __forceinline__ float fast_exp2(float x) {
 // Single-token tail ("fold"): a graph of 128 m + 1 tokens (n = 128 m nodes + the graph token) runs the MMA loop over its
 // m x m full tiles only; the last token sp = 128 m is handled by SIMT: its key column enters every row's online softmax as
 // one more (register) block in the tile epilogue, and its own query row is one block-wide softmax + a small mat-vec.
-template <bool kDrop>
+template <int kAttD, bool kDrop>
 __global__ void __launch_bounds__(256, 2)
 k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                    const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmBias,
@@ -86,8 +84,11 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     __shared__ float sTail[4 * kTile];          // fold: score (log2 units) of (row r, key sp)
     __shared__ float sTp[4 * kTile + 4];        // fold: kept probabilities of (row sp, key c)
     __shared__ float sSp[3][kAttD];             // fold: q, k, v of token sp
-    __shared__ float sRed[10][kAttD];
+    __shared__ float sRed[AttnShape<kAttD>::kSegs][kAttD];
     __shared__ float sScal[16];
+    using Sh = AttnShape<kAttD>;
+    constexpr int kAttChunks = Sh::kChunks, kDPad = Sh::kDPad, kBoxBytes = Sh::kBoxBytes, kBoxTxBytes = Sh::kBoxTxBytes;
+    constexpr int kSegs = Sh::kSegs;
 
     MOBGT_STAMP(p.timeline, 0);
     const int tid = threadIdx.x, warp = tid >> 5, wg = tid >> 7, t128 = tid & 127;
@@ -127,8 +128,8 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         tma_prefetch_desc(&tmV);
         tma_prefetch_desc(&tmBias);
     }
-    // zero the K-padding chunk (d = 24..31) of Q and of every K / V box: 128 rows x 16 B each
-    {
+    // zero the K-padding chunk (d = 24..31) of Q and of every K / V box: 128 rows x 16 B each (d = 16: no padding)
+    if (kDPad != kAttD) {
         const uint4 z = make_uint4(0, 0, 0, 0);
         if (wg == 0) *reinterpret_cast<uint4 *>(sQ + 3 * kTile * 16 + t128 * 16) = z;
         uint8_t *kv = wg == 0 ? sK : sV;
@@ -211,7 +212,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         const uint32_t idesc = make_idesc_bf16(kTile, nbj, 0, 0);
         const uint32_t aq = smem_u32(sQ), bk = smem_u32(sK + (size_t)j * kBoxBytes);
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks)
+        for (int ks = 0; ks < kDPad / 16; ++ks)
             umma_bf16(tS, make_smem_desc(aq + ks * 2 * kTile * 16, kTile * 16, 128),
                       make_smem_desc(bk + ks * 2 * kTile * 16, kTile * 16, 128), idesc, ks > 0);
         umma_commit(&bar_s);
@@ -234,14 +235,15 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         for (int u = 0; u < 2; ++u) {
             const int r = tid + u * 256;
             if (r >= sp) break;
-            float qf[24];
+            float qf[kAttD];
             if (r < kTile) {      // tile 0: from shared memory
-                const uint8_t *qb = sQ + r * 16;
-                fwd_unpack24(*reinterpret_cast<const uint4 *>(qb), *reinterpret_cast<const uint4 *>(qb + kTile * 16),
-                             *reinterpret_cast<const uint4 *>(qb + 2 * kTile * 16), qf);
+                fwd_box_row<kAttD>(sQ, r, qf);
             } else {
                 const uint4 *qg = reinterpret_cast<const uint4 *>(p.q + (size_t)(t0 + r) * p.qkv_stride + h * kAttD);
-                fwd_unpack24(qg[0], qg[1], qg[2], qf);
+                uint4 w[kAttChunks];
+#pragma unroll
+                for (int c = 0; c < kAttChunks; ++c) w[c] = qg[c];
+                unpack_words<kAttChunks>(w, qf);
             }
             float dot = 0.f;
 #pragma unroll
@@ -257,10 +259,8 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             if (c < Tg) {
                 float dot = 0.f;
                 if (c < sp) {
-                    const uint8_t *kb = sK + (size_t)(c >> 7) * kBoxBytes + (c & 127) * 16;
-                    float kf[24];
-                    fwd_unpack24(*reinterpret_cast<const uint4 *>(kb), *reinterpret_cast<const uint4 *>(kb + kTile * 16),
-                                 *reinterpret_cast<const uint4 *>(kb + 2 * kTile * 16), kf);
+                    float kf[kAttD];
+                    fwd_box_row<kAttD>(sK + (size_t)(c >> 7) * kBoxBytes, c & 127, kf);
 #pragma unroll
                     for (int e = 0; e < kAttD; ++e) dot = fmaf(sSp[0][e], kf[e], dot);
                 } else {
@@ -301,7 +301,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         if (tid < 240) {   // O[sp] = sum_c P[c] v_c : thread = (e, seg)
             const int seg = tid / kAttD, e = tid - seg * kAttD;
             float a = 0.f;
-            for (int c = seg; c < sp; c += 10) {
+            for (int c = seg; c < sp; c += kSegs) {
                 const __nv_bfloat16 *vb = reinterpret_cast<const __nv_bfloat16 *>(
                     sV + (size_t)(c >> 7) * kBoxBytes + (e >> 3) * (kTile * 16) + (c & 127) * 16) + (e & 7);
                 a = fmaf(sTp[c], __bfloat162float(*vb), a);
@@ -312,7 +312,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         if (tid < kAttD) {
             float a = sTp[sp] * sSp[2][tid];
 #pragma unroll
-            for (int sg = 0; sg < 10; ++sg) a += sRed[sg][tid];
+            for (int sg = 0; sg < kSegs; ++sg) a += sRed[sg][tid];
             p.out[(size_t)(t0 + sp) * (p.H * kAttD) + h * kAttD + tid] = __float2bfloat16_rn(a * (kDrop ? p.drop.inv_keep : 1.0f) / ls);
             if (tid == 0) p.lse[(size_t)(t0 + sp) * p.H + h] = (mx + log2f(ls)) * 0.6931471805599453f;
         }
@@ -426,7 +426,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             }
             l_run = l_run * alpha + l_blk;
             m_run = m_new;
-            if (j > 0 && warp_live) {   // rescale the running O accumulator (16 of the 32 columns per warpgroup)
+            if (j > 0 && warp_live && (kDPad == 32 || wg == 0)) {   // rescale the running O accumulator (columns [16 wg, 16 wg + 16))
                 uint32_t ov[16];
                 tmem_ld16(tO + lane_off + wg * 16, ov);
                 tmem_ld_wait();
@@ -442,7 +442,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             MOBGT_STAMP(p.timeline, 8 + 8 * (i * NB + j) + 5);   // barrier B passed
             if (warp0 && elect_one()) {
                 tc_fence_after();
-                const uint32_t idesc = make_idesc_bf16(kTile, 32, 0, 1);
+                const uint32_t idesc = make_idesc_bf16(kTile, kDPad, 0, 1);
                 const uint32_t ap = smem_u32(sP), bv = smem_u32(sV + (size_t)j * kBoxBytes);
                 for (int ks = 0; ks < nb / 16; ++ks)
                     umma_bf16(tO, make_smem_desc(ap + ks * 2 * kTile * 16, kTile * 16, 128),
@@ -452,7 +452,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             __syncwarp();
         }
         // ---- epilogue of the query tile: O / l -> bf16, lse.  The two warpgroups' shares of the row sum are exchanged
-        //      through sMax (free since the last barrier of the j loop); each warpgroup stores 16 of the 32 O columns.
+        //      through sMax (free since the last barrier of the j loop); warpgroup wg stores O columns [16 wg, 16 wg + 16) < d.
         sMax[wg][t128] = l_run;
         mbar_wait(&bar_o, ph_o);
         ph_o ^= 1;
@@ -461,7 +461,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         // shared memory is free: the next item's first loads start now and fly under this epilogue
         if (i + 1 == NB && tid == 0 && nxt.idx < p.n_items) load_item(nxt);
         __syncthreads();
-        if (warp_live) {
+        if (warp_live && (kAttD > 16 || wg == 0)) {
             uint32_t ov[16];
             tmem_ld16(tO + lane_off + wg * 16, ov);
             tmem_ld_wait();
@@ -477,7 +477,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
                     const float pd = kp ? pe : 0.f;
 #pragma unroll
                     for (int e = 0; e < 16; ++e)
-                        if (wg == 0 || e < 8)
+                        if (wg == 0 || e < kAttD - 16)
                             ov[e] = __float_as_uint(fmaf(__uint_as_float(ov[e]), al, pd * sSp[2][wg * 16 + e]));
                     m_run = m_new;
                 }
@@ -492,7 +492,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
                     dst[1] = make_uint4(w[4], w[5], w[6], w[7]);
                     p.lse[(size_t)(t0 + row) * p.H + h] = (m_run + log2f(l_tot)) * 0.6931471805599453f;
                 } else {
-                    dst[2] = make_uint4(w[0], w[1], w[2], w[3]);   // columns 16..23 (24..31 are the MMA padding)
+                    dst[2] = make_uint4(w[0], w[1], w[2], w[3]);   // d = 24: columns 16..23 (24..31 are the MMA padding)
                 }
             }
         }
@@ -514,12 +514,16 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 
 using namespace mobgt;
 
-// qkv: three bf16 matrices of [ntok, H*24] with a common row stride (elements); typically slices of one fused
-// [ntok, 3*H*24] projection.  bias: bf16 [B, H, T, Tp].  out: bf16 [ntok, H*24] (contiguous).  lse: f32 [ntok, H].
-extern "C" int32_t mobgt_attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
-                                  const int32_t *tok_off, const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok,
-                                  int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host, float scale, float drop_p, uint64_t seed,
-                                  const void *seed_dev, void *out, float *lse, void *stream) {
+namespace {
+// qkv: three bf16 matrices of [ntok, H*d] with a common row stride (elements); typically slices of one fused
+// [ntok, 3*H*d] projection.  bias: bf16 [B, H, T, Tp].  out: bf16 [ntok, H*d] (contiguous).  lse: f32 [ntok, H].
+template <int kAttD>
+int32_t attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                 const int32_t *tok_off, const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok,
+                 int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host, float scale, float drop_p, uint64_t seed,
+                 const void *seed_dev, void *out, float *lse, void *stream) {
+    using Sh = AttnShape<kAttD>;
+    constexpr int kAttChunks = Sh::kChunks, kBoxBytes = Sh::kBoxBytes;
     MOBGT_REQUIRE(q && k && v && bias && tok_off && out && lse, MOBGT_ERR_NULL, "mobgt_attn_fwd: null pointer");
     MOBGT_REQUIRE(H >= 1 && B >= 0 && ntok >= 0, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_fwd: B=%d H=%d ntok=%d", B, H, ntok);
     MOBGT_REQUIRE(qkv_row_stride % 8 == 0 && Tp % 8 == 0 && Tp >= T, MOBGT_ERR_BAD_SHAPE,
@@ -544,13 +548,13 @@ extern "C" int32_t mobgt_attn_fwd(const void *q, const void *k, const void *v, i
         sp.H = H; sp.T = T; sp.Tp = Tp; sp.scale = scale; sp.small_t = kSmallT;
         sp.drop = make_attn_drop(drop_p, seed, seed_dev);
         sp.out = static_cast<__nv_bfloat16 *>(out); sp.lse = lse;
-        if (!any_large) return launch_small_attn_fwd(sp, B, static_cast<cudaStream_t>(stream));
+        if (!any_large) return launch_small_attn_fwd<kAttD>(sp, B, static_cast<cudaStream_t>(stream));
         // both kernels: they work on disjoint graphs, so the SIMT one runs on a side stream next to the tensor-core one
         int32_t rc = get_fork_join(0, &fj);
         if (rc) return rc;
         MOBGT_CUDA_OK(cudaEventRecord(fj.fork, static_cast<cudaStream_t>(stream)));
         MOBGT_CUDA_OK(cudaStreamWaitEvent(fj.side, fj.fork, 0));
-        rc = launch_small_attn_fwd(sp, B, fj.side);
+        rc = launch_small_attn_fwd<kAttD>(sp, B, fj.side);
         MOBGT_CUDA_OK(cudaEventRecord(fj.join, fj.side));
         forked = true;
         if (rc) {
@@ -584,7 +588,7 @@ extern "C" int32_t mobgt_attn_fwd(const void *q, const void *k, const void *v, i
                     static_cast<const __nv_bfloat16 *>(q), static_cast<const __nv_bfloat16 *>(k),
                     static_cast<const __nv_bfloat16 *>(v), qkv_row_stride, static_cast<const __nv_bfloat16 *>(bias), T, Tp,
                     any_small ? kSmallT : 0, graph_order, B * H};
-    auto kern = p.drop.th16 ? k3_attn_fwd_kernel<true> : k3_attn_fwd_kernel<false>;
+    auto kern = p.drop.th16 ? k3_attn_fwd_kernel<kAttD, true> : k3_attn_fwd_kernel<kAttD, false>;
     MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = B * H < 2 * kNumSMs ? B * H : 2 * kNumSMs;     // persistent: two CTAs per SM, each loops over its items
     kern<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(tmQ, tmK, tmV, tmB, p);
@@ -594,4 +598,24 @@ extern "C" int32_t mobgt_attn_fwd(const void *q, const void *k, const void *v, i
     const int32_t rc = run_tensor_core();
     if (forked) cudaStreamWaitEvent(static_cast<cudaStream_t>(stream), fj.join, 0);   // join on every path
     return rc;
+}
+}  // namespace
+
+extern "C" int32_t mobgt_attn_fwd_hd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                                     const int32_t *tok_off, const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok,
+                                     int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host, float scale, float drop_p,
+                                     uint64_t seed, const void *seed_dev, void *out, float *lse, int32_t head_dim, void *stream) {
+    MOBGT_REQUIRE(head_dim == 16 || head_dim == 24, MOBGT_ERR_UNSUPPORTED,
+                  "mobgt_attn_fwd_hd: head_dim=%d is not built (head dims 16 and 24)", head_dim);
+    auto f = head_dim == 16 ? attn_fwd<16> : attn_fwd<24>;
+    return f(q, k, v, qkv_row_stride, bias, tok_off, graph_order, B, H, ntok, T, Tp, t_max_host, t_min_host, scale, drop_p, seed,
+             seed_dev, out, lse, stream);
+}
+
+extern "C" int32_t mobgt_attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_stride, const void *bias,
+                                  const int32_t *tok_off, const int32_t *graph_order, int32_t B, int32_t H, int32_t ntok,
+                                  int32_t T, int32_t Tp, int32_t t_max_host, int32_t t_min_host, float scale, float drop_p, uint64_t seed,
+                                  const void *seed_dev, void *out, float *lse, void *stream) {
+    return mobgt_attn_fwd_hd(q, k, v, qkv_row_stride, bias, tok_off, graph_order, B, H, ntok, T, Tp, t_max_host, t_min_host, scale,
+                             drop_p, seed, seed_dev, out, lse, 24, stream);
 }

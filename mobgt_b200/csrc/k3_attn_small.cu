@@ -27,7 +27,6 @@
 namespace mobgt {
 
 namespace {
-constexpr int kD = 24;
 constexpr float kL2e = 1.4426950408889634f;
 
 __device__ __forceinline__ float ex2(float x) {
@@ -47,8 +46,9 @@ __device__ __forceinline__ uint32_t pack2(float lo, float hi) {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t *>(&v);
 }
-__device__ __forceinline__ float dot24(const float (&a)[kD], const float *b) {   // b: shared memory, same address in every lane
-    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;     // four independent chains (a single one is 24 dependent FMAs)
+template <int kD>
+__device__ __forceinline__ float dotd(const float (&a)[kD], const float *b) {   // b: shared memory, same address in every lane
+    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;     // four independent chains (a single one is d dependent FMAs)
 #pragma unroll
     for (int e = 0; e < kD; e += 4) {
         const float4 v = *reinterpret_cast<const float4 *>(b + e);
@@ -59,7 +59,8 @@ __device__ __forceinline__ float dot24(const float (&a)[kD], const float *b) {  
     }
     return (s0 + s1) + (s2 + s3);
 }
-__device__ __forceinline__ void axpy24(float (&acc)[kD], float a, const float *b) {
+template <int kD>
+__device__ __forceinline__ void axpyd(float (&acc)[kD], float a, const float *b) {
 #pragma unroll
     for (int e = 0; e < kD; e += 4) {
         const float4 v = *reinterpret_cast<const float4 *>(b + e);
@@ -69,10 +70,11 @@ __device__ __forceinline__ void axpy24(float (&acc)[kD], float a, const float *b
         acc[e + 3] = fmaf(a, v.w, acc[e + 3]);
     }
 }
-__device__ __forceinline__ void store24(__nv_bfloat16 *dst, const float (&a)[kD], float scale) {
+template <int kD>
+__device__ __forceinline__ void stored(__nv_bfloat16 *dst, const float (&a)[kD], float scale) {
     uint4 *d = reinterpret_cast<uint4 *>(dst);
 #pragma unroll
-    for (int c = 0; c < 3; ++c)
+    for (int c = 0; c < kD / 8; ++c)
         d[c] = make_uint4(pack2(a[8 * c] * scale, a[8 * c + 1] * scale), pack2(a[8 * c + 2] * scale, a[8 * c + 3] * scale),
                           pack2(a[8 * c + 4] * scale, a[8 * c + 5] * scale), pack2(a[8 * c + 6] * scale, a[8 * c + 7] * scale));
 }
@@ -84,20 +86,26 @@ __device__ __forceinline__ void store24(__nv_bfloat16 *dst, const float (&a)[kD]
 constexpr int kHG = 4;                                   // heads per CTA
 constexpr int kRows = kSmallT;                           // 16
 constexpr int kThreads = kHG * kRows;
-// operand rows in shared memory: [head-in-group][row][24 floats] (+ 4 floats after every 8 rows): the four heads of a warp read
-// bank groups 8 apart, the rows of a warp read the same address (broadcast)
-__device__ __forceinline__ int row_off(int r) { return r * kD + (r >> 3) * 4; }
-constexpr int kOpFloats = kRows * kD + (kRows / 8) * 4;  // 392 = 8 (mod 32)
+// operand rows in shared memory: [head-in-group][row][d floats] (+ 4 floats after every 8 rows): the four heads of a warp read
+// bank groups 8 apart, the rows of a warp read the same address (broadcast).  A float4 read of a warp is served in phases of
+// 8 lanes = 2 rows x 4 heads, i.e. 4 distinct addresses h * kOpFloats + c: conflict-free when kOpFloats mod 32 puts the four
+// 4-bank windows apart.  Unpadded, 16 rows x d floats is a multiple of 32 for both head dims (384 and 256: all four heads on
+// the same banks); the 2 x 4 floats of padding make it 8 (mod 32) -> windows at banks 0, 8, 16, 24.
+template <int kD> __device__ __forceinline__ int row_off(int r) { return r * kD + (r >> 3) * 4; }
+template <int kD> constexpr int op_floats() { return kRows * kD + (kRows / 8) * 4; }
+static_assert(op_floats<24>() % 32 == 8 && op_floats<16>() % 32 == 8, "d = 24: 392 = 8 (mod 32); d = 16: 264 = 8 (mod 32)");
 constexpr int kBP = kRows + 8;                           // bias row pitch (bf16): 48 B, 8 consecutive rows hit distinct banks
 
-// rows [t0, t0 + Tg) x (4 heads x 24) bf16 of a [ntok, stride] matrix -> fp32 dst[head][row_off(row)]
+// rows [t0, t0 + Tg) x (4 heads x d) bf16 of a [ntok, stride] matrix -> fp32 dst[head][row_off(row)]
+template <int kD>
 __device__ __forceinline__ void stage_heads(const __nv_bfloat16 *src, int64_t stride, int t0, int Tg, int h0, float *dst, int nthr,
                                             int tid0 = -1) {
-    for (int i = tid0 < 0 ? (int)threadIdx.x : tid0; i < Tg * 12; i += nthr) {
-        const int r = i / 12, c = i - r * 12;            // 16-byte chunk c of the row's 192-byte slice: head c / 3, part c % 3
+    constexpr int kC = kD / 8, kRowC = kHG * kC;         // 16-byte chunks per head / per row slice of the four heads
+    for (int i = tid0 < 0 ? (int)threadIdx.x : tid0; i < Tg * kRowC; i += nthr) {
+        const int r = i / kRowC, c = i - r * kRowC;      // 16-byte chunk c of the row's 8 d-byte slice: head c / kC, part c % kC
         float f[8];
         unpack8(__ldg(reinterpret_cast<const uint4 *>(src + (size_t)(t0 + r) * stride + h0 * kD) + c), f);
-        float4 *d = reinterpret_cast<float4 *>(dst + (c / 3) * kOpFloats + row_off(r) + (c % 3) * 8);
+        float4 *d = reinterpret_cast<float4 *>(dst + (c / kC) * op_floats<kD>() + row_off<kD>(r) + (c % kC) * 8);
         d[0] = make_float4(f[0], f[1], f[2], f[3]);
         d[1] = make_float4(f[4], f[5], f[6], f[7]);
     }
@@ -114,8 +122,9 @@ __device__ __forceinline__ void stage_bias4(const __nv_bfloat16 *bias, int T, in
 }
 
 // ---------------------------------------------------------------------------------------------------------------- forward
-template <bool kDrop>
+template <int kD, bool kDrop>
 __global__ void __launch_bounds__(kThreads, 12) k3s_attn_fwd_kernel(const SmallAttnParams p) {
+    constexpr int kOpFloats = op_floats<kD>();
     __shared__ __align__(16) float sK[kHG * kOpFloats], sV[kHG * kOpFloats];
     __shared__ __align__(16) __nv_bfloat16 sB[kHG * kRows * kBP];
     const int ngrp = p.H / kHG;
@@ -128,8 +137,8 @@ __global__ void __launch_bounds__(kThreads, 12) k3s_attn_fwd_kernel(const SmallA
     if ((int)threadIdx.x >= nthr) return;
     const int h0 = hg * kHG, plane0 = g * p.H + h0;
     stage_bias4(p.bias, p.T, p.Tp, plane0, Tg, sB, nthr);
-    stage_heads(p.k, p.qkv_stride, t0, Tg, h0, sK, nthr);
-    stage_heads(p.v, p.qkv_stride, t0, Tg, h0, sV, nthr);
+    stage_heads<kD>(p.k, p.qkv_stride, t0, Tg, h0, sK, nthr);
+    stage_heads<kD>(p.v, p.qkv_stride, t0, Tg, h0, sV, nthr);
     const int r = threadIdx.x >> 2, hq = threadIdx.x & 3;
     const bool live = r < Tg;
     const int h = h0 + hq, plane = plane0 + hq;
@@ -138,7 +147,7 @@ __global__ void __launch_bounds__(kThreads, 12) k3s_attn_fwd_kernel(const SmallA
     if (live) {
         const uint4 *qg = reinterpret_cast<const uint4 *>(p.q + (size_t)(t0 + r) * p.qkv_stride + h * kD);
 #pragma unroll
-        for (int c = 0; c < 3; ++c) unpack8(__ldg(qg + c), q + 8 * c);
+        for (int c = 0; c < kD / 8; ++c) unpack8(__ldg(qg + c), q + 8 * c);
 #pragma unroll
         for (int e = 0; e < kD; ++e) q[e] *= sl2;
     }
@@ -162,7 +171,7 @@ __global__ void __launch_bounds__(kThreads, 12) k3s_attn_fwd_kernel(const SmallA
         for (int e = 0; e < 8; ++e) {
             s8[e] = -INFINITY;
             if (e < nv) {
-                s8[e] = fmaf(b8[e], kL2e, dot24(q, Kh + row_off(c8 * 8 + e)));
+                s8[e] = fmaf(b8[e], kL2e, dotd(q, Kh + row_off<kD>(c8 * 8 + e)));
                 mc = fmaxf(mc, s8[e]);
             }
         }
@@ -177,12 +186,12 @@ __global__ void __launch_bounds__(kThreads, 12) k3s_attn_fwd_kernel(const SmallA
             if (e < nv) {
                 const float pe = ex2(s8[e] - m_new);
                 l += pe;                               // the denominator is taken before the dropout mask
-                if ((keep >> e) & 1u) axpy24(o, pe, Vh + row_off(c8 * 8 + e));
+                if ((keep >> e) & 1u) axpyd(o, pe, Vh + row_off<kD>(c8 * 8 + e));
             }
         }
         m = m_new;
     }
-    store24(p.out + (size_t)(t0 + r) * (p.H * kD) + h * kD, o, (kDrop ? p.drop.inv_keep : 1.0f) / l);
+    stored(p.out + (size_t)(t0 + r) * (p.H * kD) + h * kD, o, (kDrop ? p.drop.inv_keep : 1.0f) / l);
     p.lse[(size_t)(t0 + r) * p.H + h] = (m + log2f(l)) * 0.6931471805599453f;
 }
 
@@ -193,8 +202,9 @@ __global__ void __launch_bounds__(kThreads, 12) k3s_attn_fwd_kernel(const SmallA
 // The two passes read the same staged operands and write disjoint outputs, so they run SIDE BY SIDE: threads [0, 64) take
 // pass 1, threads [64, 128) pass 2 — the kernel is bound by the dependent-instruction chain of its largest graph, and the
 // chain is now the longer of the two passes instead of their sum.
-template <bool kDrop>
+template <int kD, bool kDrop>
 __global__ void __launch_bounds__(2 * kThreads, 4) k3s_attn_bwd_kernel(const SmallAttnParams p) {
+    constexpr int kOpFloats = op_floats<kD>();
     __shared__ __align__(16) float sQ[kHG * kOpFloats], sK[kHG * kOpFloats], sV[kHG * kOpFloats], sdO[kHG * kOpFloats];
     __shared__ float sLse[kHG * kRows], sDel[kHG * kRows];
     __shared__ __align__(16) __nv_bfloat16 sB[kHG * kRows * kBP];
@@ -211,10 +221,10 @@ __global__ void __launch_bounds__(2 * kThreads, 4) k3s_attn_bwd_kernel(const Sma
     const int h0 = hg * kHG, plane0 = g * p.H + h0;
     const int HD = p.H * kD;
     stage_bias4(p.bias, p.T, p.Tp, plane0, Tg, sB, nthr, sid);
-    stage_heads(p.q, p.qkv_stride, t0, Tg, h0, sQ, nthr, sid);
-    stage_heads(p.k, p.qkv_stride, t0, Tg, h0, sK, nthr, sid);
-    stage_heads(p.v, p.qkv_stride, t0, Tg, h0, sV, nthr, sid);
-    stage_heads(p.dout, HD, t0, Tg, h0, sdO, nthr, sid);
+    stage_heads<kD>(p.q, p.qkv_stride, t0, Tg, h0, sQ, nthr, sid);
+    stage_heads<kD>(p.k, p.qkv_stride, t0, Tg, h0, sK, nthr, sid);
+    stage_heads<kD>(p.v, p.qkv_stride, t0, Tg, h0, sV, nthr, sid);
+    stage_heads<kD>(p.dout, HD, t0, Tg, h0, sdO, nthr, sid);
     const int t = lt >> 2, hq = lt & 3;
     const bool live = t < Tg;
     const int h = h0 + hq, plane = plane0 + hq;
@@ -227,7 +237,7 @@ __global__ void __launch_bounds__(2 * kThreads, 4) k3s_attn_bwd_kernel(const Sma
         const uint4 *dg = reinterpret_cast<const uint4 *>(p.dout + (size_t)(t0 + t) * HD + h * kD);
         float d = 0.f;
 #pragma unroll
-        for (int c = 0; c < 3; ++c) {
+        for (int c = 0; c < kD / 8; ++c) {
             float a[8], b[8];
             unpack8(__ldg(og + c), a);
             unpack8(__ldg(dg + c), b);
@@ -248,8 +258,8 @@ __global__ void __launch_bounds__(2 * kThreads, 4) k3s_attn_bwd_kernel(const Sma
         float q[kD], dO[kD], dq[kD];
 #pragma unroll
         for (int e = 0; e < kD; ++e) {
-            q[e] = Qh[row_off(t) + e] * sl2;
-            dO[e] = dOh[row_off(t) + e];
+            q[e] = Qh[row_off<kD>(t) + e] * sl2;
+            dO[e] = dOh[row_off<kD>(t) + e];
             dq[e] = 0.f;
         }
         const float lse2 = Lh[t], del = Dh[t];
@@ -264,11 +274,11 @@ __global__ void __launch_bounds__(2 * kThreads, 4) k3s_attn_bwd_kernel(const Sma
             for (int e = 0; e < 8; ++e) {
                 ds8[e] = 0.f;
                 if (e < nv) {
-                    const float *kc = Kh + row_off(c8 * 8 + e);
-                    const float pr = ex2(fmaf(b8[e], kL2e, dot24(q, kc)) - lse2);
-                    const float dp = ((keep >> e) & 1u) ? dot24(dO, Vh + row_off(c8 * 8 + e)) * ik : 0.f;
+                    const float *kc = Kh + row_off<kD>(c8 * 8 + e);
+                    const float pr = ex2(fmaf(b8[e], kL2e, dotd(q, kc)) - lse2);
+                    const float dp = ((keep >> e) & 1u) ? dotd(dO, Vh + row_off<kD>(c8 * 8 + e)) * ik : 0.f;
                     ds8[e] = pr * (dp - del);
-                    axpy24(dq, ds8[e], kc);
+                    axpyd(dq, ds8[e], kc);
                 }
             }
             const size_t o = pl + (size_t)t * p.Tp + c8 * 8;
@@ -282,50 +292,57 @@ __global__ void __launch_bounds__(2 * kThreads, 4) k3s_attn_bwd_kernel(const Sma
                     if (e < nv) d32[e] = (p.accumulate == 1 ? d32[e] : 0.f) + ds8[e];
             }
         }
-        store24(p.dq + (size_t)(t0 + t) * p.dqkv_stride + h * kD, dq, p.scale);
+        stored(p.dq + (size_t)(t0 + t) * p.dqkv_stride + h * kD, dq, p.scale);
     }
     // ---- pass 2: column t
     else {
         float k[kD], v[kD], dk[kD], dv[kD];
 #pragma unroll
         for (int e = 0; e < kD; ++e) {
-            k[e] = Kh[row_off(t) + e] * sl2;
-            v[e] = Vh[row_off(t) + e];
+            k[e] = Kh[row_off<kD>(t) + e] * sl2;
+            v[e] = Vh[row_off<kD>(t) + e];
             dk[e] = dv[e] = 0.f;
         }
         const __nv_bfloat16 *bcol = sB + hq * kRows * kBP + t;
         for (int r = 0; r < Tg; ++r) {
-            const float *qr = Qh + row_off(r), *dor = dOh + row_off(r);
-            const float pr = ex2(fmaf(__bfloat162float(bcol[r * kBP]), kL2e, dot24(k, qr)) - Lh[r]);
+            const float *qr = Qh + row_off<kD>(r), *dor = dOh + row_off<kD>(r);
+            const float pr = ex2(fmaf(__bfloat162float(bcol[r * kBP]), kL2e, dotd(k, qr)) - Lh[r]);
             bool kp = true;
             if (kDrop) {
                 const uint32_t rowkey = attn_drop_rowkey((uint32_t)plane, (uint32_t)r, seed_lo, seed_hi);
                 kp = (attn_drop_keep8(rowkey, (uint32_t)(t >> 3), p.drop.th16) >> (t & 7)) & 1u;
             }
             const float pd = kp ? pr * ik : 0.f;
-            const float ds = pr * ((kp ? dot24(v, dor) * ik : 0.f) - Dh[r]);
-            axpy24(dk, ds, qr);
-            axpy24(dv, pd, dor);
+            const float ds = pr * ((kp ? dotd(v, dor) * ik : 0.f) - Dh[r]);
+            axpyd(dk, ds, qr);
+            axpyd(dv, pd, dor);
         }
-        store24(p.dk + (size_t)(t0 + t) * p.dqkv_stride + h * kD, dk, p.scale);
-        store24(p.dv + (size_t)(t0 + t) * p.dqkv_stride + h * kD, dv, 1.0f);
+        stored(p.dk + (size_t)(t0 + t) * p.dqkv_stride + h * kD, dk, p.scale);
+        stored(p.dv + (size_t)(t0 + t) * p.dqkv_stride + h * kD, dv, 1.0f);
     }
 }
 
+template <int kD>
 int32_t launch_small_attn_fwd(const SmallAttnParams &p, int B, cudaStream_t s) {
     const int grid = B * (p.H / kHG);
-    if (p.drop.th16) k3s_attn_fwd_kernel<true><<<grid, kThreads, 0, s>>>(p);
-    else k3s_attn_fwd_kernel<false><<<grid, kThreads, 0, s>>>(p);
+    if (p.drop.th16) k3s_attn_fwd_kernel<kD, true><<<grid, kThreads, 0, s>>>(p);
+    else k3s_attn_fwd_kernel<kD, false><<<grid, kThreads, 0, s>>>(p);
     MOBGT_LAUNCH_OK("k3s_attn_fwd_kernel");
     return MOBGT_OK;
 }
 
+template <int kD>
 int32_t launch_small_attn_bwd(const SmallAttnParams &p, int B, cudaStream_t s) {
     const int grid = B * (p.H / kHG);
-    if (p.drop.th16) k3s_attn_bwd_kernel<true><<<grid, 2 * kThreads, 0, s>>>(p);
-    else k3s_attn_bwd_kernel<false><<<grid, 2 * kThreads, 0, s>>>(p);
+    if (p.drop.th16) k3s_attn_bwd_kernel<kD, true><<<grid, 2 * kThreads, 0, s>>>(p);
+    else k3s_attn_bwd_kernel<kD, false><<<grid, 2 * kThreads, 0, s>>>(p);
     MOBGT_LAUNCH_OK("k3s_attn_bwd_kernel");
     return MOBGT_OK;
 }
+
+template int32_t launch_small_attn_fwd<16>(const SmallAttnParams &, int, cudaStream_t);
+template int32_t launch_small_attn_fwd<24>(const SmallAttnParams &, int, cudaStream_t);
+template int32_t launch_small_attn_bwd<16>(const SmallAttnParams &, int, cudaStream_t);
+template int32_t launch_small_attn_bwd<24>(const SmallAttnParams &, int, cudaStream_t);
 
 }  // namespace mobgt

@@ -202,6 +202,7 @@ def cli_main(argv=None):
                 break
         result["loss"] = float(loss) if loss is not None else None
         result["steps"] = tr.step_count
+        result["graph_steps"] = tr.graph_steps
         if rank == 0:
             print(f"trained {tr.step_count} steps: {tr.graph_steps} CUDA-graph replays, {tr.eager_steps} eager ({tr.graph_note})")
     if own_pg:

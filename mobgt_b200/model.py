@@ -23,6 +23,8 @@ from . import ops
 from .lr import PolynomialDecayLR
 
 NODE_DIM = 2000    # model_fqandtoyo.py:567
+# (num_heads, hidden_dim) pairs the kernels are built for: K2 is built for 8 heads, K3 for head dims (hidden_dim + 64) / 8 = 16, 24
+SUPPORTED_SHAPES = frozenset({(8, 64), (8, 128)})
 
 DATASET_TRAITS = {
     # per-dataset constructor differences (model_fqandtoyo.py:636-779, 781-900, 902-1029)
@@ -190,7 +192,8 @@ class MultiHeadAttention(nn.Module):
             wo = bo = None
         qkv = ops.LinearBiasFn.apply(x16, wq, bq, q.weight, k.weight, v.weight, q.bias, k.bias, v.bias)
         # attention output BEFORE output_layer: the caller fuses that Linear with the residual block (ops.LinearAddDropoutLNFn)
-        return ops.BiasedAttention.apply(qkv, bias_slot, layer, self.attention_dropout_rate if self.training else 0.0), wo, bo   # :1704
+        return ops.BiasedAttention.apply(qkv, bias_slot, layer, self.attention_dropout_rate if self.training else 0.0,
+                                         self.scale), wo, bo   # :1704
 
 
 class EncoderLayer(nn.Module):
@@ -224,7 +227,7 @@ class EncoderLayer(nn.Module):
         wq = torch.cat([a.linear_q.weight, a.linear_k.weight, a.linear_v.weight], 0)
         bq = torch.cat([a.linear_q.bias, a.linear_k.bias, a.linear_v.bias], 0)
         y = ops.BiasedAttentionF32.apply(F.linear(x, wq, bq), bias_slot, layer,
-                                         a.attention_dropout_rate if self.training else 0.0)             # :1693-1706
+                                         a.attention_dropout_rate if self.training else 0.0, a.scale)    # :1693-1706
         x = x + self.self_attention_dropout(a.output_layer(y))                                           # :1708, :1731-1735
         x = x + self.ffn_dropout(self.ffn(ops.layer_norm(x, self.ffn_norm1)))                            # :1737-1740
         return ops.layer_norm(x, self.ffn_norm2)                                                         # :1741
@@ -260,8 +263,12 @@ class Graphormer(nn.Module):
                              "model_fqandtoyo.py:791-832)")
         if dataset_name not in DATASET_TRAITS:
             raise NotImplementedError(f"dataset_name={dataset_name!r}: only the POI graph datasets are on the MobGT hot path")
-        if num_heads != ops.NUM_HEADS or (hidden_dim + 64) // num_heads != ops.HEAD_DIM:
-            raise NotImplementedError("libmobgt is built for the canonical MobGT shape: 8 heads, hidden 128 (+64) -> head dim 24")
+        if (num_heads, hidden_dim) not in SUPPORTED_SHAPES or (hidden_dim + 64) % num_heads:
+            raise NotImplementedError(
+                f"num_heads={num_heads}, hidden_dim={hidden_dim}: libmobgt is built for (num_heads, hidden_dim) in "
+                f"{sorted(SUPPORTED_SHAPES)}. The encoder width is hidden_dim + 64 (time and category embeddings), split over the "
+                f"heads: the attention-bias kernels (K2) are built for 8 heads, and the attention kernels (K3) for head dims "
+                f"{ops.HEAD_DIMS[0]} and {ops.HEAD_DIMS[1]}, i.e. hidden_dim 64 or 128 at 8 heads.")
         if edge_type != "multi_hop":
             raise NotImplementedError("edge_type must be 'multi_hop' (README.md:62)")
         tr = DATASET_TRAITS[dataset_name]
@@ -348,7 +355,7 @@ class Graphormer(nn.Module):
                                   self.edge_dis_encoder.weight, self.graph_token_virtual_distance.weight, dtype)
 
     def node_tokens(self, b, dtype=torch.bfloat16):
-        """K4 (model_fqandtoyo.py:1222-1344) -> packed tokens [ntok, 192]"""
+        """K4 (model_fqandtoyo.py:1222-1344) -> packed tokens [ntok, hidden_dim + 64]"""
         Gd, Gc = self.gcn_tables()
         e = ops.EmbedGather.apply(b, self.cat_of_poi, Gd, self.time_embed_model_48.weight, Gc, dtype, self.traits["time_pad"])
         hp = self.hidden_dim + self.time_embed_dim

@@ -9,7 +9,8 @@ from . import _C
 
 F32, BF16 = 0, 1
 NUM_HEADS = 8
-HEAD_DIM = 24
+HEAD_DIM = 24            # the canonical shape's head dim (hidden 128: (128 + 64) / 8)
+HEAD_DIMS = (16, 24)     # head dims the attention kernels are built for (csrc/k3_small.cuh AttnShape)
 
 
 def _dt(t):
@@ -110,40 +111,50 @@ def _t_min(batch):
     return int(min(batch.n_host)) + 1 if all_large(batch) else 0
 
 
+def _head_dim(qkv, H):
+    """Head dim of a fused [ntok, 3*H*d] projection."""
+    d, r = divmod(qkv.shape[1], 3 * H)
+    assert r == 0, f"qkv width {qkv.shape[1]} is not 3 * H * d for H={H}"
+    return d
+
+
 def attn_fwd_raw(qkv, bias, batch, scale=None, drop_p=0.0, seed=0):
-    """qkv bf16 [ntok, 3*H*24] (fused projection) ; bias bf16 [B,H,T,Tp] -> (out bf16 [ntok, H*24], lse f32 [ntok,H]).
+    """qkv bf16 [ntok, 3*H*d] (fused projection) ; bias bf16 [B,H,T,Tp] -> (out bf16 [ntok, H*d], lse f32 [ntok,H]).
+    The head dim d comes from the qkv width (built: 16, 24); scale defaults to d ** -0.5.
     drop_p > 0: attention dropout on the probabilities (model_fqandtoyo.py:1704), mask = hash(seed, plane, row, col)."""
     ntok = qkv.shape[0]
     B, H, T, Tp = bias.shape
-    D = H * HEAD_DIM
-    assert qkv.dtype == torch.bfloat16 and bias.dtype == torch.bfloat16 and qkv.shape[1] == 3 * D and qkv.is_contiguous()
+    hd = _head_dim(qkv, H)
+    D = H * hd
+    assert qkv.dtype == torch.bfloat16 and bias.dtype == torch.bfloat16 and qkv.is_contiguous()
     # a bucketed batch carries padding token rows no graph owns: the kernels never touch them, and they must hold finite values
     # (they flow through the row-wise layers and meet their zero gradients in the weight-gradient GEMMs)
     alloc = torch.zeros if getattr(batch, "padded", False) else torch.empty
     out = alloc(ntok, D, dtype=torch.bfloat16, device=qkv.device)
     lse = alloc(ntok, H, dtype=torch.float32, device=qkv.device)
-    scale = float(HEAD_DIM ** -0.5) if scale is None else float(scale)
+    scale = float(hd ** -0.5) if scale is None else float(scale)
     base = qkv.data_ptr()
-    _C.call("mobgt_attn_fwd", base, base + 2 * D, base + 4 * D, 3 * D, _C.ptr(bias), _C.ptr(batch.tok_off), _C.ptr(getattr(batch, "size_order", None)), B, H,
+    _C.call("mobgt_attn_fwd_hd", base, base + 2 * D, base + 4 * D, 3 * D, _C.ptr(bias), _C.ptr(batch.tok_off), _C.ptr(getattr(batch, "size_order", None)), B, H,
             ntok, T, Tp, int(batch.N) + 1, _t_min(batch), scale, float(drop_p), int(seed), _C.ptr(_seed_dev) if drop_p > 0 else None, _C.ptr(out),
-            _C.ptr(lse), _C.stream_ptr())
+            _C.ptr(lse), hd, _C.stream_ptr())
     return out, lse
 
 
 def attn_bwd_raw(qkv, bias, out, dout, lse, batch, dbias, accumulate, scale=None, drop_p=0.0, seed=0):
-    """-> dqkv bf16 [ntok, 3*H*24]; dbias [B,H,T,Tp] is written in place: f32 overwritten (accumulate=0) / added to
+    """-> dqkv bf16 [ntok, 3*H*d]; dbias [B,H,T,Tp] is written in place: f32 overwritten (accumulate=0) / added to
     (accumulate=1), or bf16 overwritten (accumulate=2: this layer's own dS plane, TMA-stored)."""
     ntok = qkv.shape[0]
     B, H, T, Tp = bias.shape
-    D = H * HEAD_DIM
+    hd = _head_dim(qkv, H)
+    D = H * hd
     assert dout.is_contiguous() and out.is_contiguous() and dbias.shape == bias.shape and dbias.is_contiguous()
     assert dbias.dtype == (torch.bfloat16 if accumulate == 2 else torch.float32)
     dqkv = torch.zeros_like(qkv) if getattr(batch, "padded", False) else torch.empty_like(qkv)    # padding rows: zero gradient
-    scale = float(HEAD_DIM ** -0.5) if scale is None else float(scale)
+    scale = float(hd ** -0.5) if scale is None else float(scale)
     base, dbase = qkv.data_ptr(), dqkv.data_ptr()
-    _C.call("mobgt_attn_bwd", base, base + 2 * D, base + 4 * D, 3 * D, _C.ptr(bias), _C.ptr(out), _C.ptr(dout), _C.ptr(lse),
+    _C.call("mobgt_attn_bwd_hd", base, base + 2 * D, base + 4 * D, 3 * D, _C.ptr(bias), _C.ptr(out), _C.ptr(dout), _C.ptr(lse),
             _C.ptr(batch.tok_off), _C.ptr(getattr(batch, "size_order", None)), B, H, ntok, T, Tp, int(batch.N) + 1, _t_min(batch), scale, dbase, dbase + 2 * D, dbase + 4 * D, 3 * D,
-            _C.ptr(dbias), int(accumulate), float(drop_p), int(seed), _C.ptr(_seed_dev) if drop_p > 0 else None, _C.stream_ptr())
+            _C.ptr(dbias), int(accumulate), float(drop_p), int(seed), _C.ptr(_seed_dev) if drop_p > 0 else None, hd, _C.stream_ptr())
     return dqkv
 
 
@@ -155,12 +166,13 @@ class BiasedAttention(torch.autograd.Function):
     w.r.t. the bias tables is produced once, by BiasLink below, where mobgt_bias_bwd sums the planes in fp32."""
 
     @staticmethod
-    def forward(ctx, qkv, bias_slot, layer, drop_p=0.0):
-        """drop_p: the attention dropout rate when training (`att_dropout`, model_fqandtoyo.py:1674, 1704), else 0."""
+    def forward(ctx, qkv, bias_slot, layer, drop_p=0.0, scale=None):
+        """drop_p: the attention dropout rate when training (`att_dropout`, model_fqandtoyo.py:1674, 1704), else 0.
+        scale: MultiHeadAttention.scale (att_size ** -0.5); None: head dim ** -0.5."""
         seed = _next_drop_seed() if drop_p > 0 else 0
-        out, lse = attn_fwd_raw(qkv, bias_slot.bias, bias_slot.batch, drop_p=drop_p, seed=seed)
+        out, lse = attn_fwd_raw(qkv, bias_slot.bias, bias_slot.batch, scale=scale, drop_p=drop_p, seed=seed)
         ctx.save_for_backward(qkv, out, lse)
-        ctx.slot, ctx.layer, ctx.drop = bias_slot, layer, (drop_p, seed)
+        ctx.slot, ctx.layer, ctx.drop, ctx.scale = bias_slot, layer, (drop_p, seed), scale
         return out
 
     @staticmethod
@@ -170,41 +182,43 @@ class BiasedAttention(torch.autograd.Function):
         if slot.planes is None:
             slot.planes = torch.empty((slot.n_layers,) + tuple(slot.bias.shape), dtype=torch.bfloat16, device=qkv.device)
             slot.written = set()
-        dqkv = attn_bwd_raw(qkv, slot.bias, out, dout.contiguous(), lse, slot.batch, slot.planes[ctx.layer], 2,
+        dqkv = attn_bwd_raw(qkv, slot.bias, out, dout.contiguous(), lse, slot.batch, slot.planes[ctx.layer], 2, scale=ctx.scale,
                             drop_p=ctx.drop[0], seed=ctx.drop[1])
         slot.written.add(ctx.layer)
-        return dqkv, None, None, None
+        return dqkv, None, None, None, None
 
 
 def attn_f32_fwd_raw(qkv, bias, batch, scale=None, drop_p=0.0, seed=0):
-    """fp32 mode of K3 (csrc/k3_attn_f32.cu): qkv f32 [ntok, 3*H*24], bias f32 [B,H,T,Tp] -> (out f32 [ntok, H*24], lse f32 [ntok,H])."""
+    """fp32 mode of K3 (csrc/k3_attn_f32.cu): qkv f32 [ntok, 3*H*d], bias f32 [B,H,T,Tp] -> (out f32 [ntok, H*d], lse f32 [ntok,H])."""
     ntok = qkv.shape[0]
     B, H, T, Tp = bias.shape
-    D = H * HEAD_DIM
-    assert qkv.dtype == torch.float32 and bias.dtype == torch.float32 and qkv.shape[1] == 3 * D and qkv.is_contiguous()
+    hd = _head_dim(qkv, H)
+    D = H * hd
+    assert qkv.dtype == torch.float32 and bias.dtype == torch.float32 and qkv.is_contiguous()
     alloc = torch.zeros if getattr(batch, "padded", False) else torch.empty
     out = alloc(ntok, D, dtype=torch.float32, device=qkv.device)
     lse = alloc(ntok, H, dtype=torch.float32, device=qkv.device)
-    scale = float(HEAD_DIM ** -0.5) if scale is None else float(scale)
+    scale = float(hd ** -0.5) if scale is None else float(scale)
     base = qkv.data_ptr()
-    _C.call("mobgt_attn_f32_fwd", base, base + 4 * D, base + 8 * D, 3 * D, _C.ptr(bias), _C.ptr(batch.tok_off), B, H, ntok, T, Tp,
+    _C.call("mobgt_attn_f32_fwd_hd", base, base + 4 * D, base + 8 * D, 3 * D, _C.ptr(bias), _C.ptr(batch.tok_off), B, H, ntok, T, Tp,
             int(batch.N) + 1, scale, float(drop_p), int(seed), _C.ptr(_seed_dev) if drop_p > 0 else None, _C.ptr(out), _C.ptr(lse),
-            _C.stream_ptr())
+            hd, _C.stream_ptr())
     return out, lse
 
 
 def attn_f32_bwd_raw(qkv, bias, out, dout, lse, batch, dbias, accumulate, scale=None, drop_p=0.0, seed=0):
-    """-> dqkv f32 [ntok, 3*H*24]; dbias f32 [B,H,T,Tp] overwritten (accumulate=0) or added to (accumulate=1), live cells only."""
+    """-> dqkv f32 [ntok, 3*H*d]; dbias f32 [B,H,T,Tp] overwritten (accumulate=0) or added to (accumulate=1), live cells only."""
     B, H, T, Tp = bias.shape
-    D = H * HEAD_DIM
+    hd = _head_dim(qkv, H)
+    D = H * hd
     assert dout.is_contiguous() and out.is_contiguous() and dbias.shape == bias.shape and dbias.is_contiguous()
     assert dbias.dtype == torch.float32 and dout.dtype == torch.float32 and accumulate in (0, 1)
     dqkv = torch.zeros_like(qkv) if getattr(batch, "padded", False) else torch.empty_like(qkv)
-    scale = float(HEAD_DIM ** -0.5) if scale is None else float(scale)
+    scale = float(hd ** -0.5) if scale is None else float(scale)
     base, dbase = qkv.data_ptr(), dqkv.data_ptr()
-    _C.call("mobgt_attn_f32_bwd", base, base + 4 * D, base + 8 * D, 3 * D, _C.ptr(bias), _C.ptr(out), _C.ptr(dout), _C.ptr(lse),
+    _C.call("mobgt_attn_f32_bwd_hd", base, base + 4 * D, base + 8 * D, 3 * D, _C.ptr(bias), _C.ptr(out), _C.ptr(dout), _C.ptr(lse),
             _C.ptr(batch.tok_off), B, H, qkv.shape[0], T, Tp, int(batch.N) + 1, scale, dbase, dbase + 4 * D, dbase + 8 * D, 3 * D,
-            _C.ptr(dbias), int(accumulate), float(drop_p), int(seed), _C.ptr(_seed_dev) if drop_p > 0 else None, _C.stream_ptr())
+            _C.ptr(dbias), int(accumulate), float(drop_p), int(seed), _C.ptr(_seed_dev) if drop_p > 0 else None, hd, _C.stream_ptr())
     return dqkv
 
 
@@ -214,11 +228,11 @@ class BiasedAttentionF32(torch.autograd.Function):
     sum has a fixed order); BiasLink hands it to mobgt_bias_bwd."""
 
     @staticmethod
-    def forward(ctx, qkv, bias_slot, layer, drop_p=0.0):
+    def forward(ctx, qkv, bias_slot, layer, drop_p=0.0, scale=None):
         seed = _next_drop_seed() if drop_p > 0 else 0
-        out, lse = attn_f32_fwd_raw(qkv, bias_slot.bias, bias_slot.batch, drop_p=drop_p, seed=seed)
+        out, lse = attn_f32_fwd_raw(qkv, bias_slot.bias, bias_slot.batch, scale=scale, drop_p=drop_p, seed=seed)
         ctx.save_for_backward(qkv, out, lse)
-        ctx.slot, ctx.layer, ctx.drop = bias_slot, layer, (drop_p, seed)
+        ctx.slot, ctx.layer, ctx.drop, ctx.scale = bias_slot, layer, (drop_p, seed), scale
         return out
 
     @staticmethod
@@ -227,10 +241,10 @@ class BiasedAttentionF32(torch.autograd.Function):
         slot = ctx.slot
         if slot.planes is None:
             slot.planes = torch.zeros_like(slot.bias)
-        dqkv = attn_f32_bwd_raw(qkv, slot.bias, out, dout.contiguous(), lse, slot.batch, slot.planes, 1, drop_p=ctx.drop[0],
-                                seed=ctx.drop[1])
+        dqkv = attn_f32_bwd_raw(qkv, slot.bias, out, dout.contiguous(), lse, slot.batch, slot.planes, 1, scale=ctx.scale,
+                                drop_p=ctx.drop[0], seed=ctx.drop[1])
         slot.written.add(ctx.layer)
-        return dqkv, None, None, None
+        return dqkv, None, None, None, None
 
 
 class BiasSlot:
@@ -587,7 +601,7 @@ def gemm_bf16(a, w, bias=None, mode=0, a2=None, w2=None, want_colsum=False, cols
 class FfnBlockFn(torch.autograd.Function):
     """FeedForwardNetwork + the residual block behind it (model_fqandtoyo.py:1644-1656, 1737-1741) as ONE autograd node:
         a = gelu(x W1^T + b1)            K10 mode 1: GEMM + bias + GELU in one kernel, the pre-activation never reaches HBM
-        y = a W2^T + b2                  library GEMM (192 output columns)
+        y = a W2^T + b2                  library GEMM (hidden output columns: 192 or 128)
         s = resid + dropout(y) ; out = LayerNorm(s)                                   K6
     backward:
         (dres, dy, dgamma, dbeta, db2)   K6 LayerNorm backward, db2 = column sums of dy from the same pass
@@ -597,7 +611,7 @@ class FfnBlockFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x16, w1, w2, b2, resid, gamma, beta, eps, p, want, need_s, m_w1, m_b1, m_w2, m_b2):
         a = gemm_bf16(x16, w1, m_b1, mode=1)
-        y = torch.nn.functional.linear(a, w2, b2)            # N = hidden (192): below K10's 128-column tile granularity
+        y = torch.nn.functional.linear(a, w2, b2)            # N = encoder width (192, or 128 at hidden_dim 64): library GEMM
         s, out, out16, saved, seed = _adln_fwd(resid, y, gamma, beta, eps, p, want)
         ctx.save_for_backward(x16, w1, w2, a, *saved)
         ctx.cfg = (float(p), seed, want, need_s)

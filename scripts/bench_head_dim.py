@@ -1,0 +1,137 @@
+"""Head dim 16 against head dim 24: the canonical 6-layer model (ffn 1024, 8 heads) at hidden_dim 128 (d = 24) and at hidden_dim 64
+(d = 16), on the c2-dense128 and c2-natural batches of bench.py (256 graphs, toyotagraph-shaped world of 60 000 POIs).
+
+    python scripts/bench_head_dim.py OUT_DIR [--steps 20] [--warmup 5] [--iters 20]
+
+For every (workload, hidden_dim) it reports, as OUT_DIR/bench_head_dim.json (one JSON object) and one line per case on stdout:
+  * step: ms / step and graphs / s of the replayed training step (trainer.Trainer with CUDA graphs, as bench.py times it);
+  * k3: one layer's attention forward and backward (mode 2: the per-layer bf16 dS plane the training step writes), dropout on
+    (p = 0.1), CUDA events around each launch with the L2 overwritten (a 256 MB buffer zeroed) before it; mean ms over --iters;
+  * bytes: what one K3 launch must move at these shapes (the live bias cells and q / k / v / out / lse, plus dout / o / dq / dk /
+    dv and the dS plane in the backward), and the resulting GB/s;
+  * the card's name and power limit, read in the same run.
+The numbers are only meaningful with a GPU: without one the script stops."""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
+
+import bench  # noqa: E402  (the workloads, the canonical hyper-parameters and the kernel timer of bench.py)
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True).stdout.strip().splitlines()
+    name, plim, clk = [s.strip() for s in q[0].split(",")] if q else (torch.cuda.get_device_name(0), "unknown", "unknown")
+    return dict(name=name, power_limit=plim, max_sm_clock=clk, torch_name=torch.cuda.get_device_name(0))
+
+
+def k3_bytes(batch, d, H=8):
+    """bytes one attention launch must read and write at this batch: live bias cells (bf16) + q, k, v (bf16) + out (bf16) + lse
+    (fp32) forward; backward: bias + q, k, v, o, dout + lse + dq, dk, dv + the live dS cells (bf16 plane)."""
+    n = batch.n_host.astype(np.int64) + 1
+    cells = int((n * n).sum()) * H
+    ntok = int(batch.tok_pos.numel())
+    fwd = 2 * cells + ntok * H * d * 2 * 4 + ntok * H * 4
+    bwd = 2 * cells + ntok * H * d * 2 * 5 + ntok * H * 4 + ntok * H * d * 2 * 3 + 2 * cells
+    return fwd, bwd
+
+
+def run_case(workload, hidden_dim, args, flush):
+    from mobgt_b200 import collator, model as M, ops
+    from mobgt_b200.trainer import Trainer
+    dev = torch.device("cuda")
+    cfg, ds, cap, n_fixed, nbatches = bench.TRAIN_WORKLOADS[workload]
+    world = bench.make_world_for(workload)
+    B = args.batch
+    item_sets = [bench.make_workload(workload, world, B, 0, batch_id=i) for i in range(nbatches)]
+    torch.manual_seed(1)
+    hp = dict(bench.HP, hidden_dim=hidden_dim)
+    model = M.Graphormer(dataset_name=ds, world=world, **hp).to(dev).train()
+    tr = Trainer(model, dev, 1, cuda_graph=True)
+    latlon = torch.from_numpy(world.latlon).to(dev)
+    ckw = dict(world=world, latlon_dev=latlon, multi_hop_max_dist=hp["multi_hop_max_dist"], rel_pos_max=1024, device=dev)
+    batches = [collator.collate_packed(its, max_node=512, bucket=nbatches > 1, **ckw) for its in item_sets]
+    state = dict(i=0)
+
+    def step():
+        b = batches[state["i"] % nbatches]
+        state["i"] += 1
+        state["loss"] = tr.train_step(b)
+
+    for _ in range(max(args.warmup, 2 * nbatches)):
+        step()
+    g0 = tr.graph_steps
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for _ in range(args.steps):
+        step()
+    torch.cuda.synchronize()
+    ms = (time.perf_counter() - t0) * 1e3 / args.steps
+    replays = tr.graph_steps - g0
+    loss = float(state["loss"])
+
+    # one layer's K3 at the first batch's shapes, dropout on, L2 overwritten before every launch
+    b = batches[0]
+    d = (hidden_dim + 64) // 8
+    tabs = [t.detach().float().contiguous() for t in (model.rel_pos_encoder.weight, model.poi_pos_encoder.weight,
+                                                       model.edge_encoder.weight, model.edge_dis_encoder.weight.view(-1),
+                                                       model.graph_token_virtual_distance.weight.view(-1))]
+    bias = ops.bias_fwd_raw(b, *tabs)
+    ntok = int(b.tok_pos.numel())
+    qkv = torch.randn(ntok, 3 * 8 * d, device=dev).to(torch.bfloat16)
+    dout = torch.randn(ntok, 8 * d, device=dev).to(torch.bfloat16)
+    dp, sd = hp["attention_dropout_rate"], 0x5DEECE66D1234567
+    out, lse = ops.attn_fwd_raw(qkv, bias, b, drop_p=dp, seed=sd)
+    plane = torch.empty(tuple(bias.shape), dtype=torch.bfloat16, device=dev)
+    scale = model.layers[0].self_attention.scale
+    t_f = bench.time_kernel(lambda: ops.attn_fwd_raw(qkv, bias, b, scale=scale, drop_p=dp, seed=sd), flush, iters=args.iters)
+    t_b = bench.time_kernel(lambda: ops.attn_bwd_raw(qkv, bias, out, dout, lse, b, plane, 2, scale=scale, drop_p=dp, seed=sd),
+                            flush, iters=args.iters)
+    fb, bb = k3_bytes(b, d)
+    n = b.n_host
+    return dict(workload=workload, hidden_dim=hidden_dim, head_dim=d, n_layers=hp["n_layers"], ffn_dim=hp["ffn_dim"],
+                graphs_per_step=B, tokens=ntok, nodes_max=int(n.max()), nodes_median=float(np.median(n)), padded=bool(getattr(b, "padded", False)),
+                step=dict(ms=ms, graphs_per_s=B * 1e3 / ms, steps=args.steps, graph_replays=replays, loss=loss),
+                k3=dict(fwd_ms=t_f, bwd_ms=t_b, fwd_bytes=fb, bwd_bytes=bb, fwd_gbs=fb / t_f / 1e6, bwd_gbs=bb / t_b / 1e6,
+                        iters=args.iters, dropout=dp, l2="256 MB buffer zeroed before every launch"))
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("out_dir")
+    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--batch", type=int, default=256)
+    ap.add_argument("--workloads", default="c2-dense128,c2-natural")
+    ap.add_argument("--hidden", default="128,64")
+    args = ap.parse_args()
+    from mobgt_b200 import _C
+    _C.require_cuda()
+    os.makedirs(args.out_dir, exist_ok=True)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
+    res = dict(card=card(), cases=[])
+    for wl in args.workloads.split(","):
+        for hd in (int(x) for x in args.hidden.split(",")):
+            r = run_case(wl, hd, args, flush)
+            res["cases"].append(r)
+            print(json.dumps(dict(workload=wl, hidden_dim=hd, step_ms=round(r["step"]["ms"], 3),
+                                  graphs_per_s=round(r["step"]["graphs_per_s"], 1), k3_fwd_ms=round(r["k3"]["fwd_ms"], 4),
+                                  k3_bwd_ms=round(r["k3"]["bwd_ms"], 4))), flush=True)
+    with open(os.path.join(args.out_dir, "bench_head_dim.json"), "w") as f:
+        json.dump(res, f, indent=1)
+    print(json.dumps(res["card"]))
+
+
+if __name__ == "__main__":
+    main()
