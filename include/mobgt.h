@@ -104,12 +104,14 @@ int32_t mobgt_poi_pos(const int32_t *x, const int32_t *n, const int64_t *sq_off,
  * poi_pos (collator.py:428-437), all per ordered node pair of each graph.
  *   bias [B,H,T,Tp] (f32 or bf16; Tp = row pitch, multiple of 8): only rows/cols < n[g]+1 are written;
  *   padding columns are masked inside the attention kernel from the sequence lengths.
+ *   H = num_heads: built for 8 and 12; any other value returns MOBGT_ERR_UNSUPPORTED.
  *   tables: R [512,H] rel_pos_encoder, Ppos [bins,H] poi_pos_encoder, E [128,H] edge_encoder,
  *           W [>=hops*H*H] edge_dis_encoder (viewed [k,h',h]), tvd [H] graph_token_virtual_distance.
  *   hops is the byte stride of an edge_in row (a multiple of 4, as written by K1); dk = multi_hop_max_dist is the number of
  *   live hop slots and the clamp of the mean (sp = clamp(M, 1, dk), model_fqandtoyo.py:1168-1174); 1 <= dk <= hops.
  *   forward workspace: mobgt_bias_fwd_workspace_bytes() (the E.W table [hops,128,H] and the rel_pos-keyed table RL [512,H]);
- *   backward workspace: mobgt_bias_bwd_workspace_bytes().
+ *   backward workspace: mobgt_bias_bwd_heads_workspace_bytes(T, hops, num_bins, H) (mobgt_bias_bwd_workspace_bytes() is the
+ *   same for H = 8).
  * Input domain (not checked on the device; K1 writes only values inside it):
  *   rel_pos in 0..511 (511: unreachable pair); poi_pos in 0..num_bins-1; edge_in bytes in 0..127, bytes [dk, hops) of
  *   every row 0; E row 0 (edge_encoder's padding row) zero.  Cells with rel_pos - 1 >= rel_pos_max are -inf in the forward.
@@ -128,8 +130,10 @@ int32_t mobgt_bias_fwd(const int32_t *n, const int64_t *sq_off, const int16_t *r
                        const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t H,
                        int32_t rel_pos_max, int32_t num_bins, const float *R, const float *Ppos, const float *E,
                        const float *W, const float *tvd, void *workspace, void *out, int32_t out_dtype, void *stream);
-/* bytes of `workspace` mobgt_bias_bwd needs (per-CTA partial histograms + totals); < 0 on bad arguments */
+/* bytes of `workspace` mobgt_bias_bwd needs at 8 heads (per-CTA partial histograms + totals); < 0 on bad arguments */
 int64_t mobgt_bias_bwd_workspace_bytes(int32_t T, int32_t hops, int32_t num_bins);
+/* the same at H heads (8 or 12); < 0 on bad arguments or another head count */
+int64_t mobgt_bias_bwd_heads_workspace_bytes(int32_t T, int32_t hops, int32_t num_bins, int32_t H);
 int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
                        const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t H,
                        int32_t rel_pos_max, int32_t num_bins, const void *dBias, int32_t dbias_dtype, int32_t n_layers,

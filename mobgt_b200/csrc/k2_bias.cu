@@ -26,7 +26,8 @@
 
 namespace mobgt {
 
-constexpr int kH = 8;          // heads (one float4 pair per table row); other head counts: UNSUPPORTED
+// Head counts: every kernel takes H as a template parameter, built for 8 (two float4s per table row) and 12 (three float4s);
+// other head counts are UNSUPPORTED.  The tables are [rows][H] fp32, so a row is H / 4 16-byte words.
 constexpr int kEdgeVocab = 128;  // edge_encoder rows (model_fqandtoyo.py:784)
 
 struct K2Common {
@@ -49,29 +50,30 @@ __host__ __device__ __forceinline__ int expected_walk(int rp, int hops) {
 }
 
 // Prologue tables (workspace):
-//   EW[k][v][h] = sum_h' E[v][h'] * W[k][h'][h]                                            [hops][128][8]
-//   RL[rp][h]   = R[rp][h] + ( sum_{k < L(rp)} EW[k][dom][h] ) / clamp(rp-1, 1, hops)       [512][8]
+//   EW[k][v][h] = sum_h' E[v][h'] * W[k][h'][h]                                            [hops][128][H]
+//   RL[rp][h]   = R[rp][h] + ( sum_{k < L(rp)} EW[k][dom][h] ) / clamp(rp-1, 1, hops)       [512][H]
 // RL is the whole rel_pos-keyed part of the bias of a pair whose walk is the EXPECTED one: L(rp) hops that all carry the
 // dominant edge feature (a single transition).  -inf where rp-1 >= rel_pos_max (collator.py:354-358).
+template <int H>
 __global__ void k2_prep_kernel(const float *__restrict__ E, const float *__restrict__ W, const float *__restrict__ R, int hops,
                                int dk, int rel_pos_max, float *__restrict__ EW, float *__restrict__ RL) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    const int nEW = hops * kEdgeVocab * kH;
+    const int nEW = hops * kEdgeVocab * H;
     if (idx < nEW) {
-        const int h = idx % kH, v = (idx / kH) % kEdgeVocab, k = idx / (kH * kEdgeVocab);
+        const int h = idx % H, v = (idx / H) % kEdgeVocab, k = idx / (H * kEdgeVocab);
         float acc = 0.f;
 #pragma unroll
-        for (int hp = 0; hp < kH; ++hp) acc += E[v * kH + hp] * W[(k * kH + hp) * kH + h];
+        for (int hp = 0; hp < H; ++hp) acc += E[v * H + hp] * W[(k * H + hp) * H + h];
         EW[idx] = acc;
-    } else if (idx < nEW + kRelRows * kH) {
+    } else if (idx < nEW + kRelRows * H) {
         const int j = idx - nEW;
-        const int h = j % kH, rp = j / kH;
+        const int h = j % H, rp = j / H;
         const int L = expected_walk(rp, dk);
         float ps = 0.f;
         for (int k = 0; k < L; ++k) {
             float acc = 0.f;
 #pragma unroll
-            for (int hp = 0; hp < kH; ++hp) acc += E[kDomEdge * kH + hp] * W[(k * kH + hp) * kH + h];
+            for (int hp = 0; hp < H; ++hp) acc += E[kDomEdge * H + hp] * W[(k * H + hp) * H + h];
             ps += acc;
         }
         const int M = rp - 1;
@@ -80,17 +82,42 @@ __global__ void k2_prep_kernel(const float *__restrict__ E, const float *__restr
     }
 }
 
-__device__ __forceinline__ void add8(float (&a)[8], const float *__restrict__ p) {
-    const float4 x = *reinterpret_cast<const float4 *>(p);
-    const float4 y = *reinterpret_cast<const float4 *>(p + 4);
-    a[0] += x.x; a[1] += x.y; a[2] += x.z; a[3] += x.w;
-    a[4] += y.x; a[5] += y.y; a[6] += y.z; a[7] += y.w;
+// one H-float table row as H / 4 float4 loads, all issued before the first is used
+template <int H>
+__device__ __forceinline__ void load_row(float4 (&x)[H / 4], const float *__restrict__ p) {
+#pragma unroll
+    for (int i = 0; i < H / 4; ++i) x[i] = *reinterpret_cast<const float4 *>(p + 4 * i);
 }
-__device__ __forceinline__ void sub8(float (&a)[8], const float *__restrict__ p) {
-    const float4 x = *reinterpret_cast<const float4 *>(p);
-    const float4 y = *reinterpret_cast<const float4 *>(p + 4);
-    a[0] -= x.x; a[1] -= x.y; a[2] -= x.z; a[3] -= x.w;
-    a[4] -= y.x; a[5] -= y.y; a[6] -= y.z; a[7] -= y.w;
+// a[h] += p[h] / a[h] -= p[h] over one table row
+template <int H>
+__device__ __forceinline__ void add_row(float (&a)[H], const float *__restrict__ p) {
+    float4 x[H / 4];
+    load_row<H>(x, p);
+#pragma unroll
+    for (int i = 0; i < H / 4; ++i) {
+        a[4 * i] += x[i].x; a[4 * i + 1] += x[i].y; a[4 * i + 2] += x[i].z; a[4 * i + 3] += x[i].w;
+    }
+}
+template <int H>
+__device__ __forceinline__ void sub_row(float (&a)[H], const float *__restrict__ p) {
+    float4 x[H / 4];
+    load_row<H>(x, p);
+#pragma unroll
+    for (int i = 0; i < H / 4; ++i) {
+        a[4 * i] -= x[i].x; a[4 * i + 1] -= x[i].y; a[4 * i + 2] -= x[i].z; a[4 * i + 3] -= x[i].w;
+    }
+}
+
+// i % H and i / H of a non-negative index (8 heads: the mask and shift the 8-head kernels were written with)
+template <int H>
+__device__ __forceinline__ int mod_h(int i) {
+    if constexpr (H == 8) return i & 7;
+    else return (int)((uint32_t)i % H);
+}
+template <int H>
+__device__ __forceinline__ int div_h(int i) {
+    if constexpr (H == 8) return i >> 3;
+    else return (int)((uint32_t)i / H);
 }
 
 __device__ __forceinline__ float bf16lo(uint32_t w) { return __uint_as_float(w << 16); }
@@ -117,23 +144,33 @@ __device__ __forceinline__ uint32_t expected_word(int L, int q) {
     return (0x01010101u * (uint32_t)kDomEdge) & mask;
 }
 
-// Forward.  Persistent CTAs; RL [512][8], Ppos [bins][8] and the expected-walk words XW [hops+1][8] are staged once per
-// CTA in shared memory.  One thread per PAIR OF ADJACENT CELLS (a, b) (a, b+1), b even, of the Tp-pitched plane row, so
-// every head plane is written as 4-byte (bf16x2) / 8-byte (f32x2) words and a warp covers 64 consecutive columns.  All
-// index bytes of a thread's two cells (2 x (2 + 2 + hops) B) are fetched up front as independent loads.
+// cells per forward thread (see the forward's comment)
+template <int H>
+struct K2FwdCells {
+    static constexpr int kCells = H == 8 ? 2 : 1;
+};
+
+// Forward.  Persistent CTAs; RL [512][H], Ppos [bins][H] and the expected-walk words XW [hops+1][8] are staged once per
+// CTA in shared memory.  At 8 heads, one thread per PAIR OF ADJACENT CELLS (a, b) (a, b+1), b even, of the Tp-pitched
+// plane row, so every head plane is written as 4-byte (bf16x2) / 8-byte (f32x2) words and a warp covers 64 consecutive
+// columns.  All index bytes of a thread's cells (2 + 2 + hops B each) are fetched up front as independent loads.
+// At 12 heads a thread takes ONE cell (K2FwdCells): two cells would keep 2 x 12 accumulators, the correction row and up to
+// 2 x 8 walk words live under the 64 registers __launch_bounds__(512, 2) leaves, and spill 32-88 bytes of stack per thread
+// (56 at hops = 20).  With one cell the spill is 8 bytes at hops 12..24 and 16 / 24 at hops 28 / 32, no more than the
+// 8-head kernel's.  A warp then covers 32 consecutive columns with 2-byte (bf16) / 4-byte (f32) stores.
 //
 // Per cell the work is TWO table gathers: bias = RL[rp] + Ppos[pp].  The walk bytes are only compared (XOR) against the
 // walk the distance predicts; the bytes that differ — another edge feature (0.7 % of the hops of trajectory graphs) or a
 // walk cut short by the reference's node-0 quirk (algos.pyx:57-62) — are corrected one by one from the EW table in
 // global memory (L1-resident):   Edge = sum_k EW[k][e_k]  =  PS[L] + sum_{k : e_k != x_k} ( EW[k][e_k] - EW[k][x_k] ).
 // The identity holds for ANY byte pattern (EW[k][0] = 0: edge_encoder row 0 is the padding row, model_fqandtoyo.py:784).
-template <typename OutT, int HOPW>
+template <int H, typename OutT, int HOPW>
 __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, const float *__restrict__ RLg,
                                                              const float *__restrict__ Pg, int num_bins,
                                                              const float *__restrict__ tvd,
                                                              const float *__restrict__ EWg, OutT *__restrict__ out) {
     extern __shared__ __align__(16) float sm[];
-    const int nR = kRelRows * kH, nP = num_bins * kH;
+    const int nR = kRelRows * H, nP = num_bins * H;
     float *RL = sm, *Pp = RL + nR;
     uint32_t *XW = reinterpret_cast<uint32_t *>(Pp + nP);          // [hops + 1][8]
     for (int i = threadIdx.x * 4; i < nR; i += blockDim.x * 4)
@@ -143,32 +180,33 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
     constexpr int hopw = HOPW;                    // hops = 4 * HOPW
     for (int i = threadIdx.x; i < (c.hops + 1) * 8; i += blockDim.x) XW[i] = (i & 7) < hopw ? expected_word(i >> 3, i & 7) : 0u;
     __syncthreads();
-    const int half = c.Tp >> 1;                   // cell pairs per plane row
+    constexpr int kCells = K2FwdCells<H>::kCells;
+    const int half = c.Tp >> (kCells - 1);        // threads per plane row (cell pairs at 8 heads, cells at 12)
     const int per_graph = c.T * half;
     const int tiles = ceil_div(per_graph, (int)blockDim.x);
-    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^18
+    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^19
     const size_t hs = (size_t)c.T * c.Tp;
     for (int w = blockIdx.x; w < tiles * c.B; w += gridDim.x) {
         const int g = w / tiles, tile = w - g * tiles;
         const int n = c.n[g];
         const int Tg = n + 1;
         const int f = tile * blockDim.x + threadIdx.x;
-        const int a = (int)(((uint64_t)f * half_magic) >> 40), b = (f - a * half) * 2;
+        const int a = (int)(((uint64_t)f * half_magic) >> 40), b = (f - a * half) * kCells;
         if (a >= Tg || b >= Tg) continue;
-        const bool two = b + 1 < Tg;
-        float acc[2][8];
+        const bool two = kCells == 2 && b + 1 < Tg;
+        float acc[kCells][H];
 #pragma unroll
-        for (int s = 0; s < 2; ++s)
+        for (int s = 0; s < kCells; ++s)
 #pragma unroll
-            for (int h = 0; h < 8; ++h) acc[s][h] = 0.f;
+            for (int h = 0; h < H; ++h) acc[s][h] = 0.f;
         if (a >= 1) {
             const int64_t rowp = c.sq_off[g] + (int64_t)(a - 1) * n;   // pair (a-1, j) lives at rowp + j
             // cell s of this thread is the pair j = b - 1 + s  (b == 0, s == 0: the virtual-distance column)
-            int rp[2], pp[2];
-            uint32_t ew[2][HOPW];
-            bool is_pair[2];
+            int rp[kCells], pp[kCells];
+            uint32_t ew[kCells][HOPW];
+            bool is_pair[kCells];
 #pragma unroll
-            for (int s = 0; s < 2; ++s) {
+            for (int s = 0; s < kCells; ++s) {
                 const int j = b - 1 + s;
                 is_pair[s] = j >= 0 && j < n;
                 rp[s] = 0; pp[s] = 0;
@@ -184,11 +222,11 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
                 }
             }
 #pragma unroll
-            for (int s = 0; s < 2; ++s) {
+            for (int s = 0; s < kCells; ++s) {
                 if (!is_pair[s]) {
                     if (b == 0 && s == 0) {
 #pragma unroll
-                        for (int h = 0; h < 8; ++h) acc[0][h] = __ldg(tvd + h);
+                        for (int h = 0; h < H; ++h) acc[0][h] = __ldg(tvd + h);
                     }
                     continue;
                 }
@@ -199,13 +237,17 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
                 uint32_t any = 0u;
 #pragma unroll
                 for (int q = 0; q < HOPW; ++q) any |= ew[s][q] ^ xw[q];
-                const float *r = RL + rk * kH, *q_ = Pp + min(max(pp[s], 0), num_bins - 1) * kH;
-                const float4 r0 = *reinterpret_cast<const float4 *>(r), r1 = *reinterpret_cast<const float4 *>(r + 4);
-                const float4 p0 = *reinterpret_cast<const float4 *>(q_), p1 = *reinterpret_cast<const float4 *>(q_ + 4);
-                acc[s][0] = r0.x + p0.x; acc[s][1] = r0.y + p0.y; acc[s][2] = r0.z + p0.z; acc[s][3] = r0.w + p0.w;
-                acc[s][4] = r1.x + p1.x; acc[s][5] = r1.y + p1.y; acc[s][6] = r1.z + p1.z; acc[s][7] = r1.w + p1.w;
+                const float *r = RL + rk * H, *q_ = Pp + min(max(pp[s], 0), num_bins - 1) * H;
+                float4 r0[H / 4], p0[H / 4];
+                load_row<H>(r0, r);
+                load_row<H>(p0, q_);
+#pragma unroll
+                for (int i = 0; i < H / 4; ++i) {
+                    acc[s][4 * i] = r0[i].x + p0[i].x; acc[s][4 * i + 1] = r0[i].y + p0[i].y;
+                    acc[s][4 * i + 2] = r0[i].z + p0[i].z; acc[s][4 * i + 3] = r0[i].w + p0[i].w;
+                }
                 if (any != 0u) {
-                    float corr[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+                    float corr[H] = {};
 #pragma unroll
                     for (int q = 0; q < HOPW; ++q) {
                         {
@@ -213,26 +255,26 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
                             while (d != 0u) {
                                 const int e = (__ffs(d) - 1) >> 3;
                                 const int v = (ew[s][q] >> (8 * e)) & 0xFF, x = (xw[q] >> (8 * e)) & 0xFF;
-                                const float *row = EWg + (size_t)(q * 4 + e) * kEdgeVocab * kH;
-                                add8(corr, row + min(v, kEdgeVocab - 1) * kH);
-                                sub8(corr, row + x * kH);
+                                const float *row = EWg + (size_t)(q * 4 + e) * kEdgeVocab * H;
+                                add_row<H>(corr, row + min(v, kEdgeVocab - 1) * H);
+                                sub_row<H>(corr, row + x * H);
                                 d &= ~(0xFFu << (8 * e));
                             }
                         }
                     }
                     const float inv = 1.0f / (float)min(max(rk - 1, 1), c.dk);
 #pragma unroll
-                    for (int h = 0; h < 8; ++h) acc[s][h] += corr[h] * inv;
+                    for (int h = 0; h < H; ++h) acc[s][h] += corr[h] * inv;
                 }
             }
         }
-        OutT *o = out + ((size_t)g * kH * c.T + a) * c.Tp + b;
+        OutT *o = out + ((size_t)g * H * c.T + a) * c.Tp + b;
         if (two) {
 #pragma unroll
-            for (int h = 0; h < 8; ++h) store2<OutT>(o + h * hs, acc[0][h], acc[1][h]);
+            for (int h = 0; h < H; ++h) store2<OutT>(o + h * hs, acc[0][h], acc[kCells - 1][h]);
         } else {
 #pragma unroll
-            for (int h = 0; h < 8; ++h) store1<OutT>(o + h * hs, acc[0][h]);
+            for (int h = 0; h < H; ++h) store1<OutT>(o + h * hs, acc[0][h]);
         }
     }
 }
@@ -240,7 +282,7 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
 // ---- backward --------------------------------------------------------------------------------------
 // dBias (per-layer bf16 dS planes, or one fp32 buffer) -> table gradients.  With the forward's decomposition
 //   bias(cell) = RL[rp] + Ppos[pp] + ( sum over the bytes that deviate from the expected walk ) / sp
-// every cell contributes its 8-vector d[h] to exactly TWO keyed sums, dRL[rp] and dPpos[pp] (plus dt for column 0); only
+// every cell contributes its H-vector d[h] to exactly TWO keyed sums, dRL[rp] and dPpos[pp] (plus dt for column 0); only
 // the deviating bytes (0.09 per cell on trajectory graphs) touch dEW directly.  The finish kernels unfold dRL:
 //   dR[rp] = dRL[rp] ;   dEW[k][dom] += sum_{rp : L(rp) > k} dRL[rp] / sp(rp).
 // One WARP per plane row (g, a), 1 persistent CTA per SM, three phases per row:
@@ -249,14 +291,30 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
 //   2. index phase — lane = cell: rel_pos, poi_pos and the walk words are read once and packed into cinfo[b] (histogram
 //                    rows + flags) and cdev[b] (up to two deviating bytes, so the histogram phase never touches global
 //                    memory);
-//   3. histogram   — lanes = (table: R | P) x (2 cells) x (8 heads): ONE read-modify-write per lane and step into
-//                    warp-private histograms laid out [key][cell slot][head] — no atomics, no cross-lane hazards; two
-//                    steps are in flight per lane (equal keys are merged in registers).
+//   3. histogram   — lanes = (table: R | P) x (cell slot) x (head) (K2Heads below): ONE read-modify-write per lane and
+//                    step into warp-private histograms laid out [key][cell slot][head] — no atomics, no cross-lane
+//                    hazards; two steps are in flight per lane (equal keys are merged in registers).
 //   Deviating bytes (the rare path): 64-bit FIXED-POINT integer atomics (value * 2^38) into the CTA's own small dEW table in
 //   global memory (features < 16) or into the launch-wide table (other features, rel_pos keys outside the plan).  Integer
 //   addition is associative, so the sums do not depend on the order in which the atomics land.
 // Per-CTA totals go to a partial buffer and are reduced in a fixed order: the whole backward is bitwise reproducible.
 constexpr int kSmallVocab = 16;   // edge features kept in the CTA's shared dEW table
+
+// Lane maps of the backward.  In the histogram phase every lane owns one (table, cell slot, head) column of the warp's
+// histograms, so no two lanes ever write the same word, and each step a lane adds two adjacent cells of its slot.
+//   H = 8:  2 tables x 2 cell slots x 8 heads = 32 lanes; a step covers 4 cells.
+//   H = 12: 2 tables x 12 heads = 24 columns already; a second cell slot would need 48 lanes.  So there is one cell slot, a
+//           step covers 2 cells and lanes 24..31 sit the phase out (75 % of the lanes busy).  Splitting the heads over two
+//           passes instead (8 + 4 heads, 2 cell slots each) keeps the same 96 read-modify-writes per 64 lane-steps, with
+//           a second pass over cinfo; one slot also halves the histograms' shared memory, which buys warps per CTA.
+// The slow path gives each listed cell H lanes (one per head): 32 / H cells at a time (4 at H = 8, 2 at H = 12).
+template <int H>
+struct K2Heads {
+    static_assert(H == 8 || H == 12, "the attention-bias kernels are built for 8 and 12 heads");
+    static constexpr int kSlots = 32 / (2 * H);       // histogram cell slots
+    static constexpr int kLanes = 2 * kSlots * H;     // lanes that own a histogram column
+    static constexpr int kSlowCells = 32 / H;         // slow-path cells per round
+};
 
 // 12 warps at most: 384 threads leave 170 registers per thread, which the sum phase (18 x 16-byte loads in flight per lane)
 // and the index phase (the indices of up to 160 cells of the row loaded before any is decoded) are sized for
@@ -266,24 +324,26 @@ constexpr int kIdxUnroll = 5;    // 32-cell groups whose index loads are issued 
 
 struct K2BwdPlan {
     int Rrows;      // rel_pos histogram rows: keys 0..Rrows-2 direct, key 511 -> row Rrows-1
-    int nEWs, nR, nP, stride;   // floats; partial row = [EWsmall | R | P | t(8)]
+    int nEWs, nR, nP, stride;   // floats; partial row = [EWsmall | R | P | t(H)]
     int pitch;      // floats per head in the dsum strip: >= T rounded up to 4, == 4 (mod 32)
     int per_warp;   // floats of warp-private shared memory
     int cta_words;  // floats of CTA-wide shared memory in front of the warp strips
     int warps;
 };
 
+template <int H>
 __host__ __device__ inline K2BwdPlan k2_bwd_plan(int T, int Tp, int hops, int num_bins) {
+    constexpr int S = K2Heads<H>::kSlots;
     K2BwdPlan p;
     p.Rrows = min(T, 511) + 1;
-    p.nEWs = hops * kSmallVocab * kH;
-    p.nR = p.Rrows * kH;
-    p.nP = num_bins * kH;
-    p.stride = p.nEWs + p.nR + p.nP + kH;
+    p.nEWs = hops * kSmallVocab * H;
+    p.nR = p.Rrows * H;
+    p.nP = num_bins * H;
+    p.stride = p.nEWs + p.nR + p.nP + H;
     // cells b < (T + 3) & ~3 are the ones the index / histogram phases touch; the sum phase clips its 8-cell stores at the pitch
     (void)Tp;
     p.pitch = ((((T + 3) & ~3) + 27) / 32) * 32 + 4;
-    p.per_warp = 2 * (p.nR + kH) + 2 * (p.nP + kH) + kH * p.pitch + 3 * p.pitch + kH;   // hR+trash | hP+trash | dsum | cinfo | cdev | dlist | t
+    p.per_warp = S * (p.nR + H) + S * (p.nP + H) + H * p.pitch + 3 * p.pitch + H;   // hR+trash | hP+trash | dsum | cinfo | cdev | dlist | t
     p.cta_words = (hops + 1) * 8 + 40;                                     // XW | 1/sp table
     int w = (int)((227 * 1024 - 2048 - p.cta_words * 4) / (p.per_warp * 4));
     p.warps = w > kK2BwdMaxWarps ? kK2BwdMaxWarps : w;
@@ -315,7 +375,7 @@ __device__ __forceinline__ void sts_f32x4(uint32_t a, float x, float y, float z,
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(x), "f"(y), "f"(z), "f"(w) : "memory");
 }
 
-template <typename DT, int HOPW>
+template <int H, typename DT, int HOPW>
 __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(const K2Common c, const DT *__restrict__ dB, int nlayers,
                                                              int64_t layer_stride, int num_bins,
                                                              const K2BwdPlan pl, float *__restrict__ partial,
@@ -323,20 +383,22 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
                                                              long long *__restrict__ dR64) {
     extern __shared__ __align__(16) float sm[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
-    const int ty = lane >> 4, c2 = (lane >> 3) & 1, h = lane & 7;      // table (0 = R, 1 = P), cell slot, head
-    long long *sEW = ews64 + (size_t)blockIdx.x * pl.nEWs;        // this CTA's [hops][16][8] table (global memory, zeroed by the host)
+    constexpr int S = K2Heads<H>::kSlots;
+    const int ty = lane / (S * H), c2 = (lane / H) % S, h = lane % H;      // table (0 = R, 1 = P), cell slot, head
+    long long *sEW = ews64 + (size_t)blockIdx.x * pl.nEWs;        // this CTA's [hops][16][H] table (global memory, zeroed by the host)
     uint32_t *XW = reinterpret_cast<uint32_t *>(sm);              // [hops + 1][8]
     float *invT = sm + (c.hops + 1) * 8;                          // [40]: 1 / sp
     float *wbase = sm + pl.cta_words;
     const uint32_t s_warp = (uint32_t)__cvta_generic_to_shared(wbase + (size_t)warp * pl.per_warp);
-    const uint32_t s_hR = s_warp;                                 // [Rrows + 1][2][8]   (last row: trash)
-    const uint32_t s_hP = s_hR + 2u * (pl.nR + kH) * 4u;          // [bins + 1][2][8]    (last row: trash)
-    const uint32_t s_dsum = s_hP + 2u * (pl.nP + kH) * 4u;        // [8][pitch]
-    const uint32_t s_cinfo = s_dsum + (uint32_t)(kH * pl.pitch) * 4u;   // [pitch]: R row | P row << 16
+    const uint32_t s_hR = s_warp;                                 // [Rrows + 1][S][H]   (last row: trash)
+    const uint32_t s_hP = s_hR + (uint32_t)S * (pl.nR + H) * 4u;  // [bins + 1][S][H]    (last row: trash)
+    const uint32_t s_dsum = s_hP + (uint32_t)S * (pl.nP + H) * 4u;        // [H][pitch]
+    const uint32_t s_cinfo = s_dsum + (uint32_t)(H * pl.pitch) * 4u;    // [pitch]: R row | P row << 16
     const uint32_t s_cdev = s_cinfo + (uint32_t)pl.pitch * 4u;    // [pitch]
     const uint32_t s_dlist = s_cdev + (uint32_t)pl.pitch * 4u;    // [pitch]: cells that need the slow path
-    const uint32_t s_T = s_dlist + (uint32_t)pl.pitch * 4u;       // [8]
-    const uint32_t s_hist = (ty ? s_hP : s_hR) + (uint32_t)(c2 * kH + h) * 4u;      // + key * 64 B
+    const uint32_t s_T = s_dlist + (uint32_t)pl.pitch * 4u;       // [H]
+    const uint32_t s_hist = (ty ? s_hP : s_hR) + (uint32_t)(c2 * H + h) * 4u;       // + key * S * H * 4 B
+    constexpr uint32_t key_bytes = S * H * 4;
     const uint32_t key_shift = ty ? 16u : 0u;
     const uint32_t trashR = (uint32_t)pl.Rrows, trashP = (uint32_t)num_bins;
     constexpr int hopw = HOPW;                                   // 32-bit words per walk (hops / 4)
@@ -354,9 +416,9 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
         const int Tg = n + 1;
         const int64_t rowp = c.sq_off[g] + (int64_t)(a - 1) * n - 1;     // pair of cell b lives at rowp + b
         // ---- 1. sum phase: dsum[h][b] = sum over layers of plane[l][g][h][a][b]
-        const DT *rowbase = dB + ((size_t)g * kH * c.T + a) * c.Tp;
+        const DT *rowbase = dB + ((size_t)g * H * c.T + a) * c.Tp;
         constexpr int kPer = 16 / (int)sizeof(DT);           // cells per 16-byte load
-        const int nitems = ceil_div(Tg, kPer) * kH;
+        const int nitems = ceil_div(Tg, kPer) * H;           // item i = (chunk i / H, head i % H)
         for (int i0 = 0; i0 < nitems; i0 += 32 * kSumItems) {
             const int ns = min(kSumItems, (nitems - i0 + 31) >> 5);   // 32-item slots of this round that hold an item (warp-uniform)
             float accv[kSumItems][8];
@@ -371,7 +433,7 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
                 const int i = i0 + 32 * s + lane;
                 ok[s] = i < nitems;
                 const int ic = min(i, nitems - 1);           // lanes past the last item re-read it (no predicate on the loads)
-                src[s] = rowbase + (size_t)(ic & 7) * hs + (ic >> 3) * kPer;
+                src[s] = rowbase + (size_t)mod_h<H>(ic) * hs + div_h<H>(ic) * kPer;
             }
             for (int l0 = 0; l0 < nlayers; l0 += 6) {
                 uint4 v[kSumItems][6];
@@ -417,10 +479,10 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
             for (int s = 0; s < kSumItems; ++s) {
                 const int i = i0 + 32 * s + lane;
                 if (ok[s]) {
-                    const uint32_t dst = s_dsum + (uint32_t)(i & 7) * pitch4 + (uint32_t)((i >> 3) * kPer) * 4u;
+                    const uint32_t dst = s_dsum + (uint32_t)mod_h<H>(i) * pitch4 + (uint32_t)(div_h<H>(i) * kPer) * 4u;
                     sts_f32x4(dst, accv[s][0], accv[s][1], accv[s][2], accv[s][3]);
                     if constexpr (sizeof(DT) == 2) {         // cells past the pitch lie beyond the graph's last token: never read
-                        if ((i >> 3) * kPer + 8 <= pl.pitch) sts_f32x4(dst + 16u, accv[s][4], accv[s][5], accv[s][6], accv[s][7]);
+                        if (div_h<H>(i) * kPer + 8 <= pl.pitch) sts_f32x4(dst + 16u, accv[s][4], accv[s][5], accv[s][6], accv[s][7]);
                     }
                 }
             }
@@ -492,16 +554,16 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
         __syncwarp();
         // ---- 3. histogram phase: lane = (table, cell slot c2, head h); adjacent cells b0 + 2 c2, b0 + 2 c2 + 1 per step.
         //         Cells without a gradient point at the trash rows, so the loop carries no predicates.
-        if (lane < 8) tacc += lds_f32(s_dsum + (uint32_t)h * pitch4);          // column 0: graph-token virtual distance
-        {
+        if (lane < H) tacc += lds_f32(s_dsum + (uint32_t)h * pitch4);          // column 0: graph-token virtual distance
+        if (K2Heads<H>::kLanes == 32 || lane < K2Heads<H>::kLanes) {
             uint32_t pi = s_cinfo + (uint32_t)c2 * 8u, pd = s_dsum + (uint32_t)h * pitch4 + (uint32_t)c2 * 8u;
-            for (int b0 = 0; b0 < Tg4; b0 += 4, pi += 16u, pd += 16u) {
+            for (int b0 = 0; b0 < Tg4; b0 += 2 * S, pi += 8u * S, pd += 8u * S) {
                 uint32_t iA, iB;
                 float dA, dB_;
                 asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(iA), "=r"(iB) : "r"(pi) : "memory");
                 asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(dA), "=f"(dB_) : "r"(pd) : "memory");
-                const uint32_t aA = s_hist + ((iA >> key_shift) & 0xFFFFu) * 64u;
-                const uint32_t aB = s_hist + ((iB >> key_shift) & 0xFFFFu) * 64u;
+                const uint32_t aA = s_hist + ((iA >> key_shift) & 0xFFFFu) * key_bytes;
+                const uint32_t aB = s_hist + ((iB >> key_shift) & 0xFFFFu) * key_bytes;
                 // two read-modify-writes in flight; equal addresses are chained in registers, the second store wins
                 const float vA = lds_f32(aA), vB = lds_f32(aB);
                 const float nA = vA + dA;
@@ -510,11 +572,12 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
                 sts_f32(aB, nB);
             }
         }
-        // ---- slow path (rare): walk bytes that differ from the expected walk, keys outside the plan; 8 lanes = 8 heads per
-        //      listed cell, 4 cells at a time
-        for (int e0 = 0; e0 < ndl; e0 += 4) {
-            const int e = e0 + (lane >> 3);
-            if (e >= ndl) continue;
+        // ---- slow path (rare): walk bytes that differ from the expected walk, keys outside the plan; H lanes = H heads per
+        //      listed cell, 32 / H cells at a time
+        constexpr int SC = K2Heads<H>::kSlowCells;
+        for (int e0 = 0; e0 < ndl; e0 += SC) {
+            const int e = e0 + lane / H;
+            if (e >= ndl || (SC * H < 32 && lane >= SC * H)) continue;
             const uint32_t ent = lds_u32(s_dlist + (uint32_t)e * 4u);
             const int b = ent & 0xFFF;
             const float d = lds_f32(s_dsum + (uint32_t)h * pitch4 + (uint32_t)b * 4u);
@@ -522,10 +585,10 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
                 // a key outside the plan has no histogram row, so the dRL unfold of the scatter kernel never sees it: its
                 // expected-walk share d / sp for each of the L(rk) hops goes into dEW[k][dom] here (sp = L: rk >= 2 here)
                 const int rk = min(max((int)c.rel_pos[rowp + b], 0), kRelRows - 1);
-                fx_add(dR64 + rk * kH + h, d);
+                fx_add(dR64 + rk * H + h, d);
                 const int Lk = expected_walk(rk, c.dk);
                 const float dl = d * invT[max(Lk, 1)];
-                for (int k = 0; k < Lk; ++k) fx_add(sEW + (k * kSmallVocab + kDomEdge) * kH + h, dl);
+                for (int k = 0; k < Lk; ++k) fx_add(sEW + (k * kSmallVocab + kDomEdge) * H + h, dl);
             }
             if (!(ent & (1u << 14))) continue;
             const uint32_t cd = lds_u32(s_cdev + (uint32_t)b * 4u);
@@ -536,10 +599,10 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
                     const uint32_t en = (cd >> (8 + 12 * j)) & 4095u;
                     const int k = en >> 7, v = en & 127, x = k < L ? kDomEdge : 0;
                     if (v != 0) {
-                        if (v < kSmallVocab) fx_add(sEW + (k * kSmallVocab + v) * kH + h, dinv);
-                        else fx_add(dEWfull64 + ((size_t)k * kEdgeVocab + v) * kH + h, dinv);
+                        if (v < kSmallVocab) fx_add(sEW + (k * kSmallVocab + v) * H + h, dinv);
+                        else fx_add(dEWfull64 + ((size_t)k * kEdgeVocab + v) * H + h, dinv);
                     }
-                    if (x != 0) fx_add(sEW + (k * kSmallVocab + x) * kH + h, -dinv);
+                    if (x != 0) fx_add(sEW + (k * kSmallVocab + x) * H + h, -dinv);
                 }
             } else {
                 const uint32_t *ei = reinterpret_cast<const uint32_t *>(c.edge_in + (rowp + b) * c.hops);
@@ -551,10 +614,10 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
                         const int v = (ew >> (8 * eb)) & 0xFF, x = (xw >> (8 * eb)) & 0xFF;
                         const int k = q * 4 + eb;
                         if (v != 0) {
-                            if (v < kSmallVocab) fx_add(sEW + (k * kSmallVocab + v) * kH + h, dinv);
-                            else fx_add(dEWfull64 + ((size_t)k * kEdgeVocab + min(v, kEdgeVocab - 1)) * kH + h, dinv);
+                            if (v < kSmallVocab) fx_add(sEW + (k * kSmallVocab + v) * H + h, dinv);
+                            else fx_add(dEWfull64 + ((size_t)k * kEdgeVocab + min(v, kEdgeVocab - 1)) * H + h, dinv);
                         }
-                        if (x != 0) fx_add(sEW + (k * kSmallVocab + x) * kH + h, -dinv);
+                        if (x != 0) fx_add(sEW + (k * kSmallVocab + x) * H + h, -dinv);
                         df &= ~(0xFFu << (8 * eb));
                     }
                 }
@@ -562,35 +625,36 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
         }
         __syncwarp();
     }
-    // column-0 sums: lanes 0..7 hold them
-    if (lane < 8) sts_f32(s_T + (uint32_t)h * 4u, tacc);
+    // column-0 sums: lanes 0..H-1 hold them
+    if (lane < H) sts_f32(s_T + (uint32_t)h * 4u, tacc);
     __syncthreads();
     // CTA totals -> partial[blockIdx]
     float *out = partial + (size_t)blockIdx.x * pl.stride;
     for (int i = threadIdx.x; i < pl.nR; i += blockDim.x) {
-        const int key = i / kH, hh = i % kH;
+        const int key = i / H, hh = i % H;
         float s = 0.f;
         for (int w = 0; w < nwarp; ++w)
-            for (int r = 0; r < 2; ++r) s += wbase[(size_t)w * pl.per_warp + (key * 2 + r) * kH + hh];
+            for (int r = 0; r < S; ++r) s += wbase[(size_t)w * pl.per_warp + (key * S + r) * H + hh];
         out[pl.nEWs + i] = s;
     }
     for (int i = threadIdx.x; i < pl.nP; i += blockDim.x) {
-        const int key = i / kH, hh = i % kH;
+        const int key = i / H, hh = i % H;
         float s = 0.f;
         for (int w = 0; w < nwarp; ++w)
-            for (int r = 0; r < 2; ++r) s += wbase[(size_t)w * pl.per_warp + 2 * (pl.nR + kH) + (key * 2 + r) * kH + hh];
+            for (int r = 0; r < S; ++r) s += wbase[(size_t)w * pl.per_warp + S * (pl.nR + H) + (key * S + r) * H + hh];
         out[pl.nEWs + pl.nR + i] = s;
     }
-    if (threadIdx.x < kH) {
+    if (threadIdx.x < H) {
         float s = 0.f;
-        for (int w = 0; w < nwarp; ++w) s += wbase[(size_t)w * pl.per_warp + pl.per_warp - kH + threadIdx.x];
+        for (int w = 0; w < nwarp; ++w) s += wbase[(size_t)w * pl.per_warp + pl.per_warp - H + threadIdx.x];
         out[pl.nEWs + pl.nR + pl.nP + threadIdx.x] = s;
     }
 }
 
 // tot[i] = sum over CTAs of partial[cta][i] (fixed order); the EWsmall part [0, nEWs) is the exact integer sum of the CTAs'
 // fixed-point tables.  The same launch converts the launch-wide fixed-point tables: dEWfull (threads [stride, stride + nEW))
-// and the rel_pos overflow rows into dR (the next kRelRows * kH threads).
+// and the rel_pos overflow rows into dR (the next kRelRows * H threads).
+template <int H>
 __global__ void k2_bias_bwd_reduce_kernel(const float *__restrict__ partial, int nparts, int stride, int nEWs,
                                           const long long *__restrict__ ews64, float *__restrict__ tot,
                                           const long long *__restrict__ dEWfull64, int nEW, float *__restrict__ dEWfull,
@@ -608,62 +672,64 @@ __global__ void k2_bias_bwd_reduce_kernel(const float *__restrict__ partial, int
         tot[i] = s;
     } else if ((i -= stride) < nEW) {
         dEWfull[i] = fx_to_float(dEWfull64[i]);
-    } else if ((i -= nEW) < kRelRows * kH) {
+    } else if ((i -= nEW) < kRelRows * H) {
         dR[i] = fx_to_float(dR64[i]);
     }
 }
 
 // totals -> dR, dPpos, dt, and the full dEW[k][v][h] (which already holds the global rare-path atomics):
 //   dEW[k][v] += EWsmall[k][v] (v < 16) ;  dEW[k][dom] += sum_{rp : L(rp) > k} dRL[rp] / sp(rp)   (one warp per (k, h))
+template <int H>
 __global__ void k2_bias_bwd_scatter_kernel(const float *__restrict__ tot, const K2BwdPlan pl, int hops, int dk, int num_bins,
                                            float *__restrict__ dEWfull, float *__restrict__ dR, float *__restrict__ dP,
                                            float *__restrict__ dt) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const float *tE = tot, *tR = tot + pl.nEWs, *tP = tR + pl.nR, *tT = tP + pl.nP;
-    if (i < kRelRows * kH) {
-        const int rp = i / kH, hh = i % kH;
+    if (i < kRelRows * H) {
+        const int rp = i / H, hh = i % H;
         const int row = (rp == 511) ? pl.Rrows - 1 : (rp < pl.Rrows - 1 ? rp : -1);
-        dR[i] += (row >= 0) ? tR[row * kH + hh] : 0.f;     // dR holds the (normally empty) overflow atomics
+        dR[i] += (row >= 0) ? tR[row * H + hh] : 0.f;     // dR holds the (normally empty) overflow atomics
     }
-    if (i < num_bins * kH) dP[i] = tP[i];
-    if (i < kH) dt[i] = tT[i];
-    if (i < hops * kSmallVocab * kH) {
-        const int hh = i % kH, v = (i / kH) % kSmallVocab, k = i / (kH * kSmallVocab);
-        if (v != kDomEdge) dEWfull[((size_t)k * kEdgeVocab + v) * kH + hh] += tE[i];
+    if (i < num_bins * H) dP[i] = tP[i];
+    if (i < H) dt[i] = tT[i];
+    if (i < hops * kSmallVocab * H) {
+        const int hh = i % H, v = (i / H) % kSmallVocab, k = i / (H * kSmallVocab);
+        if (v != kDomEdge) dEWfull[((size_t)k * kEdgeVocab + v) * H + hh] += tE[i];
     }
     const int wid = i >> 5, lane = i & 31;
-    if (wid < hops * kH) {                                  // warp-uniform
-        const int k = wid / kH, hh = wid % kH;
+    if (wid < hops * H) {                                  // warp-uniform
+        const int k = wid / H, hh = wid % H;
         float s = 0.f;
         for (int row = lane; row < pl.Rrows; row += 32) {
             const int rp = (row == pl.Rrows - 1) ? 511 : row;
-            if (expected_walk(rp, dk) > k) s += tR[row * kH + hh] / (float)min(max(rp - 1, 1), dk);
+            if (expected_walk(rp, dk) > k) s += tR[row * H + hh] / (float)min(max(rp - 1, 1), dk);
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
         if (lane == 0)
-            dEWfull[((size_t)k * kEdgeVocab + kDomEdge) * kH + hh] += s + tE[(k * kSmallVocab + kDomEdge) * kH + hh];
+            dEWfull[((size_t)k * kEdgeVocab + kDomEdge) * H + hh] += s + tE[(k * kSmallVocab + kDomEdge) * H + hh];
     }
 }
 
 // dE[v][h'] = sum_k sum_h dEW[k][v][h] W[k][h'][h] ;  dW[k][h'][h] = sum_v E[v][h'] dEW[k][v][h]
+template <int H>
 __global__ void k2_bias_bwd_finish_kernel(const float *__restrict__ dEW, const float *__restrict__ E,
                                           const float *__restrict__ W, int hops, float *__restrict__ dE,
                                           float *__restrict__ dW) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    const int nE = kEdgeVocab * kH, nW = hops * kH * kH;
+    const int nE = kEdgeVocab * H, nW = hops * H * H;
     if (idx < nE) {
-        const int v = idx / kH, hp = idx % kH;
+        const int v = idx / H, hp = idx % H;
         float acc = 0.f;
         for (int k = 0; k < hops; ++k)
 #pragma unroll
-            for (int h = 0; h < kH; ++h) acc += dEW[((size_t)k * kEdgeVocab + v) * kH + h] * W[(k * kH + hp) * kH + h];
+            for (int h = 0; h < H; ++h) acc += dEW[((size_t)k * kEdgeVocab + v) * H + h] * W[(k * H + hp) * H + h];
         dE[idx] = (v == 0) ? 0.f : acc;   // padding_idx row
     } else if (idx < nE + nW) {
         const int j = idx - nE;
-        const int h = j % kH, hp = (j / kH) % kH, k = j / (kH * kH);
+        const int h = j % H, hp = (j / H) % H, k = j / (H * H);
         float acc = 0.f;
-        for (int v = 0; v < kEdgeVocab; ++v) acc += E[v * kH + hp] * dEW[((size_t)k * kEdgeVocab + v) * kH + h];
+        for (int v = 0; v < kEdgeVocab; ++v) acc += E[v * H + hp] * dEW[((size_t)k * kEdgeVocab + v) * H + h];
         dW[j] = acc;
     }
 }
@@ -672,35 +738,27 @@ __global__ void k2_bias_bwd_finish_kernel(const float *__restrict__ dEW, const f
 
 using namespace mobgt;
 
+// head counts the kernels are instantiated for (K2Heads); any other value is MOBGT_ERR_UNSUPPORTED
+static bool k2_heads_built(int H) { return H == 8 || H == 12; }
+
 extern "C" int64_t mobgt_bias_fwd_workspace_bytes(int32_t hops, int32_t H) {
-    if (H != kH || hops < 4 || hops > MOBGT_MAX_HOPS || hops % 4 != 0) return -1;
-    return (int64_t)(hops * kEdgeVocab + kRelRows) * kH * (int64_t)sizeof(float);
+    if (!k2_heads_built(H) || hops < 4 || hops > MOBGT_MAX_HOPS || hops % 4 != 0) return -1;
+    return (int64_t)(hops * kEdgeVocab + kRelRows) * H * (int64_t)sizeof(float);
 }
 
-extern "C" int32_t mobgt_bias_fwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
-                                  const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t H,
-                                  int32_t rel_pos_max, int32_t num_bins, const float *R, const float *Ppos, const float *E,
-                                  const float *W, const float *tvd, void *workspace, void *out, int32_t out_dtype,
-                                  void *stream) {
-    MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && edge_in && R && Ppos && E && W && tvd && workspace && out,
-                  MOBGT_ERR_NULL, "mobgt_bias_fwd: null pointer");
-    MOBGT_REQUIRE(H == kH, MOBGT_ERR_UNSUPPORTED, "mobgt_bias_fwd: num_heads=%d (only 8 is built)", H);
-    MOBGT_REQUIRE(hops >= 4 && hops <= MOBGT_MAX_HOPS && hops % 4 == 0, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_bias_fwd: hops=%d must be a multiple of 4 in [4,%d]", hops, MOBGT_MAX_HOPS);
-    MOBGT_REQUIRE(dk >= 1 && dk <= hops, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: dk=%d outside [1, hops=%d]", dk, hops);
-    MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: num_bins=%d", num_bins);
-    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: T=%d Tp=%d", T, Tp);
-    MOBGT_REQUIRE(out_dtype == MOBGT_F32 || out_dtype == MOBGT_BF16, MOBGT_ERR_BAD_DTYPE, "mobgt_bias_fwd: dtype");
-    if (B <= 0) return MOBGT_OK;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    float *EW = static_cast<float *>(workspace);                 // [hops][128][8] then RL [512][8]
-    const int tabn = hops * kEdgeVocab * kH;
+template <int H>
+static int32_t bias_fwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                        const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t rel_pos_max,
+                        int32_t num_bins, const float *R, const float *Ppos, const float *E, const float *W, const float *tvd,
+                        void *workspace, void *out, int32_t out_dtype, cudaStream_t s) {
+    float *EW = static_cast<float *>(workspace);                 // [hops][128][H] then RL [512][H]
+    const int tabn = hops * kEdgeVocab * H;
     float *RL = EW + tabn;
-    k2_prep_kernel<<<ceil_div(tabn + kRelRows * kH, 256), 256, 0, s>>>(E, W, R, hops, dk, rel_pos_max, EW, RL);
+    k2_prep_kernel<H><<<ceil_div(tabn + kRelRows * H, 256), 256, 0, s>>>(E, W, R, hops, dk, rel_pos_max, EW, RL);
     MOBGT_LAUNCH_OK("k2_prep_kernel");
     K2Common c{n, sq_off, rel_pos, poi_pos, edge_in, B, T, Tp, hops, rel_pos_max, dk};
-    const size_t smem = (size_t)(kRelRows * kH + num_bins * kH + (hops + 1) * 8) * sizeof(float);
-    const int tiles_total = ceil_div(T * (Tp / 2), 512) * B;
+    const size_t smem = (size_t)(kRelRows * H + num_bins * H + (hops + 1) * 8) * sizeof(float);
+    const int tiles_total = ceil_div(T * (Tp / K2FwdCells<H>::kCells), 512) * B;
     dim3 grid((unsigned)min(2 * kNumSMs, tiles_total));
     auto launch = [&](auto kern, auto *o) -> int32_t {
         MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -708,10 +766,10 @@ extern "C" int32_t mobgt_bias_fwd(const int32_t *n, const int64_t *sq_off, const
         return MOBGT_OK;
     };
     int32_t rc = MOBGT_OK;
-#define MOBGT_K2_CASE(HW)                                                                                             \
-    case HW:                                                                                                          \
-        rc = (out_dtype == MOBGT_F32) ? launch(k2_bias_fwd_kernel<float, HW>, static_cast<float *>(out))              \
-                                      : launch(k2_bias_fwd_kernel<__nv_bfloat16, HW>, static_cast<__nv_bfloat16 *>(out)); \
+#define MOBGT_K2_CASE(HW)                                                                                                \
+    case HW:                                                                                                             \
+        rc = (out_dtype == MOBGT_F32) ? launch(k2_bias_fwd_kernel<H, float, HW>, static_cast<float *>(out))              \
+                                      : launch(k2_bias_fwd_kernel<H, __nv_bfloat16, HW>, static_cast<__nv_bfloat16 *>(out)); \
         break;
     switch (hops / 4) {
         MOBGT_K2_CASE(1) MOBGT_K2_CASE(2) MOBGT_K2_CASE(3) MOBGT_K2_CASE(4) MOBGT_K2_CASE(5) MOBGT_K2_CASE(6) MOBGT_K2_CASE(7)
@@ -724,52 +782,72 @@ extern "C" int32_t mobgt_bias_fwd(const int32_t *n, const int64_t *sq_off, const
     return MOBGT_OK;
 }
 
+extern "C" int32_t mobgt_bias_fwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                                  const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t H,
+                                  int32_t rel_pos_max, int32_t num_bins, const float *R, const float *Ppos, const float *E,
+                                  const float *W, const float *tvd, void *workspace, void *out, int32_t out_dtype,
+                                  void *stream) {
+    MOBGT_REQUIRE(k2_heads_built(H), MOBGT_ERR_UNSUPPORTED, "mobgt_bias_fwd: num_heads=%d is not built (8 and 12 heads)", H);
+    MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && edge_in && R && Ppos && E && W && tvd && workspace && out,
+                  MOBGT_ERR_NULL, "mobgt_bias_fwd: null pointer");
+    MOBGT_REQUIRE(hops >= 4 && hops <= MOBGT_MAX_HOPS && hops % 4 == 0, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_fwd: hops=%d must be a multiple of 4 in [4,%d]", hops, MOBGT_MAX_HOPS);
+    MOBGT_REQUIRE(dk >= 1 && dk <= hops, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: dk=%d outside [1, hops=%d]", dk, hops);
+    MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: num_bins=%d", num_bins);
+    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE(out_dtype == MOBGT_F32 || out_dtype == MOBGT_BF16, MOBGT_ERR_BAD_DTYPE, "mobgt_bias_fwd: dtype");
+    if (B <= 0) return MOBGT_OK;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    auto f = H == 8 ? bias_fwd<8> : bias_fwd<12>;
+    return f(n, sq_off, rel_pos, poi_pos, edge_in, B, T, Tp, hops, dk, rel_pos_max, num_bins, R, Ppos, E, W, tvd, workspace, out,
+             out_dtype, s);
+}
+
 // 64-bit words of the fixed-point rare-path tables: per-CTA EWsmall | launch-wide dEW | rel_pos overflow rows
+template <int H>
 static int64_t k2_bwd_fx_words(int hops, const K2BwdPlan &pl) {
-    return (int64_t)kNumSMs * pl.nEWs + (int64_t)hops * kEdgeVocab * kH + (int64_t)kRelRows * kH;
+    return (int64_t)kNumSMs * pl.nEWs + (int64_t)hops * kEdgeVocab * H + (int64_t)kRelRows * H;
+}
+
+template <int H>
+static int64_t bias_bwd_workspace_bytes(int32_t T, int32_t hops, int32_t num_bins) {
+    if (T < 2 || hops < 4 || hops > MOBGT_MAX_HOPS || num_bins < 1 || num_bins > 1024) return -1;
+    const K2BwdPlan pl = k2_bwd_plan<H>(T, round_up(T, 8), hops, num_bins);
+    return ((int64_t)hops * kEdgeVocab * H + (int64_t)(kNumSMs + 1) * pl.stride) * (int64_t)sizeof(float) + 16 +
+           k2_bwd_fx_words<H>(hops, pl) * (int64_t)sizeof(long long);
 }
 
 extern "C" int64_t mobgt_bias_bwd_workspace_bytes(int32_t T, int32_t hops, int32_t num_bins) {
-    if (T < 2 || hops < 4 || hops > MOBGT_MAX_HOPS || num_bins < 1 || num_bins > 1024) return -1;
-    const K2BwdPlan pl = k2_bwd_plan(T, round_up(T, 8), hops, num_bins);
-    return ((int64_t)hops * kEdgeVocab * kH + (int64_t)(kNumSMs + 1) * pl.stride) * (int64_t)sizeof(float) + 16 +
-           k2_bwd_fx_words(hops, pl) * (int64_t)sizeof(long long);
+    return bias_bwd_workspace_bytes<8>(T, hops, num_bins);
 }
 
-extern "C" int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
-                                  const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t H,
-                                  int32_t rel_pos_max, int32_t num_bins, const void *dBias, int32_t dbias_dtype,
-                                  int32_t n_layers, int64_t layer_stride, const float *E, const float *W,
-                                  void *workspace, int64_t workspace_bytes, float *dR, float *dPpos, float *dE, float *dW,
-                                  float *dtvd, void *stream) {
-    MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && edge_in && dBias && E && W && workspace && dR && dPpos && dE && dW && dtvd,
-                  MOBGT_ERR_NULL, "mobgt_bias_bwd: null pointer");
-    MOBGT_REQUIRE(H == kH, MOBGT_ERR_UNSUPPORTED, "mobgt_bias_bwd: num_heads=%d (only 8 is built)", H);
-    MOBGT_REQUIRE(hops >= 4 && hops <= MOBGT_MAX_HOPS && hops % 4 == 0 && num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_bias_bwd: hops=%d num_bins=%d", hops, num_bins);
-    MOBGT_REQUIRE(dk >= 1 && dk <= hops, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: dk=%d outside [1, hops=%d]", dk, hops);
-    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: T=%d Tp=%d", T, Tp);
-    MOBGT_REQUIRE((dbias_dtype == MOBGT_F32 && n_layers == 1) || (dbias_dtype == MOBGT_BF16 && n_layers >= 1 && n_layers <= 64),
-                  MOBGT_ERR_BAD_DTYPE, "mobgt_bias_bwd: dbias dtype %d with %d layer planes", dbias_dtype, n_layers);
-    MOBGT_REQUIRE(((uintptr_t)dBias & 15) == 0 && (dbias_dtype == MOBGT_F32 || layer_stride % 8 == 0), MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_bias_bwd: dBias planes must be 16-byte aligned");
-    const K2BwdPlan pl = k2_bwd_plan(T, Tp, hops, num_bins);
+extern "C" int64_t mobgt_bias_bwd_heads_workspace_bytes(int32_t T, int32_t hops, int32_t num_bins, int32_t H) {
+    if (!k2_heads_built(H)) return -1;
+    return H == 8 ? bias_bwd_workspace_bytes<8>(T, hops, num_bins) : bias_bwd_workspace_bytes<12>(T, hops, num_bins);
+}
+
+template <int H>
+static int32_t bias_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                        const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t rel_pos_max,
+                        int32_t num_bins, const void *dBias, int32_t dbias_dtype, int32_t n_layers, int64_t layer_stride,
+                        const float *E, const float *W, void *workspace, int64_t workspace_bytes, float *dR, float *dPpos,
+                        float *dE, float *dW, float *dtvd, cudaStream_t s) {
+    const K2BwdPlan pl = k2_bwd_plan<H>(T, Tp, hops, num_bins);
     MOBGT_REQUIRE(pl.warps >= 1, MOBGT_ERR_UNSUPPORTED, "mobgt_bias_bwd: no shared-memory plan for T=%d bins=%d", T, num_bins);
-    const int64_t nEW = (int64_t)hops * kEdgeVocab * kH;
+    const int64_t nEW = (int64_t)hops * kEdgeVocab * H;
     const int64_t nfloat = nEW + (int64_t)(kNumSMs + 1) * pl.stride;
     const int64_t fx_off = (nfloat * (int64_t)sizeof(float) + 15) / 16 * 16;
-    const int64_t need = fx_off + k2_bwd_fx_words(hops, pl) * (int64_t)sizeof(long long);
+    const int64_t need = fx_off + k2_bwd_fx_words<H>(hops, pl) * (int64_t)sizeof(long long);
     MOBGT_REQUIRE(workspace_bytes >= need, MOBGT_ERR_WORKSPACE_TOO_SMALL, "mobgt_bias_bwd: workspace %lld < %lld bytes",
                   (long long)workspace_bytes, (long long)need);
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    float *dEWfull = static_cast<float *>(workspace);      // [hops][128][8], then [stride] totals, then [kNumSMs][stride] partials
+    float *dEWfull = static_cast<float *>(workspace);      // [hops][128][H], then [stride] totals, then [kNumSMs][stride] partials
     float *tot = dEWfull + nEW;
     float *partial = tot + pl.stride;
     MOBGT_REQUIRE(((uintptr_t)workspace & 15) == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: workspace must be 16-byte aligned");
     long long *ews64 = reinterpret_cast<long long *>(static_cast<char *>(workspace) + fx_off);   // [kNumSMs][nEWs]
-    long long *dEWfull64 = ews64 + (size_t)kNumSMs * pl.nEWs;                                     // [hops][128][8]
-    long long *dR64 = dEWfull64 + nEW;                                                            // [512][8]
-    MOBGT_CUDA_OK(cudaMemsetAsync(ews64, 0, (size_t)k2_bwd_fx_words(hops, pl) * sizeof(long long), s));
+    long long *dEWfull64 = ews64 + (size_t)kNumSMs * pl.nEWs;                                     // [hops][128][H]
+    long long *dR64 = dEWfull64 + nEW;                                                            // [512][H]
+    MOBGT_CUDA_OK(cudaMemsetAsync(ews64, 0, (size_t)k2_bwd_fx_words<H>(hops, pl) * sizeof(long long), s));
     const int nparts = B > 0 ? kNumSMs : 0;
     if (B > 0) {
         K2Common c{n, sq_off, rel_pos, poi_pos, edge_in, B, T, Tp, hops, rel_pos_max, dk};
@@ -783,8 +861,9 @@ extern "C" int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const
 #define MOBGT_K2B_CASE(HW)                                                                                                   \
     case HW:                                                                                                                 \
         rc = (dbias_dtype == MOBGT_F32)                                                                                      \
-                 ? launch(k2_bias_bwd_kernel<float, HW>, static_cast<const float *>(dBias), 1, (int64_t)0)                   \
-                 : launch(k2_bias_bwd_kernel<__nv_bfloat16, HW>, static_cast<const __nv_bfloat16 *>(dBias), n_layers, layer_stride); \
+                 ? launch(k2_bias_bwd_kernel<H, float, HW>, static_cast<const float *>(dBias), 1, (int64_t)0)                \
+                 : launch(k2_bias_bwd_kernel<H, __nv_bfloat16, HW>, static_cast<const __nv_bfloat16 *>(dBias), n_layers,     \
+                          layer_stride);                                                                                     \
         break;
         switch (hops / 4) {
             MOBGT_K2B_CASE(1) MOBGT_K2B_CASE(2) MOBGT_K2B_CASE(3) MOBGT_K2B_CASE(4) MOBGT_K2B_CASE(5) MOBGT_K2B_CASE(6)
@@ -795,12 +874,35 @@ extern "C" int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const
         if (rc) return rc;
         MOBGT_LAUNCH_OK("k2_bias_bwd_kernel");
     }
-    k2_bias_bwd_reduce_kernel<<<ceil_div(pl.stride + (int)nEW + kRelRows * kH, 256), 256, 0, s>>>(
+    k2_bias_bwd_reduce_kernel<H><<<ceil_div(pl.stride + (int)nEW + kRelRows * H, 256), 256, 0, s>>>(
         partial, nparts, pl.stride, pl.nEWs, ews64, tot, dEWfull64, (int)nEW, dEWfull, dR64, dR);
     MOBGT_LAUNCH_OK("k2_bias_bwd_reduce_kernel");
-    k2_bias_bwd_scatter_kernel<<<ceil_div(max(max(kRelRows, num_bins) * kH, hops * kH * 32), 256), 256, 0, s>>>(tot, pl, hops, dk, num_bins, dEWfull, dR, dPpos, dtvd);
+    k2_bias_bwd_scatter_kernel<H><<<ceil_div(max(max(kRelRows, num_bins) * H, hops * H * 32), 256), 256, 0, s>>>(
+        tot, pl, hops, dk, num_bins, dEWfull, dR, dPpos, dtvd);
     MOBGT_LAUNCH_OK("k2_bias_bwd_scatter_kernel");
-    k2_bias_bwd_finish_kernel<<<ceil_div(kEdgeVocab * kH + hops * kH * kH, 256), 256, 0, s>>>(dEWfull, E, W, hops, dE, dW);
+    k2_bias_bwd_finish_kernel<H><<<ceil_div(kEdgeVocab * H + hops * H * H, 256), 256, 0, s>>>(dEWfull, E, W, hops, dE, dW);
     MOBGT_LAUNCH_OK("k2_bias_bwd_finish_kernel");
     return MOBGT_OK;
+}
+
+extern "C" int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                                  const uint8_t *edge_in, int32_t B, int32_t T, int32_t Tp, int32_t hops, int32_t dk, int32_t H,
+                                  int32_t rel_pos_max, int32_t num_bins, const void *dBias, int32_t dbias_dtype,
+                                  int32_t n_layers, int64_t layer_stride, const float *E, const float *W,
+                                  void *workspace, int64_t workspace_bytes, float *dR, float *dPpos, float *dE, float *dW,
+                                  float *dtvd, void *stream) {
+    MOBGT_REQUIRE(k2_heads_built(H), MOBGT_ERR_UNSUPPORTED, "mobgt_bias_bwd: num_heads=%d is not built (8 and 12 heads)", H);
+    MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && edge_in && dBias && E && W && workspace && dR && dPpos && dE && dW && dtvd,
+                  MOBGT_ERR_NULL, "mobgt_bias_bwd: null pointer");
+    MOBGT_REQUIRE(hops >= 4 && hops <= MOBGT_MAX_HOPS && hops % 4 == 0 && num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_bwd: hops=%d num_bins=%d", hops, num_bins);
+    MOBGT_REQUIRE(dk >= 1 && dk <= hops, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: dk=%d outside [1, hops=%d]", dk, hops);
+    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE((dbias_dtype == MOBGT_F32 && n_layers == 1) || (dbias_dtype == MOBGT_BF16 && n_layers >= 1 && n_layers <= 64),
+                  MOBGT_ERR_BAD_DTYPE, "mobgt_bias_bwd: dbias dtype %d with %d layer planes", dbias_dtype, n_layers);
+    MOBGT_REQUIRE(((uintptr_t)dBias & 15) == 0 && (dbias_dtype == MOBGT_F32 || layer_stride % 8 == 0), MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_bwd: dBias planes must be 16-byte aligned");
+    auto f = H == 8 ? bias_bwd<8> : bias_bwd<12>;
+    return f(n, sq_off, rel_pos, poi_pos, edge_in, B, T, Tp, hops, dk, rel_pos_max, num_bins, dBias, dbias_dtype, n_layers,
+             layer_stride, E, W, workspace, workspace_bytes, dR, dPpos, dE, dW, dtvd, static_cast<cudaStream_t>(stream));
 }

@@ -23,8 +23,9 @@ from . import ops
 from .lr import PolynomialDecayLR
 
 NODE_DIM = 2000    # model_fqandtoyo.py:567
-# (num_heads, hidden_dim) pairs the kernels are built for: K2 is built for 8 heads, K3 for head dims (hidden_dim + 64) / 8 = 16, 24
-SUPPORTED_SHAPES = frozenset({(8, 64), (8, 128)})
+# (num_heads, hidden_dim) pairs the kernels are built for: K2 is built for 8 and 12 heads, K3 for head dims
+# (hidden_dim + 64) / num_heads = 16, 24.  Each pair also fixes the final LayerNorm / K5 head width 2 * hidden_dim + 64.
+SUPPORTED_SHAPES = frozenset({(8, 64), (8, 128), (12, 128)})
 
 DATASET_TRAITS = {
     # per-dataset constructor differences (model_fqandtoyo.py:636-779, 781-900, 902-1029)
@@ -267,8 +268,9 @@ class Graphormer(nn.Module):
             raise NotImplementedError(
                 f"num_heads={num_heads}, hidden_dim={hidden_dim}: libmobgt is built for (num_heads, hidden_dim) in "
                 f"{sorted(SUPPORTED_SHAPES)}. The encoder width is hidden_dim + 64 (time and category embeddings), split over the "
-                f"heads: the attention-bias kernels (K2) are built for 8 heads, and the attention kernels (K3) for head dims "
-                f"{ops.HEAD_DIMS[0]} and {ops.HEAD_DIMS[1]}, i.e. hidden_dim 64 or 128 at 8 heads.")
+                f"heads: the attention-bias kernels (K2) are built for 8 heads and for 12 heads, and the attention kernels (K3) "
+                f"for head dims {ops.HEAD_DIMS[0]} and {ops.HEAD_DIMS[1]}, i.e. hidden_dim 64 or 128 at 8 heads and hidden_dim "
+                f"128 at 12 heads.")
         if edge_type != "multi_hop":
             raise NotImplementedError("edge_type must be 'multi_hop' (README.md:62)")
         tr = DATASET_TRAITS[dataset_name]

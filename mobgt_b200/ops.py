@@ -8,7 +8,8 @@ import torch
 from . import _C
 
 F32, BF16 = 0, 1
-NUM_HEADS = 8
+NUM_HEADS = 8            # the canonical shape's head count
+BIAS_HEADS = (8, 12)     # head counts the attention-bias kernels are built for (csrc/k2_bias.cu K2Heads)
 HEAD_DIM = 24            # the canonical shape's head dim (hidden 128: (128 + 64) / 8)
 HEAD_DIMS = (16, 24)     # head dims the attention kernels are built for (csrc/k3_small.cuh AttnShape)
 
@@ -58,9 +59,9 @@ def bias_bwd_raw(batch, dbias, E, W, num_bins):
         L, dt, stride = 1, F32, 0
     dev = dbias.device
     hops = batch.hops
-    ws_bytes = int(_C.lib().mobgt_bias_bwd_workspace_bytes(T, hops, num_bins))
+    ws_bytes = int(_C.lib().mobgt_bias_bwd_heads_workspace_bytes(T, hops, num_bins, H))
     if ws_bytes < 0:
-        raise _C.MobgtError(f"mobgt_bias_bwd_workspace_bytes rejected T={T} hops={hops} num_bins={num_bins}")
+        raise _C.MobgtError(f"mobgt_bias_bwd_heads_workspace_bytes rejected T={T} hops={hops} num_bins={num_bins} H={H}")
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     dR = torch.empty(512, H, dtype=torch.float32, device=dev)
     dP = torch.empty(num_bins, H, dtype=torch.float32, device=dev)

@@ -1,14 +1,16 @@
-"""Head dim 16 against head dim 24: the canonical 6-layer model (ffn 1024, 8 heads) at hidden_dim 128 (d = 24) and at hidden_dim 64
-(d = 16), on the c2-dense128 and c2-natural batches of bench.py (256 graphs, toyotagraph-shaped world of 60 000 POIs).
+"""The built encoder shapes against each other: the canonical 6-layer model (ffn 1024) at 8 heads x hidden_dim 128 (d = 24),
+8 heads x hidden_dim 64 (d = 16) and 12 heads x hidden_dim 128 (d = 16), on the c2-dense128 and c2-natural batches of bench.py
+(256 graphs, toyotagraph-shaped world of 60 000 POIs).
 
-    python scripts/bench_head_dim.py OUT_DIR [--steps 20] [--warmup 5] [--iters 20]
+    python scripts/bench_head_dim.py OUT_DIR [--steps 20] [--warmup 5] [--iters 20] [--shapes 8x128,8x64,12x128]
 
-For every (workload, hidden_dim) it reports, as OUT_DIR/bench_head_dim.json (one JSON object) and one line per case on stdout:
+For every (workload, shape) it reports, as OUT_DIR/bench_head_dim.json (one JSON object) and one line per case on stdout:
   * step: ms / step and graphs / s of the replayed training step (trainer.Trainer with CUDA graphs, as bench.py times it);
   * k3: one layer's attention forward and backward (mode 2: the per-layer bf16 dS plane the training step writes), dropout on
     (p = 0.1), CUDA events around each launch with the L2 overwritten (a 256 MB buffer zeroed) before it; mean ms over --iters;
+  * k2: the attention-bias build (bf16 bias, once per step) and its backward from the n_layers bf16 dS planes, same timer;
   * bytes: what one K3 launch must move at these shapes (the live bias cells and q / k / v / out / lse, plus dout / o / dq / dk /
-    dv and the dS plane in the backward), and the resulting GB/s;
+    dv and the dS plane in the backward), the live bias bytes per layer, and the resulting GB/s;
   * the card's name and power limit, read in the same run.
 The numbers are only meaningful with a GPU: without one the script stops."""
 import argparse
@@ -46,7 +48,7 @@ def k3_bytes(batch, d, H=8):
     return fwd, bwd
 
 
-def run_case(workload, hidden_dim, args, flush):
+def run_case(workload, num_heads, hidden_dim, args, flush):
     from mobgt_b200 import collator, model as M, ops
     from mobgt_b200.trainer import Trainer
     dev = torch.device("cuda")
@@ -55,7 +57,7 @@ def run_case(workload, hidden_dim, args, flush):
     B = args.batch
     item_sets = [bench.make_workload(workload, world, B, 0, batch_id=i) for i in range(nbatches)]
     torch.manual_seed(1)
-    hp = dict(bench.HP, hidden_dim=hidden_dim)
+    hp = dict(bench.HP, hidden_dim=hidden_dim, num_heads=num_heads)
     model = M.Graphormer(dataset_name=ds, world=world, **hp).to(dev).train()
     tr = Trainer(model, dev, 1, cuda_graph=True)
     latlon = torch.from_numpy(world.latlon).to(dev)
@@ -82,14 +84,15 @@ def run_case(workload, hidden_dim, args, flush):
 
     # one layer's K3 at the first batch's shapes, dropout on, L2 overwritten before every launch
     b = batches[0]
-    d = (hidden_dim + 64) // 8
+    H = num_heads
+    d = (hidden_dim + 64) // H
     tabs = [t.detach().float().contiguous() for t in (model.rel_pos_encoder.weight, model.poi_pos_encoder.weight,
                                                        model.edge_encoder.weight, model.edge_dis_encoder.weight.view(-1),
                                                        model.graph_token_virtual_distance.weight.view(-1))]
     bias = ops.bias_fwd_raw(b, *tabs)
     ntok = int(b.tok_pos.numel())
-    qkv = torch.randn(ntok, 3 * 8 * d, device=dev).to(torch.bfloat16)
-    dout = torch.randn(ntok, 8 * d, device=dev).to(torch.bfloat16)
+    qkv = torch.randn(ntok, 3 * H * d, device=dev).to(torch.bfloat16)
+    dout = torch.randn(ntok, H * d, device=dev).to(torch.bfloat16)
     dp, sd = hp["attention_dropout_rate"], 0x5DEECE66D1234567
     out, lse = ops.attn_fwd_raw(qkv, bias, b, drop_p=dp, seed=sd)
     plane = torch.empty(tuple(bias.shape), dtype=torch.bfloat16, device=dev)
@@ -97,13 +100,23 @@ def run_case(workload, hidden_dim, args, flush):
     t_f = bench.time_kernel(lambda: ops.attn_fwd_raw(qkv, bias, b, scale=scale, drop_p=dp, seed=sd), flush, iters=args.iters)
     t_b = bench.time_kernel(lambda: ops.attn_bwd_raw(qkv, bias, out, dout, lse, b, plane, 2, scale=scale, drop_p=dp, seed=sd),
                             flush, iters=args.iters)
-    fb, bb = k3_bytes(b, d)
+    fb, bb = k3_bytes(b, d, H)
+    # K2 at the same batch: the forward writes the bf16 bias, the backward sums the n_layers bf16 dS planes
+    planes = torch.randn((hp["n_layers"],) + tuple(bias.shape), device=dev).to(torch.bfloat16)
+    bins = tabs[1].shape[0]
+    t_k2f = bench.time_kernel(lambda: ops.bias_fwd_raw(b, *tabs), flush, iters=args.iters)
+    t_k2b = bench.time_kernel(lambda: ops.bias_bwd_raw(b, planes, tabs[2], tabs[3], bins), flush, iters=args.iters)
     n = b.n_host
-    return dict(workload=workload, hidden_dim=hidden_dim, head_dim=d, n_layers=hp["n_layers"], ffn_dim=hp["ffn_dim"],
+    live = int(((n.astype(np.int64) + 1) ** 2).sum())
+    bias_bytes = 2 * live * H                      # live bf16 bias cells of one layer (= one dS plane)
+    return dict(workload=workload, num_heads=H, hidden_dim=hidden_dim, head_dim=d, n_layers=hp["n_layers"], ffn_dim=hp["ffn_dim"],
                 graphs_per_step=B, tokens=ntok, nodes_max=int(n.max()), nodes_median=float(np.median(n)), padded=bool(getattr(b, "padded", False)),
                 step=dict(ms=ms, graphs_per_s=B * 1e3 / ms, steps=args.steps, graph_replays=replays, loss=loss),
                 k3=dict(fwd_ms=t_f, bwd_ms=t_b, fwd_bytes=fb, bwd_bytes=bb, fwd_gbs=fb / t_f / 1e6, bwd_gbs=bb / t_b / 1e6,
-                        iters=args.iters, dropout=dp, l2="256 MB buffer zeroed before every launch"))
+                        iters=args.iters, dropout=dp, l2="256 MB buffer zeroed before every launch"),
+                k2=dict(fwd_ms=t_k2f, bwd_ms=t_k2b, bias_bytes_per_layer=bias_bytes, bwd_planes=hp["n_layers"],
+                        fwd_gbs=bias_bytes / t_k2f / 1e6, bwd_gbs=hp["n_layers"] * bias_bytes / t_k2b / 1e6, iters=args.iters,
+                        l2="256 MB buffer zeroed before every launch"))
 
 
 def main():
@@ -114,7 +127,7 @@ def main():
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--batch", type=int, default=256)
     ap.add_argument("--workloads", default="c2-dense128,c2-natural")
-    ap.add_argument("--hidden", default="128,64")
+    ap.add_argument("--shapes", default="8x128,8x64,12x128", help="num_heads x hidden_dim, comma-separated")
     args = ap.parse_args()
     from mobgt_b200 import _C
     _C.require_cuda()
@@ -122,12 +135,14 @@ def main():
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
     res = dict(card=card(), cases=[])
     for wl in args.workloads.split(","):
-        for hd in (int(x) for x in args.hidden.split(",")):
-            r = run_case(wl, hd, args, flush)
+        for nh, hd in (map(int, x.split("x")) for x in args.shapes.split(",")):
+            r = run_case(wl, nh, hd, args, flush)
             res["cases"].append(r)
-            print(json.dumps(dict(workload=wl, hidden_dim=hd, step_ms=round(r["step"]["ms"], 3),
+            print(json.dumps(dict(workload=wl, num_heads=nh, hidden_dim=hd, step_ms=round(r["step"]["ms"], 3),
                                   graphs_per_s=round(r["step"]["graphs_per_s"], 1), k3_fwd_ms=round(r["k3"]["fwd_ms"], 4),
-                                  k3_bwd_ms=round(r["k3"]["bwd_ms"], 4))), flush=True)
+                                  k3_bwd_ms=round(r["k3"]["bwd_ms"], 4), k2_fwd_ms=round(r["k2"]["fwd_ms"], 4),
+                                  k2_bwd_ms=round(r["k2"]["bwd_ms"], 4), bias_mb=round(r["k2"]["bias_bytes_per_layer"] / 1e6, 2))),
+                  flush=True)
     with open(os.path.join(args.out_dir, "bench_head_dim.json"), "w") as f:
         json.dump(res, f, indent=1)
     print(json.dumps(res["card"]))
