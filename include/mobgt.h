@@ -140,6 +140,31 @@ int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *r
                        int64_t layer_stride, const float *E, const float *W, void *workspace, int64_t workspace_bytes,
                        float *dR, float *dPpos, float *dE, float *dW, float *dtvd, void *stream);
 
+/* K2, direct edge encoding (Graphormer's encoding for any edge_type other than multi_hop): the edge term of a pair is
+ * E[f][h] with f = attn_edge_type of the pair, instead of the walk mean through edge_dis_encoder.
+ *   bias[g,h,a,b] = R[rel_pos][h] + Ppos[poi_pos][h] + E[feat][h]   (a, b >= 1; indices of pair (a-1, b-1));
+ *   column 0 of rows 1..n[g] = tvd[h]; row 0 = 0; -inf where rel_pos - 1 >= rel_pos_max; same [B,H,T,Tp] layout and
+ *   written cells as mobgt_bias_fwd.  H = 8 or 12; any other value returns MOBGT_ERR_UNSUPPORTED.
+ *   feat: packed u8 [sum n^2] (the batch's feat8 plane: 0 for no edge, else edge count + 2).
+ * Input domain (not checked on the device): feat in 0..127; rel_pos in 0..511; poi_pos in 0..num_bins-1.  E row 0 is read
+ *   for pairs without an edge (it need not be zero).
+ * Backward: dBias (one f32 buffer or n_layers bf16 planes layer_stride elements apart, as mobgt_bias_bwd) -> dR [512,H],
+ *   dPpos [bins,H], dE [128,H], dtvd [H] (all overwritten).  dE row 0 (edge_encoder's padding row) is 0: only pairs with
+ *   feat != 0 contribute to dE.  There is no edge_dis_encoder gradient.  The backward never reads a dBias cell outside a
+ *   graph's live (n[g]+1)^2 square, in row 0, or masked by rel_pos_max.  Bitwise reproducible (fixed-order histogram sums;
+ *   dE and rel_pos keys outside the histogram plan accumulate in 64-bit fixed point).  `workspace` must be 16-byte aligned. */
+int32_t mobgt_bias_direct_fwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                              const uint8_t *feat, int32_t B, int32_t T, int32_t Tp, int32_t H, int32_t rel_pos_max,
+                              int32_t num_bins, const float *R, const float *Ppos, const float *E, const float *tvd, void *out,
+                              int32_t out_dtype, void *stream);
+/* bytes of `workspace` mobgt_bias_direct_bwd needs; < 0 on bad arguments or a head count other than 8 and 12 */
+int64_t mobgt_bias_direct_bwd_workspace_bytes(int32_t T, int32_t num_bins, int32_t H);
+int32_t mobgt_bias_direct_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                              const uint8_t *feat, int32_t B, int32_t T, int32_t Tp, int32_t H, int32_t rel_pos_max,
+                              int32_t num_bins, const void *dBias, int32_t dbias_dtype, int32_t n_layers, int64_t layer_stride,
+                              void *workspace, int64_t workspace_bytes, float *dR, float *dPpos, float *dE, float *dtvd,
+                              void *stream);
+
 /* ------------------------------------------------------------------------------------------
  * K3 — biased multi-head attention (tcgen05 / TMEM / TMA).  Replaces the core of
  * MultiHeadAttention.forward, model_fqandtoyo.py:1693-1706, for packed var-len graphs:

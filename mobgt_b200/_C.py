@@ -34,6 +34,10 @@ SIGNATURES = {
     "mobgt_bias_bwd_heads_workspace_bytes": [c_i32, c_i32, c_i32, c_i32],
     "mobgt_bias_bwd": [c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_p, c_i32, c_i32, c_i64, c_p,
                        c_p, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_p],
+    "mobgt_bias_direct_fwd": [c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_p, c_p, c_p, c_p, c_p, c_i32, c_p],
+    "mobgt_bias_direct_bwd_workspace_bytes": [c_i32, c_i32, c_i32],
+    "mobgt_bias_direct_bwd": [c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_p, c_i32, c_i32, c_i64, c_p, c_i64,
+                              c_p, c_p, c_p, c_p, c_p],
     "mobgt_attn_fwd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_f32, ctypes.c_uint64,
                        c_p, c_p, c_p, c_p],
     "mobgt_attn_bwd": [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_p,

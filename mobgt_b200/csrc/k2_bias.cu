@@ -375,6 +375,111 @@ __device__ __forceinline__ void sts_f32x4(uint32_t a, float x, float y, float z,
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(x), "f"(y), "f"(z), "f"(w) : "memory");
 }
 
+// Sum phase of one plane row (g, a) of the backward: dsum[h][b] = sum over layers of plane[l][g][h][a][b] for b < Tg, into the
+// warp's shared-memory strip (row pitch `pitch` floats).  The lanes take 16-byte chunks of the row (lane = 8-cell chunk of one
+// head), all layers of a chunk in flight together.
+template <int H, typename DT>
+__device__ __forceinline__ void k2_bwd_sum_row(const DT *__restrict__ rowbase, int Tg, int nlayers, int64_t layer_stride, size_t hs,
+                                               uint32_t s_dsum, uint32_t pitch4, int pitch, int lane) {
+    constexpr int kPer = 16 / (int)sizeof(DT);           // cells per 16-byte load
+    const int nitems = ceil_div(Tg, kPer) * H;           // item i = (chunk i / H, head i % H)
+    for (int i0 = 0; i0 < nitems; i0 += 32 * kSumItems) {
+        const int ns = min(kSumItems, (nitems - i0 + 31) >> 5);   // 32-item slots of this round that hold an item (warp-uniform)
+        float accv[kSumItems][8];
+#pragma unroll
+        for (int s = 0; s < kSumItems; ++s)
+#pragma unroll
+            for (int q = 0; q < 8; ++q) accv[s][q] = 0.f;
+        const DT *src[kSumItems];
+        bool ok[kSumItems];
+#pragma unroll
+        for (int s = 0; s < kSumItems; ++s) {
+            const int i = i0 + 32 * s + lane;
+            ok[s] = i < nitems;
+            const int ic = min(i, nitems - 1);           // lanes past the last item re-read it (no predicate on the loads)
+            src[s] = rowbase + (size_t)mod_h<H>(ic) * hs + div_h<H>(ic) * kPer;
+        }
+        for (int l0 = 0; l0 < nlayers; l0 += 6) {
+            uint4 v[kSumItems][6];
+            if (l0 + 6 <= nlayers) {
+#pragma unroll
+                for (int s = 0; s < kSumItems; ++s)
+                    if (s < ns) {
+                        const DT *pl0 = src[s] + (size_t)l0 * layer_stride;
+#pragma unroll
+                        for (int j = 0; j < 6; ++j) v[s][j] = __ldg(reinterpret_cast<const uint4 *>(pl0 + (size_t)j * layer_stride));
+                    }
+            } else {
+#pragma unroll
+                for (int s = 0; s < kSumItems; ++s)
+                    if (s < ns) {
+#pragma unroll
+                        for (int j = 0; j < 6; ++j)
+                            v[s][j] = (l0 + j < nlayers)
+                                          ? __ldg(reinterpret_cast<const uint4 *>(src[s] + (size_t)(l0 + j) * layer_stride))
+                                          : make_uint4(0u, 0u, 0u, 0u);
+                    }
+            }
+#pragma unroll
+            for (int s = 0; s < kSumItems; ++s)
+                if (s < ns) {
+#pragma unroll
+                    for (int j = 0; j < 6; ++j) {
+                        const uint32_t w4[4] = {v[s][j].x, v[s][j].y, v[s][j].z, v[s][j].w};
+                        if constexpr (sizeof(DT) == 4) {
+#pragma unroll
+                            for (int q = 0; q < 4; ++q) accv[s][q] += __uint_as_float(w4[q]);
+                        } else {
+#pragma unroll
+                            for (int q = 0; q < 4; ++q) {
+                                accv[s][2 * q] += bf16lo(w4[q]);
+                                accv[s][2 * q + 1] += __uint_as_float(w4[q] & 0xFFFF0000u);
+                            }
+                        }
+                    }
+                }
+        }
+#pragma unroll
+        for (int s = 0; s < kSumItems; ++s) {
+            const int i = i0 + 32 * s + lane;
+            if (ok[s]) {
+                const uint32_t dst = s_dsum + (uint32_t)mod_h<H>(i) * pitch4 + (uint32_t)(div_h<H>(i) * kPer) * 4u;
+                sts_f32x4(dst, accv[s][0], accv[s][1], accv[s][2], accv[s][3]);
+                if constexpr (sizeof(DT) == 2) {         // cells past the pitch lie beyond the graph's last token: never read
+                    if (div_h<H>(i) * kPer + 8 <= pitch) sts_f32x4(dst + 16u, accv[s][4], accv[s][5], accv[s][6], accv[s][7]);
+                }
+            }
+        }
+    }
+}
+
+// Histogram phase of one plane row: lane = (table, cell slot c2, head h) adds dsum[h][b] of adjacent cells b0 + 2 c2,
+// b0 + 2 c2 + 1 per step into the row of its table that cinfo[b] names (R row in the low 16 bits, P row in the high 16).
+// Cells without a gradient point at the trash rows, so the loop carries no predicates.
+template <int H>
+__device__ __forceinline__ void k2_bwd_hist_row(uint32_t s_cinfo, uint32_t s_dsum, uint32_t s_hist, uint32_t key_shift,
+                                                uint32_t pitch4, int Tg4, int lane, int c2, int h) {
+    constexpr int S = K2Heads<H>::kSlots;
+    constexpr uint32_t key_bytes = S * H * 4;
+    if (K2Heads<H>::kLanes == 32 || lane < K2Heads<H>::kLanes) {
+        uint32_t pi = s_cinfo + (uint32_t)c2 * 8u, pd = s_dsum + (uint32_t)h * pitch4 + (uint32_t)c2 * 8u;
+        for (int b0 = 0; b0 < Tg4; b0 += 2 * S, pi += 8u * S, pd += 8u * S) {
+            uint32_t iA, iB;
+            float dA, dB_;
+            asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(iA), "=r"(iB) : "r"(pi) : "memory");
+            asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(dA), "=f"(dB_) : "r"(pd) : "memory");
+            const uint32_t aA = s_hist + ((iA >> key_shift) & 0xFFFFu) * key_bytes;
+            const uint32_t aB = s_hist + ((iB >> key_shift) & 0xFFFFu) * key_bytes;
+            // two read-modify-writes in flight; equal addresses are chained in registers, the second store wins
+            const float vA = lds_f32(aA), vB = lds_f32(aB);
+            const float nA = vA + dA;
+            const float nB = ((aA == aB) ? nA : vB) + dB_;
+            sts_f32(aA, nA);
+            sts_f32(aB, nB);
+        }
+    }
+}
+
 template <int H, typename DT, int HOPW>
 __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(const K2Common c, const DT *__restrict__ dB, int nlayers,
                                                              int64_t layer_stride, int num_bins,
@@ -398,7 +503,6 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
     const uint32_t s_dlist = s_cdev + (uint32_t)pl.pitch * 4u;    // [pitch]: cells that need the slow path
     const uint32_t s_T = s_dlist + (uint32_t)pl.pitch * 4u;       // [H]
     const uint32_t s_hist = (ty ? s_hP : s_hR) + (uint32_t)(c2 * H + h) * 4u;       // + key * S * H * 4 B
-    constexpr uint32_t key_bytes = S * H * 4;
     const uint32_t key_shift = ty ? 16u : 0u;
     const uint32_t trashR = (uint32_t)pl.Rrows, trashP = (uint32_t)num_bins;
     constexpr int hopw = HOPW;                                   // 32-bit words per walk (hops / 4)
@@ -416,77 +520,7 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
         const int Tg = n + 1;
         const int64_t rowp = c.sq_off[g] + (int64_t)(a - 1) * n - 1;     // pair of cell b lives at rowp + b
         // ---- 1. sum phase: dsum[h][b] = sum over layers of plane[l][g][h][a][b]
-        const DT *rowbase = dB + ((size_t)g * H * c.T + a) * c.Tp;
-        constexpr int kPer = 16 / (int)sizeof(DT);           // cells per 16-byte load
-        const int nitems = ceil_div(Tg, kPer) * H;           // item i = (chunk i / H, head i % H)
-        for (int i0 = 0; i0 < nitems; i0 += 32 * kSumItems) {
-            const int ns = min(kSumItems, (nitems - i0 + 31) >> 5);   // 32-item slots of this round that hold an item (warp-uniform)
-            float accv[kSumItems][8];
-#pragma unroll
-            for (int s = 0; s < kSumItems; ++s)
-#pragma unroll
-                for (int q = 0; q < 8; ++q) accv[s][q] = 0.f;
-            const DT *src[kSumItems];
-            bool ok[kSumItems];
-#pragma unroll
-            for (int s = 0; s < kSumItems; ++s) {
-                const int i = i0 + 32 * s + lane;
-                ok[s] = i < nitems;
-                const int ic = min(i, nitems - 1);           // lanes past the last item re-read it (no predicate on the loads)
-                src[s] = rowbase + (size_t)mod_h<H>(ic) * hs + div_h<H>(ic) * kPer;
-            }
-            for (int l0 = 0; l0 < nlayers; l0 += 6) {
-                uint4 v[kSumItems][6];
-                if (l0 + 6 <= nlayers) {
-#pragma unroll
-                    for (int s = 0; s < kSumItems; ++s)
-                        if (s < ns) {
-                            const DT *pl0 = src[s] + (size_t)l0 * layer_stride;
-#pragma unroll
-                            for (int j = 0; j < 6; ++j) v[s][j] = __ldg(reinterpret_cast<const uint4 *>(pl0 + (size_t)j * layer_stride));
-                        }
-                } else {
-#pragma unroll
-                    for (int s = 0; s < kSumItems; ++s)
-                        if (s < ns) {
-#pragma unroll
-                            for (int j = 0; j < 6; ++j)
-                                v[s][j] = (l0 + j < nlayers)
-                                              ? __ldg(reinterpret_cast<const uint4 *>(src[s] + (size_t)(l0 + j) * layer_stride))
-                                              : make_uint4(0u, 0u, 0u, 0u);
-                        }
-                }
-#pragma unroll
-                for (int s = 0; s < kSumItems; ++s)
-                    if (s < ns) {
-#pragma unroll
-                        for (int j = 0; j < 6; ++j) {
-                            const uint32_t w4[4] = {v[s][j].x, v[s][j].y, v[s][j].z, v[s][j].w};
-                            if constexpr (sizeof(DT) == 4) {
-#pragma unroll
-                                for (int q = 0; q < 4; ++q) accv[s][q] += __uint_as_float(w4[q]);
-                            } else {
-#pragma unroll
-                                for (int q = 0; q < 4; ++q) {
-                                    accv[s][2 * q] += bf16lo(w4[q]);
-                                    accv[s][2 * q + 1] += __uint_as_float(w4[q] & 0xFFFF0000u);
-                                }
-                            }
-                        }
-                    }
-            }
-#pragma unroll
-            for (int s = 0; s < kSumItems; ++s) {
-                const int i = i0 + 32 * s + lane;
-                if (ok[s]) {
-                    const uint32_t dst = s_dsum + (uint32_t)mod_h<H>(i) * pitch4 + (uint32_t)(div_h<H>(i) * kPer) * 4u;
-                    sts_f32x4(dst, accv[s][0], accv[s][1], accv[s][2], accv[s][3]);
-                    if constexpr (sizeof(DT) == 2) {         // cells past the pitch lie beyond the graph's last token: never read
-                        if (div_h<H>(i) * kPer + 8 <= pl.pitch) sts_f32x4(dst + 16u, accv[s][4], accv[s][5], accv[s][6], accv[s][7]);
-                    }
-                }
-            }
-        }
+        k2_bwd_sum_row<H>(dB + ((size_t)g * H * c.T + a) * c.Tp, Tg, nlayers, layer_stride, hs, s_dsum, pitch4, pl.pitch, lane);
         // ---- 2. index phase: cinfo[b] = R row | P row << 16 (the trash rows for cells that carry no gradient) ;
         //         cdev[b] = up to two deviating bytes ;  dlist = the cells that need the slow path
         int ndl = 0;
@@ -552,26 +586,9 @@ __global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_bias_bwd_kernel(con
           }
         }
         __syncwarp();
-        // ---- 3. histogram phase: lane = (table, cell slot c2, head h); adjacent cells b0 + 2 c2, b0 + 2 c2 + 1 per step.
-        //         Cells without a gradient point at the trash rows, so the loop carries no predicates.
+        // ---- 3. histogram phase: lane = (table, cell slot c2, head h)
         if (lane < H) tacc += lds_f32(s_dsum + (uint32_t)h * pitch4);          // column 0: graph-token virtual distance
-        if (K2Heads<H>::kLanes == 32 || lane < K2Heads<H>::kLanes) {
-            uint32_t pi = s_cinfo + (uint32_t)c2 * 8u, pd = s_dsum + (uint32_t)h * pitch4 + (uint32_t)c2 * 8u;
-            for (int b0 = 0; b0 < Tg4; b0 += 2 * S, pi += 8u * S, pd += 8u * S) {
-                uint32_t iA, iB;
-                float dA, dB_;
-                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(iA), "=r"(iB) : "r"(pi) : "memory");
-                asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(dA), "=f"(dB_) : "r"(pd) : "memory");
-                const uint32_t aA = s_hist + ((iA >> key_shift) & 0xFFFFu) * key_bytes;
-                const uint32_t aB = s_hist + ((iB >> key_shift) & 0xFFFFu) * key_bytes;
-                // two read-modify-writes in flight; equal addresses are chained in registers, the second store wins
-                const float vA = lds_f32(aA), vB = lds_f32(aB);
-                const float nA = vA + dA;
-                const float nB = ((aA == aB) ? nA : vB) + dB_;
-                sts_f32(aA, nA);
-                sts_f32(aB, nB);
-            }
-        }
+        k2_bwd_hist_row<H>(s_cinfo, s_dsum, s_hist, key_shift, pitch4, Tg4, lane, c2, h);
         // ---- slow path (rare): walk bytes that differ from the expected walk, keys outside the plan; H lanes = H heads per
         //      listed cell, 32 / H cells at a time
         constexpr int SC = K2Heads<H>::kSlowCells;
@@ -732,6 +749,237 @@ __global__ void k2_bias_bwd_finish_kernel(const float *__restrict__ dEW, const f
         for (int v = 0; v < kEdgeVocab; ++v) acc += E[v * H + hp] * dEW[((size_t)k * kEdgeVocab + v) * H + h];
         dW[j] = acc;
     }
+}
+
+// ---- direct edge encoding ----------------------------------------------------------------------------
+// Graphormer's encoding for any edge_type other than multi_hop (the reference's else-branch between the multi-hop block,
+// model_fqandtoyo.py:1168-1208, and the add into the bias, :1213-1216):
+//   bias[g,h,a,b] = [a>=1, b>=1] ( R[rp[g,a-1,b-1],h] + Ppos[pp[g,a-1,b-1],h] + E[f[g,a-1,b-1],h] ) + [a>=1, b==0] t[h]
+// with f = attn_edge_type (the packed u8 plane feat8: 0 for no edge, else count + 2) and -inf where rp-1 >= rel_pos_max.
+// No walk, no edge_dis_encoder, no division by the distance.  E row 0 is read like any other row (cells without an edge).
+
+// Forward.  Persistent CTAs; R (its -inf rows applied while staging), Ppos and E sit in shared memory.  Per cell 5 index bytes
+// and three table gathers.  Cells per thread as in the multi-hop forward (K2FwdCells): at 8 heads a pair of adjacent cells
+// (a, b) (a, b+1), b even; at 12 heads one cell (two cells keep 2 x 12 accumulators and three 12-float rows per cell live
+// and spill 36-76 bytes per thread under __launch_bounds__(512, 2)).
+template <int H, typename OutT>
+__global__ void __launch_bounds__(512, 2) k2_direct_fwd_kernel(const K2Common c, const uint8_t *__restrict__ feat,
+                                                               const float *__restrict__ Rg, const float *__restrict__ Pg,
+                                                               int num_bins, const float *__restrict__ Eg,
+                                                               const float *__restrict__ tvd, OutT *__restrict__ out) {
+    extern __shared__ __align__(16) float sm[];
+    const int nR = kRelRows * H, nP = num_bins * H, nE = kEdgeVocab * H;
+    float *Rs = sm, *Ps = Rs + nR, *Es = Ps + nP;
+    for (int i = threadIdx.x * 4; i < nR; i += blockDim.x * 4) {
+        const float4 v = *reinterpret_cast<const float4 *>(Rg + i);
+        *reinterpret_cast<float4 *>(Rs + i) = (i / H - 1 >= c.rel_pos_max) ? make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY) : v;
+    }
+    for (int i = threadIdx.x * 4; i < nP; i += blockDim.x * 4)
+        *reinterpret_cast<float4 *>(Ps + i) = *reinterpret_cast<const float4 *>(Pg + i);
+    for (int i = threadIdx.x * 4; i < nE; i += blockDim.x * 4)
+        *reinterpret_cast<float4 *>(Es + i) = *reinterpret_cast<const float4 *>(Eg + i);
+    __syncthreads();
+    constexpr int kCells = K2FwdCells<H>::kCells;
+    const int half = c.Tp >> (kCells - 1);        // threads per plane row
+    const int per_graph = c.T * half;
+    const int tiles = ceil_div(per_graph, (int)blockDim.x);
+    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^19
+    const size_t hs = (size_t)c.T * c.Tp;
+    for (int w = blockIdx.x; w < tiles * c.B; w += gridDim.x) {
+        const int g = w / tiles, tile = w - g * tiles;
+        const int n = c.n[g];
+        const int Tg = n + 1;
+        const int f = tile * blockDim.x + threadIdx.x;
+        const int a = (int)(((uint64_t)f * half_magic) >> 40), b = (f - a * half) * kCells;
+        if (a >= Tg || b >= Tg) continue;
+        float acc[kCells][H];
+#pragma unroll
+        for (int s = 0; s < kCells; ++s)
+#pragma unroll
+            for (int h = 0; h < H; ++h) acc[s][h] = 0.f;
+        if (a >= 1) {
+            const int64_t rowp = c.sq_off[g] + (int64_t)(a - 1) * n;   // pair (a-1, j) lives at rowp + j
+            // cell s of this thread is the pair j = b - 1 + s  (b == 0, s == 0: the virtual-distance column)
+            int rp[kCells], pp[kCells], fe[kCells];
+#pragma unroll
+            for (int s = 0; s < kCells; ++s) {
+                const int j = b - 1 + s;
+                rp[s] = pp[s] = fe[s] = -1;
+                if (j >= 0 && j < n) {
+                    rp[s] = c.rel_pos[rowp + j];
+                    pp[s] = c.poi_pos[rowp + j];
+                    fe[s] = __ldg(feat + rowp + j);
+                }
+            }
+#pragma unroll
+            for (int s = 0; s < kCells; ++s) {
+                if (fe[s] < 0) {
+                    if (b == 0 && s == 0) {
+#pragma unroll
+                        for (int h = 0; h < H; ++h) acc[0][h] = __ldg(tvd + h);
+                    }
+                    continue;
+                }
+                float4 r0[H / 4], p0[H / 4], e0[H / 4];
+                load_row<H>(r0, Rs + min(max(rp[s], 0), kRelRows - 1) * H);
+                load_row<H>(p0, Ps + min(max(pp[s], 0), num_bins - 1) * H);
+                load_row<H>(e0, Es + min(fe[s], kEdgeVocab - 1) * H);
+#pragma unroll
+                for (int i = 0; i < H / 4; ++i) {
+                    acc[s][4 * i] = (r0[i].x + p0[i].x) + e0[i].x; acc[s][4 * i + 1] = (r0[i].y + p0[i].y) + e0[i].y;
+                    acc[s][4 * i + 2] = (r0[i].z + p0[i].z) + e0[i].z; acc[s][4 * i + 3] = (r0[i].w + p0[i].w) + e0[i].w;
+                }
+            }
+        }
+        OutT *o = out + ((size_t)g * H * c.T + a) * c.Tp + b;
+        if (kCells == 2 && b + 1 < Tg) {
+#pragma unroll
+            for (int h = 0; h < H; ++h) store2<OutT>(o + h * hs, acc[0][h], acc[kCells - 1][h]);
+        } else {
+#pragma unroll
+            for (int h = 0; h < H; ++h) store1<OutT>(o + h * hs, acc[0][h]);
+        }
+    }
+}
+
+// Backward.  The multi-hop backward's row loop without the walk: per plane row (g, a) one warp runs the same sum phase and
+// histogram phase (dR and dPpos as warp-private shared-memory histograms, dt from column 0).  The index phase packs only the
+// R and P rows; cells with an edge (f != 0) and rel_pos keys outside the histogram plan go to a list that H lanes per cell
+// work through: dE[f] by 64-bit fixed-point atomics into the CTA's [128][H] table in shared memory, out-of-plan keys into the
+// launch-wide dR table in global memory.  Cells without an edge never touch dE: its row 0 (the padding row) stays 0.  On
+// trajectory graphs a row has a few edges, so the list is short.  Integer sums do not depend on the order of the atomics, and
+// the float histograms are reduced in a fixed order, so the result is bitwise reproducible.
+template <int H>
+static K2BwdPlan k2_direct_bwd_plan(int T, int num_bins) {
+    constexpr int S = K2Heads<H>::kSlots;
+    K2BwdPlan p = k2_bwd_plan<H>(T, round_up(T, 8), 0, num_bins);     // histogram rows and pitch as the multi-hop plan
+    p.nEWs = 0;
+    p.stride = p.nR + p.nP + H;                                         // partial row = [R | P | t(H)]
+    p.per_warp = S * (p.nR + H) + S * (p.nP + H) + H * p.pitch + 2 * p.pitch + H;   // hR+trash | hP+trash | dsum | cinfo | dlist | t
+    p.cta_words = 2 * kEdgeVocab * H;                                   // dE fixed-point table (long long)
+    const int w = (int)((227 * 1024 - 2048 - p.cta_words * 4) / (p.per_warp * 4));
+    p.warps = w > kK2BwdMaxWarps ? kK2BwdMaxWarps : w;
+    return p;
+}
+
+// dlist entry: cell b (bits 0..11) | key outside the plan (bit 12) | edge (bit 13) | f (bits 14..20) | rel_pos key (bits 21..29)
+constexpr uint32_t kDirOvf = 1u << 12, kDirEdge = 1u << 13;
+
+template <int H, typename DT>
+__global__ void __launch_bounds__(kK2BwdMaxWarps * 32, 1) k2_direct_bwd_kernel(const K2Common c, const uint8_t *__restrict__ feat,
+                                                                               const DT *__restrict__ dB, int nlayers,
+                                                                               int64_t layer_stride, int num_bins,
+                                                                               const K2BwdPlan pl, float *__restrict__ partial,
+                                                                               long long *__restrict__ dE64,
+                                                                               long long *__restrict__ dR64) {
+    extern __shared__ __align__(16) float sm[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
+    constexpr int S = K2Heads<H>::kSlots;
+    const int ty = lane / (S * H), c2 = (lane / H) % S, h = lane % H;      // table (0 = R, 1 = P), cell slot, head
+    long long *sE = reinterpret_cast<long long *>(sm);            // [128][H] fixed point
+    float *wbase = sm + pl.cta_words;
+    const uint32_t s_warp = (uint32_t)__cvta_generic_to_shared(wbase + (size_t)warp * pl.per_warp);
+    const uint32_t s_hR = s_warp;                                 // [Rrows + 1][S][H]   (last row: trash)
+    const uint32_t s_hP = s_hR + (uint32_t)S * (pl.nR + H) * 4u;  // [bins + 1][S][H]    (last row: trash)
+    const uint32_t s_dsum = s_hP + (uint32_t)S * (pl.nP + H) * 4u;        // [H][pitch]
+    const uint32_t s_cinfo = s_dsum + (uint32_t)(H * pl.pitch) * 4u;    // [pitch]: R row | P row << 16
+    const uint32_t s_dlist = s_cinfo + (uint32_t)pl.pitch * 4u;   // [pitch]: cells for the list path
+    const uint32_t s_T = s_dlist + (uint32_t)pl.pitch * 4u;       // [H]
+    const uint32_t s_hist = (ty ? s_hP : s_hR) + (uint32_t)(c2 * H + h) * 4u;
+    const uint32_t key_shift = ty ? 16u : 0u;
+    const uint32_t trashR = (uint32_t)pl.Rrows, trashP = (uint32_t)num_bins;
+    for (int i = threadIdx.x; i < kEdgeVocab * H; i += blockDim.x) sE[i] = 0;
+    for (int i = threadIdx.x; i < nwarp * pl.per_warp; i += blockDim.x) wbase[i] = 0.f;
+    __syncthreads();
+    const size_t hs = (size_t)c.T * c.Tp;
+    const uint32_t pitch4 = (uint32_t)pl.pitch * 4u;
+    float tacc = 0.f;
+    for (int u = blockIdx.x * nwarp + warp; u < c.B * c.T; u += gridDim.x * nwarp) {
+        const int g = u / c.T, a = u - g * c.T;
+        const int n = c.n[g];
+        if (a == 0 || a > n) continue;                       // row 0 carries no parameter (model_fqandtoyo.py:1160-1165)
+        const int Tg = n + 1;
+        const int64_t rowp = c.sq_off[g] + (int64_t)(a - 1) * n - 1;     // pair of cell b lives at rowp + b
+        // ---- 1. sum phase
+        k2_bwd_sum_row<H>(dB + ((size_t)g * H * c.T + a) * c.Tp, Tg, nlayers, layer_stride, hs, s_dsum, pitch4, pl.pitch, lane);
+        // ---- 2. index phase: cinfo[b] = R row | P row << 16 (the trash rows for cells that carry no gradient); dlist
+        int ndl = 0;
+        const int Tg4 = (Tg + 3) & ~3;
+        for (int bg = 0; bg < Tg4; bg += 32 * kIdxUnroll) {
+            int rpv[kIdxUnroll], ppv[kIdxUnroll], fv[kIdxUnroll];
+#pragma unroll
+            for (int u2 = 0; u2 < kIdxUnroll; ++u2) {
+                const int b = bg + 32 * u2 + lane;
+                rpv[u2] = ppv[u2] = fv[u2] = 0;
+                if (b >= 1 && b < Tg) {
+                    rpv[u2] = c.rel_pos[rowp + b];
+                    ppv[u2] = c.poi_pos[rowp + b];
+                    fv[u2] = __ldg(feat + rowp + b);
+                }
+            }
+#pragma unroll
+            for (int u2 = 0; u2 < kIdxUnroll; ++u2) {
+                const int b0 = bg + 32 * u2;
+                if (b0 >= Tg4) break;                            // warp-uniform
+                const int b = b0 + lane;
+                uint32_t info = trashR | (trashP << 16), ent = 0u;
+                if (b >= 1 && b < Tg) {
+                    const int rk = min(max(rpv[u2], 0), kRelRows - 1);
+                    const int row = (rk == 511) ? pl.Rrows - 1 : (rk < pl.Rrows - 1 ? rk : -1);
+                    if (rk - 1 < c.rel_pos_max) {                    // -inf entries carry no gradient
+                        info = (row < 0 ? trashR : (uint32_t)row) | ((uint32_t)min(max(ppv[u2], 0), num_bins - 1) << 16);
+                        const uint32_t fe = (uint32_t)min(fv[u2], kEdgeVocab - 1);
+                        if (fe != 0u || row < 0)
+                            ent = (uint32_t)b | (row < 0 ? kDirOvf : 0u) | (fe != 0u ? kDirEdge : 0u) | (fe << 14) | ((uint32_t)rk << 21);
+                    }
+                }
+                if (b < Tg4) sts_u32(s_cinfo + (uint32_t)b * 4u, info);
+                const uint32_t bal = __ballot_sync(0xffffffffu, ent != 0u);
+                if (ent) sts_u32(s_dlist + (uint32_t)(ndl + __popc(bal & ((1u << lane) - 1u))) * 4u, ent);
+                ndl += __popc(bal);
+            }
+        }
+        __syncwarp();
+        // ---- 3. histogram phase
+        if (lane < H) tacc += lds_f32(s_dsum + (uint32_t)h * pitch4);          // column 0: graph-token virtual distance
+        k2_bwd_hist_row<H>(s_cinfo, s_dsum, s_hist, key_shift, pitch4, Tg4, lane, c2, h);
+        // ---- list path: H lanes = H heads per listed cell, 32 / H cells at a time
+        constexpr int SC = K2Heads<H>::kSlowCells;
+        for (int e0 = 0; e0 < ndl; e0 += SC) {
+            const int e = e0 + lane / H;
+            if (e >= ndl || (SC * H < 32 && lane >= SC * H)) continue;
+            const uint32_t ent = lds_u32(s_dlist + (uint32_t)e * 4u);
+            const float d = lds_f32(s_dsum + (uint32_t)h * pitch4 + (ent & 0xFFFu) * 4u);
+            if (ent & kDirOvf) fx_add(dR64 + (ent >> 21) * H + h, d);
+            if (ent & kDirEdge) fx_add(sE + ((ent >> 14) & 127u) * H + h, d);
+        }
+        __syncwarp();
+    }
+    if (lane < H) sts_f32(s_T + (uint32_t)h * 4u, tacc);
+    __syncthreads();
+    // CTA totals: histograms -> partial[blockIdx] (summed in a fixed order later), dE table -> the launch-wide one
+    float *out = partial + (size_t)blockIdx.x * pl.stride;
+    for (int i = threadIdx.x; i < pl.nR; i += blockDim.x) {
+        const int key = i / H, hh = i % H;
+        float s = 0.f;
+        for (int w = 0; w < nwarp; ++w)
+            for (int r = 0; r < S; ++r) s += wbase[(size_t)w * pl.per_warp + (key * S + r) * H + hh];
+        out[i] = s;
+    }
+    for (int i = threadIdx.x; i < pl.nP; i += blockDim.x) {
+        const int key = i / H, hh = i % H;
+        float s = 0.f;
+        for (int w = 0; w < nwarp; ++w)
+            for (int r = 0; r < S; ++r) s += wbase[(size_t)w * pl.per_warp + S * (pl.nR + H) + (key * S + r) * H + hh];
+        out[pl.nR + i] = s;
+    }
+    if (threadIdx.x < H) {
+        float s = 0.f;
+        for (int w = 0; w < nwarp; ++w) s += wbase[(size_t)w * pl.per_warp + pl.per_warp - H + threadIdx.x];
+        out[pl.nR + pl.nP + threadIdx.x] = s;
+    }
+    for (int i = threadIdx.x; i < kEdgeVocab * H; i += blockDim.x)
+        if (sE[i] != 0) atomicAdd(reinterpret_cast<unsigned long long *>(dE64 + i), (unsigned long long)sE[i]);
 }
 
 }  // namespace mobgt
@@ -905,4 +1153,121 @@ extern "C" int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const
     auto f = H == 8 ? bias_bwd<8> : bias_bwd<12>;
     return f(n, sq_off, rel_pos, poi_pos, edge_in, B, T, Tp, hops, dk, rel_pos_max, num_bins, dBias, dbias_dtype, n_layers,
              layer_stride, E, W, workspace, workspace_bytes, dR, dPpos, dE, dW, dtvd, static_cast<cudaStream_t>(stream));
+}
+
+// ---- direct edge encoding: entry points ----
+
+template <int H>
+static int32_t bias_direct_fwd(const K2Common &c, const uint8_t *feat, int32_t num_bins, const float *R, const float *Ppos,
+                               const float *E, const float *tvd, void *out, int32_t out_dtype, cudaStream_t s) {
+    const size_t smem = (size_t)(kRelRows + num_bins + kEdgeVocab) * H * sizeof(float);
+    const int tiles_total = ceil_div(c.T * (c.Tp / K2FwdCells<H>::kCells), 512) * c.B;
+    dim3 grid((unsigned)min(2 * kNumSMs, tiles_total));
+    auto launch = [&](auto kern, auto *o) -> int32_t {
+        MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<grid, 512, smem, s>>>(c, feat, R, Ppos, num_bins, E, tvd, o);
+        return MOBGT_OK;
+    };
+    const int32_t rc = (out_dtype == MOBGT_F32) ? launch(k2_direct_fwd_kernel<H, float>, static_cast<float *>(out))
+                                                : launch(k2_direct_fwd_kernel<H, __nv_bfloat16>, static_cast<__nv_bfloat16 *>(out));
+    if (rc) return rc;
+    MOBGT_LAUNCH_OK("k2_direct_fwd_kernel");
+    return MOBGT_OK;
+}
+
+extern "C" int32_t mobgt_bias_direct_fwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                                         const uint8_t *feat, int32_t B, int32_t T, int32_t Tp, int32_t H, int32_t rel_pos_max,
+                                         int32_t num_bins, const float *R, const float *Ppos, const float *E, const float *tvd,
+                                         void *out, int32_t out_dtype, void *stream) {
+    MOBGT_REQUIRE(k2_heads_built(H), MOBGT_ERR_UNSUPPORTED, "mobgt_bias_direct_fwd: num_heads=%d is not built (8 and 12 heads)", H);
+    MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && feat && R && Ppos && E && tvd && out, MOBGT_ERR_NULL,
+                  "mobgt_bias_direct_fwd: null pointer");
+    MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_fwd: num_bins=%d", num_bins);
+    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_fwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE(out_dtype == MOBGT_F32 || out_dtype == MOBGT_BF16, MOBGT_ERR_BAD_DTYPE, "mobgt_bias_direct_fwd: dtype");
+    if (B <= 0) return MOBGT_OK;
+    const K2Common c{n, sq_off, rel_pos, poi_pos, nullptr, B, T, Tp, 0, rel_pos_max, 0};
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    auto f = H == 8 ? bias_direct_fwd<8> : bias_direct_fwd<12>;
+    return f(c, feat, num_bins, R, Ppos, E, tvd, out, out_dtype, s);
+}
+
+// workspace of the direct backward: [stride] totals, [kNumSMs][stride] partials, then (16-byte aligned) the fixed-point dE
+// [128][H] and rel_pos overflow [512][H] tables
+template <int H>
+static int64_t direct_fx_offset(const K2BwdPlan &pl) {
+    return ((int64_t)(kNumSMs + 1) * pl.stride * (int64_t)sizeof(float) + 15) / 16 * 16;
+}
+template <int H>
+static int64_t direct_bwd_workspace_bytes(int32_t T, int32_t num_bins) {
+    const K2BwdPlan pl = k2_direct_bwd_plan<H>(T, num_bins);
+    return direct_fx_offset<H>(pl) + (int64_t)(kEdgeVocab + kRelRows) * H * (int64_t)sizeof(long long);
+}
+
+extern "C" int64_t mobgt_bias_direct_bwd_workspace_bytes(int32_t T, int32_t num_bins, int32_t H) {
+    if (!k2_heads_built(H) || T < 2 || num_bins < 1 || num_bins > 1024) return -1;
+    return H == 8 ? direct_bwd_workspace_bytes<8>(T, num_bins) : direct_bwd_workspace_bytes<12>(T, num_bins);
+}
+
+template <int H>
+static int32_t bias_direct_bwd(const K2Common &c, const uint8_t *feat, int32_t num_bins, const void *dBias, int32_t dbias_dtype,
+                               int32_t n_layers, int64_t layer_stride, void *workspace, int64_t workspace_bytes, float *dR,
+                               float *dPpos, float *dE, float *dtvd, cudaStream_t s) {
+    const K2BwdPlan pl = k2_direct_bwd_plan<H>(c.T, num_bins);
+    MOBGT_REQUIRE(pl.warps >= 1, MOBGT_ERR_UNSUPPORTED, "mobgt_bias_direct_bwd: no shared-memory plan for T=%d bins=%d", c.T,
+                  num_bins);
+    const int64_t fx_off = direct_fx_offset<H>(pl);
+    const int64_t need = direct_bwd_workspace_bytes<H>(c.T, num_bins);
+    MOBGT_REQUIRE(workspace_bytes >= need, MOBGT_ERR_WORKSPACE_TOO_SMALL, "mobgt_bias_direct_bwd: workspace %lld < %lld bytes",
+                  (long long)workspace_bytes, (long long)need);
+    MOBGT_REQUIRE(((uintptr_t)workspace & 15) == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_bwd: workspace must be 16-byte aligned");
+    float *tot = static_cast<float *>(workspace);          // [stride] totals, then [kNumSMs][stride] partials
+    float *partial = tot + pl.stride;
+    long long *dE64 = reinterpret_cast<long long *>(static_cast<char *>(workspace) + fx_off);   // [128][H]
+    long long *dR64 = dE64 + kEdgeVocab * H;                                                     // [512][H]
+    MOBGT_CUDA_OK(cudaMemsetAsync(dE64, 0, (size_t)(kEdgeVocab + kRelRows) * H * sizeof(long long), s));
+    const int nparts = c.B > 0 ? kNumSMs : 0;
+    if (c.B > 0) {
+        const size_t smem = (size_t)(pl.cta_words + pl.warps * pl.per_warp) * sizeof(float);
+        auto launch = [&](auto kern, auto *db, int nl, int64_t ls) -> int32_t {
+            MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            kern<<<kNumSMs, pl.warps * 32, smem, s>>>(c, feat, db, nl, ls, num_bins, pl, partial, dE64, dR64);
+            return MOBGT_OK;
+        };
+        const int32_t rc = (dbias_dtype == MOBGT_F32)
+                               ? launch(k2_direct_bwd_kernel<H, float>, static_cast<const float *>(dBias), 1, (int64_t)0)
+                               : launch(k2_direct_bwd_kernel<H, __nv_bfloat16>, static_cast<const __nv_bfloat16 *>(dBias),
+                                        n_layers, layer_stride);
+        if (rc) return rc;
+        MOBGT_LAUNCH_OK("k2_direct_bwd_kernel");
+    }
+    // the multi-hop epilogue without its walk tables: fixed-order partial sums, the fixed-point dE and overflow rows to fp32,
+    // then the histogram rows into dR / dPpos / dt
+    k2_bias_bwd_reduce_kernel<H><<<ceil_div(pl.stride + (kEdgeVocab + kRelRows) * H, 256), 256, 0, s>>>(
+        partial, nparts, pl.stride, 0, nullptr, tot, dE64, kEdgeVocab * H, dE, dR64, dR);
+    MOBGT_LAUNCH_OK("k2_bias_bwd_reduce_kernel");
+    k2_bias_bwd_scatter_kernel<H><<<ceil_div(max(kRelRows, num_bins) * H, 256), 256, 0, s>>>(tot, pl, 0, 1, num_bins, nullptr, dR,
+                                                                                            dPpos, dtvd);
+    MOBGT_LAUNCH_OK("k2_bias_bwd_scatter_kernel");
+    return MOBGT_OK;
+}
+
+extern "C" int32_t mobgt_bias_direct_bwd(const int32_t *n, const int64_t *sq_off, const int16_t *rel_pos, const int16_t *poi_pos,
+                                         const uint8_t *feat, int32_t B, int32_t T, int32_t Tp, int32_t H, int32_t rel_pos_max,
+                                         int32_t num_bins, const void *dBias, int32_t dbias_dtype, int32_t n_layers,
+                                         int64_t layer_stride, void *workspace, int64_t workspace_bytes, float *dR, float *dPpos,
+                                         float *dE, float *dtvd, void *stream) {
+    MOBGT_REQUIRE(k2_heads_built(H), MOBGT_ERR_UNSUPPORTED, "mobgt_bias_direct_bwd: num_heads=%d is not built (8 and 12 heads)", H);
+    MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && feat && dBias && workspace && dR && dPpos && dE && dtvd, MOBGT_ERR_NULL,
+                  "mobgt_bias_direct_bwd: null pointer");
+    MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_bwd: num_bins=%d", num_bins);
+    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_bwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE((dbias_dtype == MOBGT_F32 && n_layers == 1) || (dbias_dtype == MOBGT_BF16 && n_layers >= 1 && n_layers <= 64),
+                  MOBGT_ERR_BAD_DTYPE, "mobgt_bias_direct_bwd: dbias dtype %d with %d layer planes", dbias_dtype, n_layers);
+    MOBGT_REQUIRE(((uintptr_t)dBias & 15) == 0 && (dbias_dtype == MOBGT_F32 || layer_stride % 8 == 0), MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_direct_bwd: dBias planes must be 16-byte aligned");
+    const K2Common c{n, sq_off, rel_pos, poi_pos, nullptr, B, T, Tp, 0, rel_pos_max, 0};
+    auto f = H == 8 ? bias_direct_bwd<8> : bias_direct_bwd<12>;
+    return f(c, feat, num_bins, dBias, dbias_dtype, n_layers, layer_stride, workspace, workspace_bytes, dR, dPpos, dE, dtvd,
+             static_cast<cudaStream_t>(stream));
 }

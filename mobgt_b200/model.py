@@ -271,15 +271,17 @@ class Graphormer(nn.Module):
                 f"heads: the attention-bias kernels (K2) are built for 8 heads and for 12 heads, and the attention kernels (K3) "
                 f"for head dims {ops.HEAD_DIMS[0]} and {ops.HEAD_DIMS[1]}, i.e. hidden_dim 64 or 128 at 8 heads and hidden_dim "
                 f"128 at 12 heads.")
-        if edge_type != "multi_hop":
-            raise NotImplementedError("edge_type must be 'multi_hop' (README.md:62)")
         tr = DATASET_TRAITS[dataset_name]
         self.traits, self.dataset_name = tr, dataset_name
         self.num_virtual_tokens, self.num_heads, self.hidden_dim = 1, num_heads, hidden_dim
         self.time_embed_dim = self.cat_embed_dim = 32
         H, C, P = num_heads, world.C, world.P
         D = hidden_dim + self.time_embed_dim + self.cat_embed_dim
+        # edge_type "multi_hop" (README.md:62): the mean over the shortest path of edge_encoder rows through edge_dis_encoder;
+        # any other value: Graphormer's direct encoding, edge_encoder[attn_edge_type] (edge_dis_encoder is kept, unused, so
+        # that both modes have the same state_dict)
         self.edge_type, self.multi_hop_max_dist = edge_type, multi_hop_max_dist
+        self.direct_edges = edge_type != "multi_hop"
         self.edge_encoder = nn.Embedding(128, H, padding_idx=0)
         self.edge_dis_encoder = nn.Embedding(128 * H * H, 1)
         self.rel_pos_encoder = nn.Embedding(512, H, padding_idx=0)
@@ -354,7 +356,7 @@ class Graphormer(nn.Module):
     def attn_bias(self, b, dtype=torch.bfloat16):
         """K2 (model_fqandtoyo.py:1143-1216)"""
         return ops.AttnBias.apply(b, self.rel_pos_encoder.weight, self.poi_pos_encoder.weight, self.edge_encoder.weight,
-                                  self.edge_dis_encoder.weight, self.graph_token_virtual_distance.weight, dtype)
+                                  self.edge_dis_encoder.weight, self.graph_token_virtual_distance.weight, dtype, self.direct_edges)
 
     def node_tokens(self, b, dtype=torch.bfloat16):
         """K4 (model_fqandtoyo.py:1222-1344) -> packed tokens [ntok, hidden_dim + 64]"""
@@ -389,7 +391,7 @@ class Graphormer(nn.Module):
         slot = ops.BiasSlot(b, len(self.layers), dtype=torch.float32 if f32 else torch.bfloat16)
         x = ops.BiasLink.apply(self.input_dropout(tok).float(), slot, self.rel_pos_encoder.weight, self.poi_pos_encoder.weight,
                                self.edge_encoder.weight, self.edge_dis_encoder.weight,
-                               self.graph_token_virtual_distance.weight)                                 # K2 (:1143-1216), :1347
+                               self.graph_token_virtual_distance.weight, self.direct_edges)              # K2 (:1143-1216), :1347
         if f32:
             for li, layer in enumerate(self.layers):                                                     # :1348-1352
                 x = layer.forward_f32(x, slot, li)

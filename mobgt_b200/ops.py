@@ -74,25 +74,80 @@ def bias_bwd_raw(batch, dbias, E, W, num_bins):
     return dR, dP, dE, dW.view_as(W), dtv
 
 
+def bias_direct_fwd_raw(batch, R, Ppos, E, tvd, out_dtype=torch.bfloat16, T=None, Tp=None):
+    """K2 for the direct edge encoding (edge_type other than multi_hop): the edge term of a pair is E[attn_edge_type], read from
+    the batch's feat8 plane.  Same output layout as bias_fwd_raw."""
+    B, H = batch.B, R.shape[1]
+    T = T or batch.N + 1
+    Tp = Tp or bias_pitch(T)
+    out = torch.empty(B, H, T, Tp, dtype=out_dtype, device=R.device)
+    _C.call("mobgt_bias_direct_fwd", _C.ptr(batch.n), _C.ptr(batch.sq_off), _C.ptr(batch.rel_pos16), _C.ptr(batch.poi_pos16),
+            _C.ptr(batch.feat8), B, T, Tp, H, batch.rel_pos_max, int(Ppos.shape[0]), _C.ptr(R), _C.ptr(Ppos), _C.ptr(E), _C.ptr(tvd),
+            _C.ptr(out), _dt(out), _C.stream_ptr())
+    return out
+
+
+def bias_direct_bwd_raw(batch, dbias, num_bins):
+    """Backward of bias_direct_fwd_raw from the same dbias forms as bias_bwd_raw -> (dR, dPpos, dE, dtvd); dE row 0 is 0."""
+    if dbias.dtype == torch.bfloat16:
+        L, B, H, T, Tp = dbias.shape
+        dt, stride = BF16, dbias.stride(0)
+    else:
+        B, H, T, Tp = dbias.shape
+        L, dt, stride = 1, F32, 0
+    dev = dbias.device
+    ws_bytes = int(_C.lib().mobgt_bias_direct_bwd_workspace_bytes(T, num_bins, H))
+    if ws_bytes < 0:
+        raise _C.MobgtError(f"mobgt_bias_direct_bwd_workspace_bytes rejected T={T} num_bins={num_bins} H={H}")
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    dR = torch.empty(512, H, dtype=torch.float32, device=dev)
+    dP = torch.empty(num_bins, H, dtype=torch.float32, device=dev)
+    dE = torch.empty(128, H, dtype=torch.float32, device=dev)
+    dtv = torch.empty(H, dtype=torch.float32, device=dev)
+    _C.call("mobgt_bias_direct_bwd", _C.ptr(batch.n), _C.ptr(batch.sq_off), _C.ptr(batch.rel_pos16), _C.ptr(batch.poi_pos16),
+            _C.ptr(batch.feat8), B, T, Tp, H, batch.rel_pos_max, num_bins, _C.ptr(dbias), dt, L, stride, _C.ptr(ws), ws_bytes,
+            _C.ptr(dR), _C.ptr(dP), _C.ptr(dE), _C.ptr(dtv), _C.stream_ptr())
+    return dR, dP, dE, dtv
+
+
+def _bias_fwd(batch, direct, R, Ppos, E, W, tvd, out_dtype):
+    """K2 forward of either edge encoding; the tables are fp32 contiguous (W is not read by the direct encoding)."""
+    if direct:
+        return bias_direct_fwd_raw(batch, R, Ppos, E, tvd.view(-1), out_dtype)
+    return bias_fwd_raw(batch, R, Ppos, E, W.view(-1), tvd.view(-1), out_dtype)
+
+
+def _bias_bwd(batch, direct, dbias, E, W, num_bins):
+    """-> the gradients of (R, Ppos, E, W, tvd) as the autograd nodes return them; W's is None for the direct encoding."""
+    if direct:
+        dR, dP, dE, dt = bias_direct_bwd_raw(batch, dbias, num_bins)
+        dW = None
+    else:
+        dR, dP, dE, dW, dt = bias_bwd_raw(batch, dbias, E, W.view(-1), num_bins)
+        dW = dW.view(-1, 1)
+    dR[0].zero_()          # padding_idx rows (never indexed by a packed pair anyway)
+    dP[0].zero_()
+    return dR, dP, dE, dW, dt.view(1, -1)
+
+
 class AttnBias(torch.autograd.Function):
     """graph_attn_bias = f(rel_pos, poi_pos, edge_input; 5 tables)   (model_fqandtoyo.py:1143-1216) as a stand-alone
     differentiable op (gradient: a plain [B,H,T,Tp] tensor).  The model's forward uses BiasLink below, whose backward
-    consumes the per-layer bf16 dS planes of the attention kernels instead."""
+    consumes the per-layer bf16 dS planes of the attention kernels instead.  direct=True: the direct edge encoding
+    (E[attn_edge_type] instead of the multi-hop walk; W gets no gradient)."""
 
     @staticmethod
-    def forward(ctx, batch, R, Ppos, E, W, tvd, out_dtype):
+    def forward(ctx, batch, R, Ppos, E, W, tvd, out_dtype, direct=False):
         Rc, Pc, Ec, Wc, tc = (t.detach().float().contiguous() for t in (R, Ppos, E, W, tvd))
-        ctx.batch, ctx.num_bins = batch, Ppos.shape[0]
+        ctx.batch, ctx.num_bins, ctx.direct = batch, Ppos.shape[0], direct
         ctx.save_for_backward(Ec, Wc)
-        return bias_fwd_raw(batch, Rc, Pc, Ec, Wc.view(-1), tc.view(-1), out_dtype)
+        return _bias_fwd(batch, direct, Rc, Pc, Ec, Wc, tc, out_dtype)
 
     @staticmethod
     def backward(ctx, dbias):
         E, W = ctx.saved_tensors
-        dR, dP, dE, dW, dt = bias_bwd_raw(ctx.batch, dbias.float().contiguous(), E, W.view(-1), ctx.num_bins)
-        dR[0].zero_()          # padding_idx rows (never indexed by a packed pair anyway)
-        dP[0].zero_()
-        return None, dR, dP, dE, dW.view(-1, 1), dt.view(1, -1), None
+        dR, dP, dE, dW, dt = _bias_bwd(ctx.batch, ctx.direct, dbias.float().contiguous(), E, W, ctx.num_bins)
+        return None, dR, dP, dE, dW, dt, None, None
 
 
 # ----------------------------------------------------------------------------------------------- K3
@@ -264,10 +319,10 @@ class BiasLink(torch.autograd.Function):
               the table gradients are one K2-backward over the stack; d(tokens) passes through."""
 
     @staticmethod
-    def forward(ctx, tok, slot, R, Ppos, E, W, tvd):
+    def forward(ctx, tok, slot, R, Ppos, E, W, tvd, direct=False):
         Rc, Pc, Ec, Wc, tc = (t.detach().float().contiguous() for t in (R, Ppos, E, W, tvd))
-        slot.bias = bias_fwd_raw(slot.batch, Rc, Pc, Ec, Wc.view(-1), tc.view(-1), slot.dtype)
-        ctx.slot, ctx.num_bins = slot, Ppos.shape[0]
+        slot.bias = _bias_fwd(slot.batch, direct, Rc, Pc, Ec, Wc, tc, slot.dtype)
+        ctx.slot, ctx.num_bins, ctx.direct = slot, Ppos.shape[0], direct
         ctx.save_for_backward(Ec, Wc)
         return tok.view_as(tok)
 
@@ -276,16 +331,14 @@ class BiasLink(torch.autograd.Function):
         slot = ctx.slot
         planes, slot.planes = slot.planes, None
         if planes is None:                      # no attention layer took part in this backward
-            return dtok, None, None, None, None, None, None
+            return dtok, None, None, None, None, None, None, None
         if planes.dtype == torch.bfloat16:
             for l in range(slot.n_layers):      # a layer whose backward never ran contributes nothing
                 if l not in slot.written:
                     planes[l].zero_()
         E, W = ctx.saved_tensors
-        dR, dP, dE, dW, dt = bias_bwd_raw(slot.batch, planes, E, W.view(-1), ctx.num_bins)
-        dR[0].zero_()                           # padding_idx rows (never indexed by a packed pair anyway)
-        dP[0].zero_()
-        return dtok, None, dR, dP, dE, dW.view(-1, 1), dt.view(1, -1)
+        dR, dP, dE, dW, dt = _bias_bwd(slot.batch, ctx.direct, planes, E, W, ctx.num_bins)
+        return dtok, None, dR, dP, dE, dW, dt, None
 
 
 # ----------------------------------------------------------------------------------------------- K4
