@@ -317,6 +317,23 @@ int32_t mobgt_head_topk(const void *z, const void *W, const float *bias, const i
 int32_t mobgt_topk_merge(const float *val, const int32_t *idx, const int32_t *cnt_gt, const int32_t *cnt_eq, int32_t M,
                          int32_t S, int32_t k, float *out_val, int32_t *out_idx, int32_t *rank, void *stream);
 
+/* K5 in fp32 mode (`--precision 32` evaluation): the same head with z f32 [M,K] and W f32 [V,K] (out_proj.weight itself),
+ * logits in IEEE fp32 on the CUDA cores (no tensor-core instruction).  Every logit is computed in ONE fixed order,
+ *     s = 0;  for k = 0 .. K-1 ascending: s = fmaf(z[row][k], W[col][k], s);   logit = bias ? s + bias[col] : s
+ * (each fmaf and the add rounded once), whatever the tiling, nsplit or vocabulary shard: results are bitwise reproducible.
+ * mode 0 runs the same chain for the target's column, so the target's own logit equals st and never counts against itself.
+ *   K multiple of 4, 4 <= K <= 320 ; 1 <= k <= 32 ; mode 1: nsplit = 4 x (vocabulary splits), a multiple of 4 in [4, 160]
+ *   z and W 16-byte aligned (rows are then too, K being a multiple of 4); bias f32 [V] or NULL, any 4-byte alignment
+ *   mode 1 outputs per (row, list), same layout and meaning as mobgt_head_topk: a sorted top-k (value, global index; ties ->
+ *   lower index; a list may hold fewer than k entries: index -1), cnt_gt = #(s > st), cnt_eq = #(s == st and idx < target);
+ *   mobgt_topk_merge gives rank = cnt_gt + cnt_eq.  logits_dump (optional [M,V] f32) receives the kernel's own logits.
+ *   thr_share is not used (the lists of a row prune independently): pass NULL.
+ * Bad arguments return MOBGT_ERR_NULL / MOBGT_ERR_BAD_SHAPE before any launch. */
+int32_t mobgt_head_topk_f32(const float *z, const float *W, const float *bias, const int32_t *target, int32_t M, int32_t V,
+                            int32_t K, int64_t vocab_offset, int32_t k, int32_t nsplit, int32_t mode, float *st,
+                            float *topk_val, int32_t *topk_idx, int32_t *cnt_gt, int32_t *cnt_eq, float *logits_dump,
+                            void *thr_share, void *stream);
+
 /* ------------------------------------------------------------------------------------------
  * Test hooks (tests/test_umma_selftest.py): exercise the tcgen05 / TMA building blocks in isolation.
  * out[128,N] (f32) = A * B, bf16 operands; a_mn / b_mn select MN-major operands

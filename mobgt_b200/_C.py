@@ -59,6 +59,8 @@ SIGNATURES = {
     "mobgt_embed_sum_fwd": [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i32, c_i32, c_p, c_i32, c_p],
     "mobgt_segment_sum": [c_p, c_i32, c_i64, c_i32, c_i32, c_p, c_p, c_i32, c_p, c_i32, c_p, c_i64, c_p],
     "mobgt_head_topk": [c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i64, c_i32, c_i32, c_i32, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
+    "mobgt_head_topk_f32": [c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_i64, c_i32, c_i32, c_i32, c_p, c_p, c_p, c_p, c_p, c_p, c_p,
+                            c_p],
     "mobgt_topk_merge": [c_p, c_p, c_p, c_p, c_i32, c_i32, c_i32, c_p, c_p, c_p, c_p],
     "mobgt_layernorm_fwd": [c_p, c_p, c_p, c_f32, c_i32, c_i32, c_p, c_p, c_p, c_p, c_p],
     "mobgt_layernorm_bwd_workspace_bytes": [c_i32],

@@ -456,16 +456,22 @@ class Graphormer(nn.Module):
         """K5: POI logits + per-row top-k + rank of the target, fused (the logits never reach HBM).  -> dict(idx [B,k] i32,
         val [B,k], rank [B] i32).  log_softmax (toyotagraph, :1425) is monotone per row, so indices and ranks are those of
         the reference's y_pred[0].  vocab_parallel: a process group -> out_proj rows sharded across its ranks, z rows of all
-        ranks gathered (SURVEY.md §8e); returns the rows of THIS rank."""
-        W = self.out_proj.weight.detach().to(torch.bfloat16)
+        ranks gathered (SURVEY.md §8e); returns the rows of THIS rank.
+        precision 32 ranks IEEE fp32 logits (the fp32 K5 head: fp32 z and the out_proj.weight master itself, no rounding);
+        precision 16 ranks bf16-operand logits on the tensor cores."""
         bias = self.out_proj.bias.detach().float()
-        z16 = z.detach().to(torch.bfloat16).contiguous()
         t32 = y_true.to(torch.int32).contiguous()
+        if self.precision == 32:
+            W = self.out_proj.weight.detach()
+            zh = z.detach().float().contiguous()
+        else:
+            W = self.out_proj.weight.detach().to(torch.bfloat16)
+            zh = z.detach().to(torch.bfloat16).contiguous()
         if vocab_parallel is None:
-            r = ops.head_topk_local(z16, W.contiguous(), bias.contiguous(), t32, k)
+            r = ops.head_topk_local(zh, W.contiguous(), bias.contiguous(), t32, k)
             return dict(idx=r["idx"], val=r["val"], rank=r["cnt"])
         from . import parallel
-        return parallel.vocab_parallel_eval_head(ops, z16, W, bias, t32, k, vocab_parallel)
+        return parallel.vocab_parallel_eval_head(ops, zh, W, bias, t32, k, vocab_parallel)
 
     def _eval_step(self, batched_data, full_logits, vocab_parallel):
         z, b = self.features(batched_data)

@@ -1103,11 +1103,14 @@ def gradient_tail_loss(logits, target, alpha=0.25, n_classes=None):
 
 
 # ----------------------------------------------------------------------------------------------- K5
-def head_split(M, V):
+def head_split(M, V, dtype=torch.bfloat16):
     """Number of per-row output lists = 2 x (vocabulary splits per 128-row tile of z): every CTA of mobgt_head_topk runs two
     epilogue groups.  The split count minimises waves x (tiles per CTA + a fixed per-CTA cost) over the 148 SMs.  (Measured on
     B200, c5 shard: 9 splits x 32 row tiles in two waves (573 us) beat 4 splits in one 86 %-full wave (638 us): the warm-up
-    of a fresh top-k list costs ~8 tiles once the lists of a row share their pruning bound.)"""
+    of a fresh top-k list costs ~8 tiles once the lists of a row share their pruning bound.)
+    dtype=torch.float32: the split rule of mobgt_head_topk_f32 (`_head_split_f32`)."""
+    if dtype == torch.float32:
+        return _head_split_f32(M, V)
     mt = (M + 127) // 128
     nt = (V + 255) // 256          # vocabulary tiles of 256 rows (csrc/k5_head.cu kNT)
     best, best_cost = 1, None
@@ -1119,25 +1122,53 @@ def head_split(M, V):
     return 2 * best
 
 
-def head_topk_local(z, W, bias, target, k, vocab_offset=0, st=None, dump_logits=False):
-    """One vocabulary shard.  z bf16 [M,K], W bf16 [V,K], bias f32 [V]|None, target i32 [M] (global ids).
-    st=None -> runs mode 0 first (single-shard use).  Returns dict(val [M,k], idx [M,k], cnt [M] (partial rank), st)."""
+def _head_split_f32(M, V):
+    """Lists per row of mobgt_head_topk_f32 = 4 x (vocabulary splits per 64-row tile of z): four scanner threads per row in
+    every CTA.  Same cost model as the bf16 head (waves x (128-column tiles per CTA + a fixed cost)), one CTA per SM, at most
+    40 splits so that the merge sees at most 160 lists."""
+    mt = (M + 63) // 64
+    nt = (V + 127) // 128          # vocabulary tiles of 128 rows (csrc/k5_head_f32.cu kBN)
+    best, best_cost = 1, None
+    for gs in range(1, min(40, nt) + 1):
+        waves = (mt * gs + 147) // 148
+        cost = waves * ((nt + gs - 1) // gs + 2)
+        if best_cost is None or cost < best_cost:
+            best, best_cost = gs, cost
+    return 4 * best
+
+
+def _head_entry(z, W):
+    """The K5 entry point for z's dtype: float32 -> mobgt_head_topk_f32 (IEEE fp32 on the CUDA cores, W float32 too: it is
+    never rounded here), anything else -> mobgt_head_topk (bf16 operands on tcgen05)."""
+    if z.dtype != torch.float32:
+        return "mobgt_head_topk"
+    if W.dtype != torch.float32:
+        raise TypeError(f"fp32 K5 head: W must be float32 like z, got {W.dtype}")
+    return "mobgt_head_topk_f32"
+
+
+def head_topk_local(z, W, bias, target, k, vocab_offset=0, st=None, dump_logits=False, nsplit=None):
+    """One vocabulary shard.  z [M,K] and W [V,K] both bf16 (tcgen05 head) or both float32 (fp32 head), bias f32 [V]|None,
+    target i32 [M] (global ids).  st=None -> runs mode 0 first (single-shard use).  nsplit: lists per row (default
+    head_split; the merged result does not depend on it).  Returns dict(val [M,k], idx [M,k], cnt [M] (partial rank), st)."""
     M, K = z.shape
     V = W.shape[0]
     dev = z.device
-    ns = head_split(M, V)
+    fn = _head_entry(z, W)
+    ns = head_split(M, V, z.dtype) if nsplit is None else nsplit
     s = _C.stream_ptr()
     args = (_C.ptr(z), _C.ptr(W), _C.ptr(bias), _C.ptr(target), M, V, K, int(vocab_offset), k, ns)
     if st is None:
         st = torch.full((M,), float("-inf"), dtype=torch.float32, device=dev)
-        _C.call("mobgt_head_topk", *args, 0, _C.ptr(st), None, None, None, None, None, None, s)
+        _C.call(fn, *args, 0, _C.ptr(st), None, None, None, None, None, None, s)
     tv = torch.empty(M, ns, k, dtype=torch.float32, device=dev)
     ti = torch.empty(M, ns, k, dtype=torch.int32, device=dev)
     cg = torch.empty(M, ns, dtype=torch.int32, device=dev)
     ce = torch.empty(M, ns, dtype=torch.int32, device=dev)
     logits = torch.empty(M, V, dtype=torch.float32, device=dev) if dump_logits else None
-    share = torch.zeros(M, dtype=torch.int32, device=dev)       # per-row pruning bound shared by all lists of the row
-    _C.call("mobgt_head_topk", *args, 1, _C.ptr(st), _C.ptr(tv), _C.ptr(ti), _C.ptr(cg), _C.ptr(ce), _C.ptr(logits), _C.ptr(share), s)
+    # per-row pruning bound shared by all lists of the row (the fp32 head keeps its lists independent and takes none)
+    share = torch.zeros(M, dtype=torch.int32, device=dev) if fn == "mobgt_head_topk" else None
+    _C.call(fn, *args, 1, _C.ptr(st), _C.ptr(tv), _C.ptr(ti), _C.ptr(cg), _C.ptr(ce), _C.ptr(logits), _C.ptr(share), s)
     val = torch.empty(M, k, dtype=torch.float32, device=dev)
     idx = torch.empty(M, k, dtype=torch.int32, device=dev)
     cnt = torch.empty(M, dtype=torch.int32, device=dev)
@@ -1146,12 +1177,14 @@ def head_topk_local(z, W, bias, target, k, vocab_offset=0, st=None, dump_logits=
 
 
 def head_target_logit(z, W, bias, target, vocab_offset=0):
-    """mode 0 only: st[row] = target logit if this shard owns the target, else -inf."""
+    """mode 0 only: st[row] = target logit if this shard owns the target, else -inf.  bf16 or float32 operands, as
+    head_topk_local."""
     M, K = z.shape
     V = W.shape[0]
     st = torch.full((M,), float("-inf"), dtype=torch.float32, device=z.device)
-    _C.call("mobgt_head_topk", _C.ptr(z), _C.ptr(W), _C.ptr(bias), _C.ptr(target), M, V, K, int(vocab_offset), 1,
-            2, 0, _C.ptr(st), None, None, None, None, None, None, _C.stream_ptr())
+    fn = _head_entry(z, W)
+    _C.call(fn, _C.ptr(z), _C.ptr(W), _C.ptr(bias), _C.ptr(target), M, V, K, int(vocab_offset), 1,
+            2 if fn == "mobgt_head_topk" else 4, 0, _C.ptr(st), None, None, None, None, None, None, _C.stream_ptr())
     return st
 
 
