@@ -36,6 +36,7 @@ extern "C" {
 
 #define MOBGT_UNREACHABLE 510 /* algos.pyx:32 — the reference's "infinity" */
 #define MOBGT_MAX_NODES 512   /* rel_pos_encoder has 512 rows (model_fqandtoyo.py:788) */
+#define MOBGT_MAX_APSP_NODES 1024 /* K1 alone (the algos drop-in): graphs the model cannot take still get M, path, edges */
 #define MOBGT_MAX_HOPS 32
 
 /* dtype tags for float tensors crossing the ABI */
@@ -56,8 +57,9 @@ int32_t mobgt_device_check(void);
  * algos.gen_edge_input (:65-96) as driven by preprocess_item (wrapper.py:42-61,99) and
  * the hop-axis slice of the collators (collator.py:323).
  *
- * Graphs are packed: graph g has n[g] nodes (1..512) and owns n[g]^2 cells starting at
- * cell offset sq_off[g] of every per-cell array.
+ * Graphs are packed: graph g has n[g] nodes (1..MOBGT_MAX_APSP_NODES = 1024) and owns n[g]^2
+ * cells starting at cell offset sq_off[g] of every per-cell array.  The model's kernels (K2/K3)
+ * take at most MOBGT_MAX_NODES = 512; larger graphs are for the algos drop-in.
  *   feat      u8  [sum n^2]       attn_edge_type (wrapper.py:49-53): 0 = no edge, else
  *                                 edge feature (count+2).  adjacency = (feat != 0).
  *   dist      i16 [sum n^2]       M + shift        (M in 0..509 | 510)          (out)
@@ -71,6 +73,10 @@ int32_t mobgt_device_check(void);
  * walked (1 <= dk <= hops; the reference's default is 5, entry.py / data.py:204): slots [dk, hops) stay "no hop".
  * gids (i32 [G_launch], may be NULL = identity) selects which graphs this launch covers;
  * n_max_host is the largest n among them (chooses the cluster size / shared-memory plan).
+ * n_max_host > 1024 returns MOBGT_ERR_BAD_SHAPE.  n_max_host > 512 needs a non-null `path`
+ * (else MOBGT_ERR_NULL): that plan keeps only M in shared memory, writes `path` to global memory
+ * and expands it into edge_in with a second kernel of the same call; MOBGT_ERR_UNSUPPORTED if its
+ * cluster (8 or 16 CTAs) cannot be resident on the device.
  * ------------------------------------------------------------------------------------------ */
 int32_t mobgt_apsp_edge_input(const uint8_t *feat, const int32_t *n, const int64_t *sq_off,
                               const int32_t *gids, int32_t G_launch, int32_t n_max_host,
@@ -80,7 +86,7 @@ int32_t mobgt_apsp_edge_input(const uint8_t *feat, const int32_t *n, const int64
 
 /* Stand-alone mirror of algos.gen_edge_input(max_dist, path, edge_feat) (algos.pyx:65-96) for a
  * caller that already holds a floyd_warshall `path` matrix (i16, packed like above).
- * Writes the first `hops` hop slots; same encoding as edge_in above. */
+ * Writes the first `hops` hop slots (1..510); same encoding as edge_in above.  n_max_host <= 1024. */
 int32_t mobgt_gen_edge_input(const int16_t *path, const uint8_t *feat, const int32_t *n,
                              const int64_t *sq_off, int32_t G, int32_t n_max_host, int32_t hops,
                              int32_t shift, uint8_t *edge_in, void *stream);

@@ -15,8 +15,9 @@ from . import _C
 
 UNREACHABLE = 510
 # size classes: one launch per class so that tiny graphs do not inherit the block / cluster
-# shape of the largest one
-_CLASSES = (8, 16, 32, 64, 128, 184, 256, 512)
+# shape of the largest one.  (512, 1024] is the plan for graphs the model cannot take (K1 only: the
+# algos drop-in); its walk reads `path`, so that class always gets a path buffer.
+_CLASSES = (8, 16, 32, 64, 128, 184, 256, 512, _C.MAX_APSP_NODES)
 
 
 def pack_graphs(n_host):
@@ -69,9 +70,12 @@ def apsp_edge_input_packed(feat, n_dev, sq_off_dev, n_host, hops, shift=0, want_
             gids = None
         else:
             gids = torch.from_numpy(sel.astype(np.int32)).to(dev, non_blocking=True)
+        p = path
+        if p is None and hi > _C.MAX_NODES:
+            p = torch.empty(cells, dtype=torch.int16, device=dev)     # the walk's input; freed after the call (stream-ordered)
         _C.call("mobgt_apsp_edge_input", _C.ptr(feat), _C.ptr(n_dev), _C.ptr(sq_off_dev), _C.ptr(gids),
                 int(len(sel)), int(n_host[sel].max()), int(hops), dk, int(shift),
-                _C.ptr(dist), _C.ptr(path), _C.ptr(edge_in), _C.ptr(maxdist), s)
+                _C.ptr(dist), _C.ptr(p), _C.ptr(edge_in), _C.ptr(maxdist), s)
     return dict(dist=dist, path=path, edge_in=edge_in, maxdist=maxdist)
 
 

@@ -514,6 +514,8 @@ def collate_from_host(hp, world=None, latlon_dev=None, multi_hop_max_dist=20, re
         b.size_order = size_order
     else:
         b.build_plans()
+    if len(ns) and int(ns.max()) > _C.MAX_NODES:        # K1 takes up to 1024 nodes, the model's kernels (K2 / K3) 512
+        raise ValueError(f"node counts must be in [1, {_C.MAX_NODES}]")
     k1 = apsp_edge_input_packed(b.feat8, b.n, b.sq_off, ns, hops=hops, shift=1, want_path=want_path, dk=dk)
     b.rel_pos16, b.edge_in8, b.maxdist, b.path16 = k1["dist"], k1["edge_in"], k1["maxdist"], k1["path"]
     b.poi_pos16 = torch.empty(hp.cells, dtype=torch.int16, device=dev)

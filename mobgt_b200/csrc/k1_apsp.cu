@@ -23,7 +23,10 @@
 //     "path == 0 means direct" short-circuit, algos.pyx:59-60).  DESIGN.md proves that
 //     walking cur = X[cur][j] emits exactly the reference's hop sequence;
 //   * the walk writes only the first `hops` hop slots (collator.py:323 slices the rest away),
-//     staged per warp in shared memory and stored as coalesced 32-bit words.
+//     staged per warp in shared memory and stored as coalesced 32-bit words;
+//   * graphs of 513..1024 nodes (the algos drop-in only) use k1_apsp_large_kernel: M alone in the
+//     shared memory of an 8- or 16-CTA cluster, `path` in global memory, expanded by
+//     k1_walk_from_path_kernel in the same call.
 #include <cooperative_groups.h>
 #include <cstdlib>
 
@@ -307,13 +310,146 @@ __global__ void __launch_bounds__(1024) k1_apsp_kernel(const K1Params p, const i
     }
 }
 
+// ---- graphs of 513..1024 nodes (MOBGT_MAX_APSP_NODES) ------------------------------------------
+// Same Floyd-Warshall (k strictly ascending, strict '>', saturating 510, one cluster barrier per k, column k of M broadcast
+// through DSMEM), but only M stays in shared memory: the state of three matrices no longer fits a cluster at n = 600.  X is
+// dropped and P, written only on a strict improvement, goes straight to the caller's `path` buffer: for n > 510 the
+// reference's `path` is needed anyway (the skip510 rule reads it), and the walk then expands it with
+// k1_walk_from_path_kernel, the reference's leftmost descent.  Rows of P start at any cell, so P is stored per cell.
+constexpr int kLargeThreads = 1024;
+
+__host__ inline size_t k1_large_smem_bytes(int n, int C) {
+    return (size_t)n * k1_W(n, C) * 2 + (size_t)2 * round_up(n, 8) * 2 + 16;   // M slice + colM[2][n8]
+}
+
+__global__ void __launch_bounds__(kLargeThreads) k1_apsp_large_kernel(const K1Params p, const int C) {
+    cg::cluster_group cluster = cg::this_cluster();
+    const int crank = (int)cluster.block_rank();
+    const int gl = blockIdx.x / C;
+    const int g = p.gids ? p.gids[gl] : gl;
+    const int n = p.n[g];
+    const int64_t off = p.sq_off[g];
+    const int W = k1_W(n, C);
+    const int c0 = crank * W;
+    const int n8 = round_up(n, 8);
+    const int cpr = W >> 3;
+    const int tid = threadIdx.x, NT = blockDim.x;
+
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    uint16_t *Msh = reinterpret_cast<uint16_t *>(smem_raw);
+    uint16_t *colM = Msh + (size_t)n * W;   // [2][n8]
+    const uint8_t *feat = p.feat + off;
+    int16_t *P = p.path + off;
+    const int ntask = n * cpr;
+
+    // ---- init (algos.pyx:27-32): diag 0, edge 1, else 510; P = 0.  Cell (i, j) is owned by one thread for the whole kernel,
+    // so its P stores (init, improvements, finalize) are ordered by program order alone.
+    for (int t = tid; t < ntask; t += NT) {
+        const int i = t / cpr, q = t - i * cpr;
+        uint32_t mw[4];
+#pragma unroll
+        for (int e2 = 0; e2 < 4; ++e2) {
+            uint32_t mm[2];
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int j = c0 + q * 8 + e2 * 2 + h;
+                uint32_t m = kInf;
+                if (j < n) {
+                    const uint8_t f = __ldg(feat + (size_t)i * n + j);
+                    m = (i == j) ? 0u : (f ? 1u : kInf);
+                    P[(size_t)i * n + j] = 0;
+                }
+                mm[h] = m;
+            }
+            mw[e2] = mm[0] | (mm[1] << 16);
+        }
+        *reinterpret_cast<uint4 *>(Msh + (size_t)i * W + q * 8) = make_uint4(mw[0], mw[1], mw[2], mw[3]);
+    }
+    for (int i = tid; i < n; i += NT) {
+        const uint8_t f = __ldg(feat + (size_t)i * n);
+        colM[i] = (uint16_t)((i == 0) ? 0u : (f ? 1u : kInf));
+    }
+    cluster.sync();
+
+    // ---- Floyd-Warshall, k strictly ascending (algos.pyx:35-45) ---------------------------------
+    const int dr = NT / cpr, dq = NT - dr * cpr;
+    const int i0 = tid / cpr, q0 = tid - i0 * cpr;
+    for (int k = 0; k < n; ++k) {
+        const uint16_t *cM = colM + (k & 1) * n8;
+        const int nb = ((k + 1) & 1) * n8;
+        const int kn = k + 1;
+        const bool own_next = (kn < n) && (kn >= c0) && (kn < c0 + W);
+        const int qn = own_next ? ((kn - c0) >> 3) : -1;
+        const int en = (kn - c0) & 7;
+        const uint16_t *rowk = Msh + (size_t)k * W;
+
+        int i = i0, q = q0;
+        for (int t = tid; t < ntask; t += NT) {
+            const uint32_t mik = cM[i];
+            const bool pub = (q == qn);
+            if (mik < kInf || pub) {
+                uint16_t *mp = Msh + (size_t)i * W + q * 8;
+                uint4 m4 = *reinterpret_cast<const uint4 *>(mp);
+                if (mik < kInf) {
+                    const uint4 r4 = *reinterpret_cast<const uint4 *>(rowk + q * 8);
+                    const uint32_t mik2 = mik * 0x10001u;
+                    const uint32_t d[4] = {relax2(m4.x, r4.x, mik2), relax2(m4.y, r4.y, mik2), relax2(m4.z, r4.z, mik2),
+                                           relax2(m4.w, r4.w, mik2)};
+                    if (d[0] | d[1] | d[2] | d[3]) {
+                        *reinterpret_cast<uint4 *>(mp) = m4;
+                        if (k != 0) {  // k == 0: path stays 0 == "direct" (algos.pyx:59-60)
+                            const int jb = c0 + q * 8;
+                            int16_t *pr = P + (size_t)i * n + jb;
+#pragma unroll
+                            for (int e = 0; e < 8; ++e)
+                                if (((d[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu) && jb + e < n) pr[e] = (int16_t)k;
+                        }
+                    }
+                }
+                if (pub) {  // broadcast column k+1 (post-step-k values) to every CTA of the cluster
+                    const uint16_t mv = (uint16_t)pick16(m4, en);
+                    for (int r = 0; r < C; ++r) cluster.map_shared_rank(colM, r)[nb + i] = mv;
+                }
+            }
+            q += dq;
+            i += dr;
+            if (q >= cpr) { q -= cpr; ++i; }
+        }
+        cluster.sync();
+    }
+
+    // ---- finalize (algos.pyx:48-52) + dist / maxdist; unreachable pairs get path = 510 -------------
+    int local_max = 0;
+    for (int t = tid; t < ntask; t += NT) {
+        const int i = t / cpr, q = t - i * cpr;
+        const uint4 m4 = *reinterpret_cast<const uint4 *>(Msh + (size_t)i * W + q * 8);
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+            const int j = c0 + q * 8 + e;
+            if (j < n) {
+                const uint32_t m = pick16(m4, e);
+                const size_t o = (size_t)i * n + j;
+                p.dist[off + o] = (int16_t)(m + p.shift);
+                if (m >= kInf) P[o] = (int16_t)kInf;
+                local_max = max(local_max, (int)m);
+            }
+        }
+    }
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) local_max = max(local_max, __shfl_xor_sync(0xffffffffu, local_max, s));
+    if ((tid & 31) == 0) atomicMax(p.maxdist + g, local_max);
+}
+
 // Stand-alone gen_edge_input from a floyd_warshall `path` matrix: hop h+1 of (cur -> j) is found
 // by the leftmost descent of the reference's recursion (algos.pyx:57-62): t = j; while path[cur][t]
-// != 0: t = path[cur][t].  One thread per ordered pair; not a hot path (API mirror).
+// != 0: t = path[cur][t].  One thread per ordered pair; walks the first `dk` hops and writes all `hops`
+// slots of the row (the rest "no hop").  gids (may be NULL = identity) maps blockIdx.y to a graph.
+// The API mirror, and the walk of the graphs above 512 nodes.
 __global__ void k1_walk_from_path_kernel(const int16_t *__restrict__ path, const uint8_t *__restrict__ feat,
                                          const int32_t *__restrict__ n_arr, const int64_t *__restrict__ sq_off,
-                                         int hops, int shift, uint8_t *__restrict__ edge_in) {
-    const int g = blockIdx.y;
+                                         const int32_t *__restrict__ gids, int hops, int dk, int shift,
+                                         uint8_t *__restrict__ edge_in) {
+    const int g = gids ? gids[blockIdx.y] : blockIdx.y;
     const int n = n_arr[g];
     const int64_t off = sq_off[g];
     const uint8_t none = (uint8_t)(shift - 1);
@@ -324,7 +460,7 @@ __global__ void k1_walk_from_path_kernel(const int16_t *__restrict__ path, const
         const int pij = path[off + c];
         if (i != j && pij != (int)kInf) {
             int cur = i;
-            for (; h < hops; ++h) {
+            for (; h < dk; ++h) {
                 int t = j;
                 for (int guard = 0; guard < n; ++guard) {
                     const int k = path[off + (size_t)cur * n + t];
@@ -393,6 +529,61 @@ static int pick_cluster(int n, int G, bool with_path, int hops, bool want_feat, 
     return -1;
 }
 
+// k1_walk_from_path_kernel grid: one thread per pair up to ~4 waves of 256-thread CTAs over the launch (a single graph of a
+// per-item call then still spreads over every SM), at least 64 CTAs per graph
+static dim3 walk_grid(int n_max, int G) {
+    const int cells = n_max * n_max;
+    return dim3((unsigned)min(ceil_div(cells, 256), max(64, ceil_div(4 * 8 * kNumSMs, G))), (unsigned)G);
+}
+
+// n in (512, MOBGT_MAX_APSP_NODES]: the smallest cluster, 8 (portable) or 16 (non-portable) CTAs, whose M slice fits.
+static int pick_cluster_large(int n, size_t *smem_out) {
+    for (int C = 8; C <= 16; C *= 2) {
+        const size_t sm = k1_large_smem_bytes(n, C);
+        if (sm <= 227 * 1024) {
+            *smem_out = sm;
+            return C;
+        }
+    }
+    return -1;
+}
+
+static int32_t apsp_edge_input_large(const K1Params &p, int G_launch, int n_max, cudaStream_t s) {
+    MOBGT_REQUIRE(G_launch <= 65535, MOBGT_ERR_BAD_SHAPE, "mobgt_apsp_edge_input: G_launch=%d > 65535 graphs of more than %d nodes",
+                  G_launch, MOBGT_MAX_NODES);
+    size_t smem = 0;
+    const int C = pick_cluster_large(n_max, &smem);
+    MOBGT_REQUIRE(C > 0, MOBGT_ERR_UNSUPPORTED, "mobgt_apsp_edge_input: no shared-memory plan for n=%d", n_max);
+    auto kern = k1_apsp_large_kernel;
+    MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (C > 8) MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)G_launch * C);
+    cfg.blockDim = dim3(kLargeThreads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = C;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    int resident = 0;
+    MOBGT_CUDA_OK(cudaOccupancyMaxActiveClusters(&resident, kern, &cfg));
+    MOBGT_REQUIRE(resident >= 1, MOBGT_ERR_UNSUPPORTED,
+                  "mobgt_apsp_edge_input: a cluster of %d CTAs x %zu B shared memory (n=%d) cannot be resident on this device",
+                  C, smem, n_max);
+    MOBGT_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, p, C));
+    count_launch();
+    if (p.edge_in != nullptr) {
+        k1_walk_from_path_kernel<<<walk_grid(n_max, G_launch), 256, 0, s>>>(p.path, p.feat, p.n, p.sq_off, p.gids, p.hops,
+                                                                             p.dk, p.shift, p.edge_in);
+        MOBGT_LAUNCH_OK("k1_walk_from_path_kernel");
+    }
+    return MOBGT_OK;
+}
+
 }  // namespace mobgt
 
 using namespace mobgt;
@@ -403,8 +594,11 @@ extern "C" int32_t mobgt_apsp_edge_input(const uint8_t *feat, const int32_t *n, 
                                          int32_t *maxdist, void *stream) {
     MOBGT_REQUIRE(feat && n && sq_off && dist && maxdist, MOBGT_ERR_NULL, "mobgt_apsp_edge_input: null pointer");
     MOBGT_REQUIRE(G_launch >= 0, MOBGT_ERR_BAD_SHAPE, "mobgt_apsp_edge_input: G_launch=%d", G_launch);
-    MOBGT_REQUIRE(n_max_host >= 1 && n_max_host <= MOBGT_MAX_NODES, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_apsp_edge_input: n_max=%d outside [1,%d]", n_max_host, MOBGT_MAX_NODES);
+    MOBGT_REQUIRE(n_max_host >= 1 && n_max_host <= MOBGT_MAX_APSP_NODES, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_apsp_edge_input: n_max=%d outside [1,%d]", n_max_host, MOBGT_MAX_APSP_NODES);
+    MOBGT_REQUIRE(path != nullptr || n_max_host <= MOBGT_MAX_NODES, MOBGT_ERR_NULL,
+                  "mobgt_apsp_edge_input: n_max=%d > %d needs a non-null path buffer (the edge walk reads it)", n_max_host,
+                  MOBGT_MAX_NODES);
     MOBGT_REQUIRE(shift == 0 || shift == 1, MOBGT_ERR_BAD_SHAPE, "mobgt_apsp_edge_input: shift must be 0 or 1");
     if (edge_in) {
         MOBGT_REQUIRE(hops >= 4 && hops <= MOBGT_MAX_HOPS && hops % 4 == 0, MOBGT_ERR_UNSUPPORTED,
@@ -415,6 +609,9 @@ extern "C" int32_t mobgt_apsp_edge_input(const uint8_t *feat, const int32_t *n, 
     }
     if (G_launch == 0) return MOBGT_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (n_max_host > MOBGT_MAX_NODES)
+        return apsp_edge_input_large(K1Params{feat, n, sq_off, gids, hops, dk, shift, dist, path, edge_in, maxdist}, G_launch,
+                                     n_max_host, s);
     const bool with_path = path != nullptr || n_max_host > MOBGT_UNREACHABLE;   // see skip510 in the kernel
     int nt = 0, feat_in_smem = 0;
     size_t smem = 0;
@@ -446,13 +643,11 @@ extern "C" int32_t mobgt_gen_edge_input(const int16_t *path, const uint8_t *feat
                                         int32_t shift, uint8_t *edge_in, void *stream) {
     MOBGT_REQUIRE(path && feat && n && sq_off && edge_in, MOBGT_ERR_NULL, "mobgt_gen_edge_input: null pointer");
     MOBGT_REQUIRE(hops >= 1 && hops <= MOBGT_UNREACHABLE, MOBGT_ERR_BAD_SHAPE, "mobgt_gen_edge_input: hops=%d", hops);
-    MOBGT_REQUIRE(n_max_host >= 1 && n_max_host <= MOBGT_MAX_NODES, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_gen_edge_input: n_max=%d", n_max_host);
+    MOBGT_REQUIRE(n_max_host >= 1 && n_max_host <= MOBGT_MAX_APSP_NODES, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_gen_edge_input: n_max=%d outside [1,%d]", n_max_host, MOBGT_MAX_APSP_NODES);
     if (G <= 0) return MOBGT_OK;
-    const int cells = n_max_host * n_max_host;
-    dim3 grid((unsigned)min(64, ceil_div(cells, 256)), (unsigned)G);
-    k1_walk_from_path_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(path, feat, n, sq_off, hops, shift,
-                                                                                 edge_in);
+    k1_walk_from_path_kernel<<<walk_grid(n_max_host, G), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        path, feat, n, sq_off, nullptr, hops, hops, shift, edge_in);
     MOBGT_LAUNCH_OK("k1_walk_from_path_kernel");
     return MOBGT_OK;
 }
