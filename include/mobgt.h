@@ -35,8 +35,9 @@ extern "C" {
 #define MOBGT_ERR_NULL (-6)
 
 #define MOBGT_UNREACHABLE 510 /* algos.pyx:32 — the reference's "infinity" */
-#define MOBGT_MAX_NODES 512   /* rel_pos_encoder has 512 rows (model_fqandtoyo.py:788) */
+#define MOBGT_MAX_NODES 512   /* rel_pos_encoder has 512 rows (model_fqandtoyo.py:788); the collator's default cap */
 #define MOBGT_MAX_APSP_NODES 1024 /* K1 alone (the algos drop-in): graphs the model cannot take still get M, path, edges */
+#define MOBGT_MAX_MODEL_NODES 1024 /* K2 / K3: graphs of up to 1024 nodes, T <= 1025 tokens (the collator's large_graphs mode) */
 #define MOBGT_MAX_HOPS 32
 
 /* dtype tags for float tensors crossing the ABI */

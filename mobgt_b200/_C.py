@@ -13,7 +13,8 @@ LIB_PATH = os.path.join(HERE, "lib", "libmobgt.so")
 c_i32, c_i64, c_p, c_f32 = ctypes.c_int32, ctypes.c_int64, ctypes.c_void_p, ctypes.c_float
 
 # include/mobgt.h limits
-MAX_NODES = 512          # MOBGT_MAX_NODES: the model's kernels (K2 / K3)
+MAX_NODES = 512          # MOBGT_MAX_NODES: the collator's default cap
+MAX_MODEL_NODES = 1024   # MOBGT_MAX_MODEL_NODES: the model's kernels (K2 / K3), T <= 1025 (collator large_graphs=True)
 MAX_APSP_NODES = 1024    # MOBGT_MAX_APSP_NODES: K1 (mobgt_apsp_edge_input, mobgt_gen_edge_input)
 
 

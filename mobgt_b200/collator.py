@@ -52,15 +52,15 @@ _staging = {}
 class _PackStream(torch.utils.data.IterableDataset):
     """Worker-side half of PackedLoader: worker w packs the batches i = w (mod num_workers) of the stream."""
 
-    def __init__(self, batches, max_node, bucket=False):
-        self.batches, self.max_node, self.bucket = batches, max_node, bucket
+    def __init__(self, batches, max_node, bucket=False, large_graphs=False):
+        self.batches, self.max_node, self.bucket, self.large_graphs = batches, max_node, bucket, large_graphs
 
     def __iter__(self):
         info = torch.utils.data.get_worker_info()
         w, nw = (info.id, info.num_workers) if info is not None else (0, 1)
         for i, items in enumerate(self.batches):
             if i % nw == w:
-                hp = pack_host(items, self.max_node, bucket=self.bucket)
+                hp = pack_host(items, self.max_node, bucket=self.bucket, large_graphs=self.large_graphs)
                 yield dict(buf=torch.from_numpy(hp.buf), layout=hp.layout, B=hp.B, N=hp.N, ns=torch.from_numpy(hp.ns), cells=hp.cells,
                            padded=hp.padded)
 
@@ -78,14 +78,16 @@ class PackedLoader:
     `current()` makes the consumer's stream wait for the batch (event) and registers the batch's memory with that stream.
     """
 
-    def __init__(self, batches, collate_fn=None, num_workers=0, max_node=512, side_stream=True, bucket=False, **collate_kw):
+    def __init__(self, batches, collate_fn=None, num_workers=0, max_node=512, side_stream=True, bucket=False, large_graphs=False,
+                 **collate_kw):
         """bucket=True: every batch is padded to a few size buckets (see `pack_host`), so that batches of different graphs
-        share packed shapes and the trainer's CUDA graphs replay instead of re-capturing / running eagerly."""
-        self._kw = collate_kw
+        share packed shapes and the trainer's CUDA graphs replay instead of re-capturing / running eagerly.
+        large_graphs=True: graphs of up to MAX_MODEL_NODES (1024) nodes are collated (see `collate_from_host`)."""
+        self._kw = dict(collate_kw, large_graphs=large_graphs)
         self._stream = torch.cuda.Stream() if (side_stream and torch.cuda.is_available()) else None
         self._gate = None
         if num_workers > 0:
-            ds = _PackStream(batches, max_node, bucket)
+            ds = _PackStream(batches, max_node, bucket, large_graphs)
             dl = torch.utils.data.DataLoader(ds, batch_size=None, num_workers=num_workers, pin_memory=False, prefetch_factor=2,
                                              persistent_workers=False)
             self._it = iter(dl)
@@ -355,9 +357,9 @@ class HostPack:
         self.buf, self.layout, self.B, self.N, self.ns, self.cells, self.padded = buf, layout, B, N, ns, cells, padded
 
 
-def _bucket_sizes(ntok, cells, nmax, B):
+def _bucket_sizes(ntok, cells, nmax, B, large_graphs=False):
     """Bucketed (tokens, cells, max nodes): tokens to a multiple of 512 (GEMM rows: the cost that scales), cells to a power
-    of two (memory only), the node cap to a power of two (tile counts of K2 / K3)."""
+    of two (memory only), the node cap to a power of two (tile counts of K2 / K3), at most 512 — or 1024 with large_graphs."""
     ntok_b = max(512, (ntok + 511) // 512 * 512)
     cells_b = 4096
     while cells_b < cells:
@@ -365,7 +367,7 @@ def _bucket_sizes(ntok, cells, nmax, B):
     n_b = 8
     while n_b < nmax:
         n_b *= 2
-    return ntok_b, cells_b, min(n_b, 512)
+    return ntok_b, cells_b, min(n_b, _node_cap(large_graphs))
 
 
 def _host_plan(keys):
@@ -376,13 +378,27 @@ def _host_plan(keys):
     return perm, k[perm].astype(np.int32)
 
 
-def pack_host(items, max_node=512, bucket=False):
+def _node_cap(large_graphs):
+    return _C.MAX_MODEL_NODES if large_graphs else _C.MAX_NODES
+
+
+def _check_node_cap(ns, large_graphs):
+    """The model's kernels (K2 / K3) take graphs of up to MAX_NODES = 512 nodes, and of up to MAX_MODEL_NODES = 1024 in the
+    opt-in large_graphs mode (K1 alone takes 1024 either way)."""
+    cap = _node_cap(large_graphs)
+    if len(ns) and int(np.max(ns)) > cap:
+        hint = "" if large_graphs else f" (large_graphs=True takes up to {_C.MAX_MODEL_NODES})"
+        raise ValueError(f"node counts must be in [1, {cap}]{hint}")
+
+
+def pack_host(items, max_node=512, bucket=False, large_graphs=False):
     """raw dataset items (owndata.py:340-349 fields; numpy or torch) -> HostPack.  No CUDA, no torch ops on the hot path.
 
     bucket=True pads the per-token / per-node / per-cell arrays to bucket sizes (`_bucket_sizes`): padding tokens are extra
     "graph tokens" that belong to no graph (no tok_off range covers them, so attention never reads or writes them and their
     gradient is exactly zero), padding nodes map to them one to one with padding-row indices, padding cells are never indexed.
-    Per-graph sizes (n, offsets) are untouched, so every result for the real graphs is identical to the unpadded batch."""
+    Per-graph sizes (n, offsets) are untouched, so every result for the real graphs is identical to the unpadded batch.
+    large_graphs: see `collate_from_host` (here it only lets the bucketed node cap reach 1024)."""
     items = [it for it in items if it is not None and len(_to_np(it.x)) <= max_node]     # collator.py:313
     B = len(items)
     ns = np.array([len(_to_np(it.x)) for it in items], np.int32)
@@ -431,7 +447,7 @@ def pack_host(items, max_node=512, bucket=False):
     in_deg, out_deg, node_rows = indeg + 1, outdeg + 1, rows.astype(np.int64)    # pad_1d_unsqueeze "+1" (collator.py:12)
     N_out, cells_alloc, padded = (int(ns.max()) if B else 0), cells, False
     if bucket and B:
-        ntok_b, cells_alloc, N_out = _bucket_sizes(Ntok, cells, int(ns.max()), B)
+        ntok_b, cells_alloc, N_out = _bucket_sizes(Ntok, cells, int(ns.max()), B, large_graphs)
         pad = ntok_b - Ntok                                   # padding tokens == padding nodes (Ntok = Nn + B)
         if pad or cells_alloc != cells or N_out != int(ns.max()):
             padded = True
@@ -496,8 +512,12 @@ def _upload_pack(hp, dev):
     return out
 
 
-def collate_from_host(hp, world=None, latlon_dev=None, multi_hop_max_dist=20, rel_pos_max=1024, device="cuda", want_path=False):
-    """The device half of collation: one H2D copy, the K4-backward sort plans, K1 (APSP + path edges) and poi_pos."""
+def collate_from_host(hp, world=None, latlon_dev=None, multi_hop_max_dist=20, rel_pos_max=1024, device="cuda", want_path=False,
+                      large_graphs=False):
+    """The device half of collation: one H2D copy, the K4-backward sort plans, K1 (APSP + path edges) and poi_pos.
+    Graphs above 512 nodes raise ValueError unless large_graphs=True, which takes up to 1024 (T <= 1025 tokens: the
+    attention-bias and attention kernels run such graphs on their large-graph paths)."""
+    _check_node_cap(hp.ns.numpy() if isinstance(hp.ns, torch.Tensor) else hp.ns, large_graphs)
     _C.require_cuda()
     dev = torch.device(device)
     views = _upload_pack(hp, dev)
@@ -514,8 +534,6 @@ def collate_from_host(hp, world=None, latlon_dev=None, multi_hop_max_dist=20, re
         b.size_order = size_order
     else:
         b.build_plans()
-    if len(ns) and int(ns.max()) > _C.MAX_NODES:        # K1 takes up to 1024 nodes, the model's kernels (K2 / K3) 512
-        raise ValueError(f"node counts must be in [1, {_C.MAX_NODES}]")
     k1 = apsp_edge_input_packed(b.feat8, b.n, b.sq_off, ns, hops=hops, shift=1, want_path=want_path, dk=dk)
     b.rel_pos16, b.edge_in8, b.maxdist, b.path16 = k1["dist"], k1["edge_in"], k1["maxdist"], k1["path"]
     b.poi_pos16 = torch.empty(hp.cells, dtype=torch.int16, device=dev)
@@ -531,13 +549,13 @@ def collate_from_host(hp, world=None, latlon_dev=None, multi_hop_max_dist=20, re
 
 
 def collate_packed(items, world=None, latlon_dev=None, max_node=512, multi_hop_max_dist=20, rel_pos_max=1024,
-                   device="cuda", want_path=False, bucket=False):
+                   device="cuda", want_path=False, bucket=False, large_graphs=False):
     """Shared body of the three POI collators.  items: raw dataset items (owndata.py:340-349 fields; numpy or
     torch).  Returns a device-resident Batch1.  bucket: see `pack_host` (training loaders; the reference-shaped dense views
     of a bucketed batch are padded to the bucket's node cap instead of the batch maximum)."""
     _C.require_cuda()
-    return collate_from_host(pack_host(items, max_node, bucket=bucket), world, latlon_dev, multi_hop_max_dist, rel_pos_max, device,
-                             want_path)
+    return collate_from_host(pack_host(items, max_node, bucket=bucket, large_graphs=large_graphs), world, latlon_dev,
+                             multi_hop_max_dist, rel_pos_max, device, want_path, large_graphs)
 
 
 def collator_foursquare(items, max_node=512, multi_hop_max_dist=20, rel_pos_max=20, world=None, latlon_dev=None, **kw):

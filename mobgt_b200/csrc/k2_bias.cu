@@ -184,7 +184,7 @@ __global__ void __launch_bounds__(512, 2) k2_bias_fwd_kernel(const K2Common c, c
     const int half = c.Tp >> (kCells - 1);        // threads per plane row (cell pairs at 8 heads, cells at 12)
     const int per_graph = c.T * half;
     const int tiles = ceil_div(per_graph, (int)blockDim.x);
-    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^19
+    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^40 / half (> 2^30)
     const size_t hs = (size_t)c.T * c.Tp;
     for (int w = blockIdx.x; w < tiles * c.B; w += gridDim.x) {
         const int g = w / tiles, tile = w - g * tiles;
@@ -783,7 +783,7 @@ __global__ void __launch_bounds__(512, 2) k2_direct_fwd_kernel(const K2Common c,
     const int half = c.Tp >> (kCells - 1);        // threads per plane row
     const int per_graph = c.T * half;
     const int tiles = ceil_div(per_graph, (int)blockDim.x);
-    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^19
+    const uint64_t half_magic = ((1ull << 40) + half - 1) / half;     // f / half == (f * magic) >> 40 for f < 2^40 / half (> 2^30)
     const size_t hs = (size_t)c.T * c.Tp;
     for (int w = blockIdx.x; w < tiles * c.B; w += gridDim.x) {
         const int g = w / tiles, tile = w - g * tiles;
@@ -1042,7 +1042,8 @@ extern "C" int32_t mobgt_bias_fwd(const int32_t *n, const int64_t *sq_off, const
                   "mobgt_bias_fwd: hops=%d must be a multiple of 4 in [4,%d]", hops, MOBGT_MAX_HOPS);
     MOBGT_REQUIRE(dk >= 1 && dk <= hops, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: dk=%d outside [1, hops=%d]", dk, hops);
     MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: num_bins=%d", num_bins);
-    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_fwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE(T >= 2 && T <= MOBGT_MAX_MODEL_NODES + 1 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_fwd: T=%d Tp=%d (T <= 1025: graphs of at most 1024 nodes)", T, Tp);
     MOBGT_REQUIRE(out_dtype == MOBGT_F32 || out_dtype == MOBGT_BF16, MOBGT_ERR_BAD_DTYPE, "mobgt_bias_fwd: dtype");
     if (B <= 0) return MOBGT_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -1145,7 +1146,8 @@ extern "C" int32_t mobgt_bias_bwd(const int32_t *n, const int64_t *sq_off, const
     MOBGT_REQUIRE(hops >= 4 && hops <= MOBGT_MAX_HOPS && hops % 4 == 0 && num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE,
                   "mobgt_bias_bwd: hops=%d num_bins=%d", hops, num_bins);
     MOBGT_REQUIRE(dk >= 1 && dk <= hops, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: dk=%d outside [1, hops=%d]", dk, hops);
-    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_bwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE(T >= 2 && T <= MOBGT_MAX_MODEL_NODES + 1 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_bwd: T=%d Tp=%d (T <= 1025: graphs of at most 1024 nodes)", T, Tp);
     MOBGT_REQUIRE((dbias_dtype == MOBGT_F32 && n_layers == 1) || (dbias_dtype == MOBGT_BF16 && n_layers >= 1 && n_layers <= 64),
                   MOBGT_ERR_BAD_DTYPE, "mobgt_bias_bwd: dbias dtype %d with %d layer planes", dbias_dtype, n_layers);
     MOBGT_REQUIRE(((uintptr_t)dBias & 15) == 0 && (dbias_dtype == MOBGT_F32 || layer_stride % 8 == 0), MOBGT_ERR_BAD_SHAPE,
@@ -1183,7 +1185,8 @@ extern "C" int32_t mobgt_bias_direct_fwd(const int32_t *n, const int64_t *sq_off
     MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && feat && R && Ppos && E && tvd && out, MOBGT_ERR_NULL,
                   "mobgt_bias_direct_fwd: null pointer");
     MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_fwd: num_bins=%d", num_bins);
-    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_fwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE(T >= 2 && T <= MOBGT_MAX_MODEL_NODES + 1 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_direct_fwd: T=%d Tp=%d (T <= 1025: graphs of at most 1024 nodes)", T, Tp);
     MOBGT_REQUIRE(out_dtype == MOBGT_F32 || out_dtype == MOBGT_BF16, MOBGT_ERR_BAD_DTYPE, "mobgt_bias_direct_fwd: dtype");
     if (B <= 0) return MOBGT_OK;
     const K2Common c{n, sq_off, rel_pos, poi_pos, nullptr, B, T, Tp, 0, rel_pos_max, 0};
@@ -1261,7 +1264,8 @@ extern "C" int32_t mobgt_bias_direct_bwd(const int32_t *n, const int64_t *sq_off
     MOBGT_REQUIRE(n && sq_off && rel_pos && poi_pos && feat && dBias && workspace && dR && dPpos && dE && dtvd, MOBGT_ERR_NULL,
                   "mobgt_bias_direct_bwd: null pointer");
     MOBGT_REQUIRE(num_bins >= 1 && num_bins <= 1024, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_bwd: num_bins=%d", num_bins);
-    MOBGT_REQUIRE(T >= 2 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE, "mobgt_bias_direct_bwd: T=%d Tp=%d", T, Tp);
+    MOBGT_REQUIRE(T >= 2 && T <= MOBGT_MAX_MODEL_NODES + 1 && Tp >= T && Tp % 8 == 0, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_bias_direct_bwd: T=%d Tp=%d (T <= 1025: graphs of at most 1024 nodes)", T, Tp);
     MOBGT_REQUIRE((dbias_dtype == MOBGT_F32 && n_layers == 1) || (dbias_dtype == MOBGT_BF16 && n_layers >= 1 && n_layers <= 64),
                   MOBGT_ERR_BAD_DTYPE, "mobgt_bias_direct_bwd: dbias dtype %d with %d layer planes", dbias_dtype, n_layers);
     MOBGT_REQUIRE(((uintptr_t)dBias & 15) == 0 && (dbias_dtype == MOBGT_F32 || layer_stride % 8 == 0), MOBGT_ERR_BAD_SHAPE,

@@ -50,6 +50,7 @@ struct AttnBwdParams {
     const __nv_bfloat16 *bias;        // [B,H,T,Tp]
     int small_t;                      // graphs of at most this many tokens belong to the SIMT kernel (k3_attn_small.cu); 0: none
     const int32_t *order;             // [B] graph ids in launch order (descending size) or NULL
+    int large_t;                      // graphs of more tokens belong to the SIMT kernels of k3_attn_large.cu
 };
 
 // the d bf16 of row `row` of a [chunk][row][8] operand box -> fp32
@@ -139,7 +140,7 @@ k3_attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     const int g = p.order ? p.order[gi] : gi;       // largest graphs first: the CTAs that return at once are dispatched behind them
     const int t0 = p.tok_off[g];
     const int Tg = p.tok_off[g + 1] - t0;
-    if (Tg <= p.small_t) return;                           // the whole CTA: nothing has been set up yet
+    if (Tg <= p.small_t || Tg > p.large_t) return;         // the whole CTA: nothing has been set up yet
     const bool fold = Tg > kTile && (Tg % kTile) == 1;     // single-token tail handled by SIMT (see above)
     const int NB = fold ? Tg / kTile : ceil_div(Tg, kTile);
     const int sp = Tg - 1;                                 // the tail token (fold only)
@@ -1084,8 +1085,8 @@ int32_t attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
                   "mobgt_attn_bwd: null pointer");
     MOBGT_REQUIRE(qkv_row_stride % 8 == 0 && dqkv_row_stride % 8 == 0 && Tp % 8 == 0 && Tp >= T, MOBGT_ERR_BAD_SHAPE,
                   "mobgt_attn_bwd: strides / Tp must be multiples of 8");
-    MOBGT_REQUIRE(t_max_host >= 1 && t_max_host <= T && T <= MOBGT_MAX_NODES + 1, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_attn_bwd: t_max=%d T=%d", t_max_host, T);
+    MOBGT_REQUIRE(t_max_host >= 1 && t_max_host <= T && T <= MOBGT_MAX_MODEL_NODES + 1, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_attn_bwd: t_max=%d T=%d (T <= 1025: graphs of at most 1024 nodes)", t_max_host, T);
     if (B == 0 || ntok == 0) return MOBGT_OK;
     MOBGT_REQUIRE(drop_p >= 0.f && drop_p < 1.f, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_bwd: drop_p=%f must be in [0, 1)", drop_p);
     // the same device-side split by graph size as the forward (k3_attn_small.cu)
@@ -1122,6 +1123,7 @@ int32_t attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
         }
     }
     auto run_tensor_core = [&]() -> int32_t {
+    if (t_min_host > kLargeT) return MOBGT_OK;    // every graph is a large one
     CUtensorMap tmQ, tmK, tmV, tmdO, tmB;
     const void *ptrs[4] = {q, k, v, dout};
     CUtensorMap *maps[4] = {&tmQ, &tmK, &tmV, &tmdO};
@@ -1147,8 +1149,10 @@ int32_t attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
         int32_t rc = encode_tmap_bf16(&tmDS, dbias, 4, dims, str, box, 0);
         if (rc) return rc;
     }
-    // a graph of 128 m + 1 tokens keeps only its m full boxes in shared memory (single-token tail), and T <= 513
-    const int max_boxes = t_max_host > kTile && t_max_host % kTile == 1 ? t_max_host / kTile : ceil_div(t_max_host, kTile);
+    // a graph of 128 m + 1 tokens keeps only its m full boxes in shared memory (single-token tail); this kernel's graphs have
+    // at most kLargeT = 513 tokens
+    const int t_tc = min(t_max_host, kLargeT);
+    const int max_boxes = t_tc > kTile && t_tc % kTile == 1 ? t_tc / kTile : ceil_div(t_tc, kTile);
     const size_t smem_base = 2 * kPBytes + 4 * kBoxBytes + (size_t)2 * max_boxes * kBoxBytes + 1024;
     const int bias_bufs = (smem_base + 2 * kBiasTileBytes <= 204 * 1024) ? 2 : 1;    // + 20 KB of static shared memory
     const size_t smem = smem_base + (size_t)bias_bufs * kBiasTileBytes;
@@ -1179,7 +1183,7 @@ int32_t attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
                     static_cast<const __nv_bfloat16 *>(v),
                     qkv_row_stride,
                     static_cast<const __nv_bfloat16 *>(bias),
-                    any_small ? kSmallT : 0, graph_order};
+                    any_small ? kSmallT : 0, graph_order, kLargeT};
     if (accumulate == 2 && t_max_host <= kTile + 1) {   // every graph fits one (query tile, key block): two CTAs per SM
         const size_t smem1 = (size_t)kBiasTileBytes + kPBytes + 4 * kBoxBytes + 1024;
         auto kern1 = drop.th16 ? k3_attn_bwd1_kernel<kAttD, true> : k3_attn_bwd1_kernel<kAttD, false>;
@@ -1193,7 +1197,15 @@ int32_t attn_bwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
     MOBGT_LAUNCH_OK("k3_attn_bwd_kernel");
     return MOBGT_OK;
     };
-    const int32_t rc = run_tensor_core();
+    int32_t rc = run_tensor_core();
+    if (rc == MOBGT_OK && t_max_host > kLargeT) {   // graphs of 514 .. 1025 tokens
+        LargeAttnParams lp{};
+        lp.tok_off = tok_off; lp.order = graph_order; lp.q = q; lp.k = k; lp.v = v; lp.qkv_stride = qkv_row_stride; lp.bias = bias;
+        lp.H = H; lp.T = T; lp.Tp = Tp; lp.scale = scale; lp.t_lo = kLargeT; lp.drop = make_attn_drop(drop_p, seed, seed_dev);
+        lp.lse = const_cast<float *>(lse); lp.o = o; lp.dout = dout; lp.dq = dq; lp.dk = dk; lp.dv = dv;
+        lp.dqkv_stride = dqkv_row_stride; lp.dbias = dbias; lp.accumulate = accumulate;
+        rc = launch_large_attn_bwd<__nv_bfloat16, kAttD>(lp, B, t_max_host, static_cast<cudaStream_t>(stream));
+    }
     if (forked) cudaStreamWaitEvent(static_cast<cudaStream_t>(stream), fj.join, 0);   // join on every path
     return rc;
 }

@@ -1,5 +1,5 @@
 // K3 (fp32 mode) — the biased attention of model_fqandtoyo.py:1693-1706 and its backward with fp32 operands, fp32 bias and
-// fp32 results, for graphs of any size up to 513 tokens.
+// fp32 results, for graphs of any size up to 1 025 tokens.
 //
 // Why: the contract of this path is "within 1e-5 relative in fp32 mode, 2e-2 in bf16 mode" against the reference's own
 // arithmetic.  The tensor-core kernels (k3_attn_fwd.cu / k3_attn_bwd.cu) round Q, K, V, the bias and the probabilities to bf16
@@ -12,16 +12,19 @@
 // (25 for head dim 24, 17 for 16: lanes read different rows, conflict-free); a warp owns one query row (forward and the dQ / dS
 // pass) or one key column (the dK / dV pass) at a time, its lanes stride over the other index, and the d-wide partial sums are
 // merged by shuffles in a fixed
-// order — no atomics, bitwise reproducible.  Scores and probabilities are recomputed, never stored.  The dropout mask is the
+// order — no atomics, bitwise reproducible.  The backward stages Q, K, V and dO together (4 T (d + 1) floats), which fits up to
+// T = 513; a batch with a larger graph runs the backward as two kernels that stage half each (k3_attn_large.cu, float
+// instantiation: the same expressions in the same order, so the same bits).  Scores and probabilities are recomputed, never stored.  The dropout mask is the
 // tensor-core path's (common.cuh attn_drop_*: same seed, same mask).
 #include "common.cuh"
+#include "k3_small.cuh"
 
 namespace mobgt {
 
 namespace {
 constexpr int kWarps = 8;
 constexpr int kThreadsF = kWarps * 32;
-constexpr int kMaxT = 513;
+constexpr int kMaxT = MOBGT_MAX_MODEL_NODES + 1;   // forward: 2 T (d + 1) floats of shared memory, 205 KB at T = 1025
 
 struct F32AttnParams {
     const int32_t *tok_off;
@@ -228,7 +231,7 @@ int32_t check_common(const void *q, const void *k, const void *v, const void *bi
     MOBGT_REQUIRE(B >= 0 && H > 0 && ntok >= 0 && T > 0 && Tp >= T, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_f32: bad sizes B=%d H=%d ntok=%d T=%d Tp=%d", B,
                   H, ntok, T, Tp);
     MOBGT_REQUIRE(t_max_host >= 1 && t_max_host <= T && T <= kMaxT, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_attn_f32: t_max_host=%d must be in [1, T=%d] and T <= %d (graphs of at most 512 nodes)", t_max_host, T, kMaxT);
+                  "mobgt_attn_f32: t_max_host=%d must be in [1, T=%d] and T <= %d (graphs of at most 1024 nodes)", t_max_host, T, kMaxT);
     MOBGT_REQUIRE(drop_p >= 0.f && drop_p < 1.f, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_f32: drop_p=%f outside [0, 1)", (double)drop_p);
     return MOBGT_OK;
 }
@@ -277,6 +280,15 @@ extern "C" int32_t mobgt_attn_f32_bwd_hd(const float *q, const float *k, const f
     p.H = H; p.T = T; p.Tp = Tp; p.scale = scale; p.drop = make_attn_drop(drop_p, seed, seed_dev);
     p.lse = const_cast<float *>(lse); p.o = o; p.dout = dout; p.dq = dq; p.dk = dk; p.dv = dv; p.dqkv_stride = dqkv_row_stride;
     p.dbias = dbias; p.accumulate = mode;
+    if (t_max_host > kLargeT) {
+        LargeAttnParams lp{};
+        lp.tok_off = tok_off; lp.q = q; lp.k = k; lp.v = v; lp.qkv_stride = qkv_row_stride; lp.bias = bias;
+        lp.H = H; lp.T = T; lp.Tp = Tp; lp.scale = scale; lp.t_lo = 0; lp.drop = p.drop;
+        lp.lse = p.lse; lp.o = o; lp.dout = dout; lp.dq = dq; lp.dk = dk; lp.dv = dv; lp.dqkv_stride = dqkv_row_stride;
+        lp.dbias = dbias; lp.accumulate = mode;
+        auto f = head_dim == 16 ? launch_large_attn_bwd<float, 16> : launch_large_attn_bwd<float, 24>;
+        return f(lp, B, t_max_host, static_cast<cudaStream_t>(stream));
+    }
     const size_t smem = ((size_t)4 * t_max_host * (head_dim + 1) + 2 * (size_t)t_max_host) * sizeof(float);   // row pitch d + 1
     auto kern = head_dim == 16 ? k3f_attn_bwd_kernel<16> : k3f_attn_bwd_kernel<24>;
     MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

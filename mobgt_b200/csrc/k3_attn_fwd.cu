@@ -43,6 +43,7 @@ struct AttnFwdParams {
     int small_t;                      // graphs of at most this many tokens belong to the SIMT kernel (k3_attn_small.cu); 0: none
     const int32_t *order;             // [B] graph ids in launch order (descending size) or NULL
     int n_items;                      // B * H work items; CTA b works on items b, b + gridDim.x, ... (persistent CTAs)
+    int large_t;                      // graphs of more tokens belong to the SIMT kernel of k3_attn_large.cu
 };
 
 // the d bf16 of row `row` of a [chunk][row][8] operand box -> fp32
@@ -104,7 +105,7 @@ k3_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             it.g = p.order ? p.order[gi] : gi;      // largest graphs first
             it.t0 = p.tok_off[it.g];
             it.Tg = p.tok_off[it.g + 1] - it.t0;
-            if (it.Tg > p.small_t) break;
+            if (it.Tg > p.small_t && it.Tg <= p.large_t) break;
         }
         return it;
     };
@@ -528,8 +529,8 @@ int32_t attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
     MOBGT_REQUIRE(H >= 1 && B >= 0 && ntok >= 0, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_fwd: B=%d H=%d ntok=%d", B, H, ntok);
     MOBGT_REQUIRE(qkv_row_stride % 8 == 0 && Tp % 8 == 0 && Tp >= T, MOBGT_ERR_BAD_SHAPE,
                   "mobgt_attn_fwd: row stride %lld and Tp=%d must be multiples of 8", (long long)qkv_row_stride, Tp);
-    MOBGT_REQUIRE(t_max_host >= 1 && t_max_host <= T && T <= MOBGT_MAX_NODES + 1, MOBGT_ERR_BAD_SHAPE,
-                  "mobgt_attn_fwd: t_max=%d T=%d", t_max_host, T);
+    MOBGT_REQUIRE(t_max_host >= 1 && t_max_host <= T && T <= MOBGT_MAX_MODEL_NODES + 1, MOBGT_ERR_BAD_SHAPE,
+                  "mobgt_attn_fwd: t_max=%d T=%d (T <= 1025: graphs of at most 1024 nodes)", t_max_host, T);
     MOBGT_REQUIRE(drop_p >= 0.f && drop_p < 1.f, MOBGT_ERR_BAD_SHAPE, "mobgt_attn_fwd: drop_p=%f must be in [0, 1)", drop_p);
     if (B == 0 || ntok == 0) return MOBGT_OK;
     // graphs of <= kSmallT tokens: SIMT kernel; the others: tensor cores.  Both kernels select their graphs on the device, so
@@ -563,6 +564,7 @@ int32_t attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
         }
     }
     auto run_tensor_core = [&]() -> int32_t {
+    if (t_min_host > kLargeT) return MOBGT_OK;    // every graph is a large one
     CUtensorMap tmQ, tmK, tmV, tmB;
     const void *ptrs[3] = {q, k, v};
     CUtensorMap *maps[3] = {&tmQ, &tmK, &tmV};
@@ -580,14 +582,16 @@ int32_t attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
         int32_t rc = encode_tmap_bf16(&tmB, bias, 3, dims, str, box, 1);
         if (rc) return rc;
     }
-    // a graph of 128 m + 1 tokens keeps only its m full boxes in shared memory (single-token tail), and T <= 513
-    const int max_boxes = t_max_host > kTile && t_max_host % kTile == 1 ? t_max_host / kTile : ceil_div(t_max_host, kTile);
+    // a graph of 128 m + 1 tokens keeps only its m full boxes in shared memory (single-token tail); this kernel's graphs have
+    // at most kLargeT = 513 tokens
+    const int t_tc = min(t_max_host, kLargeT);
+    const int max_boxes = t_tc > kTile && t_tc % kTile == 1 ? t_tc / kTile : ceil_div(t_tc, kTile);
     const size_t smem = (size_t)kBiasTileBytes + kPBytes + kBoxBytes + (size_t)2 * max_boxes * kBoxBytes + 1024;
     AttnFwdParams p{tok_off, static_cast<__nv_bfloat16 *>(out), lse, H, scale, max_boxes, g_timeline_dev,
                     make_attn_drop(drop_p, seed, seed_dev),
                     static_cast<const __nv_bfloat16 *>(q), static_cast<const __nv_bfloat16 *>(k),
                     static_cast<const __nv_bfloat16 *>(v), qkv_row_stride, static_cast<const __nv_bfloat16 *>(bias), T, Tp,
-                    any_small ? kSmallT : 0, graph_order, B * H};
+                    any_small ? kSmallT : 0, graph_order, B * H, kLargeT};
     auto kern = p.drop.th16 ? k3_attn_fwd_kernel<kAttD, true> : k3_attn_fwd_kernel<kAttD, false>;
     MOBGT_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = B * H < 2 * kNumSMs ? B * H : 2 * kNumSMs;     // persistent: two CTAs per SM, each loops over its items
@@ -595,7 +599,14 @@ int32_t attn_fwd(const void *q, const void *k, const void *v, int64_t qkv_row_st
     MOBGT_LAUNCH_OK("k3_attn_fwd_kernel");
     return MOBGT_OK;
     };
-    const int32_t rc = run_tensor_core();
+    int32_t rc = run_tensor_core();
+    if (rc == MOBGT_OK && t_max_host > kLargeT) {   // graphs of 514 .. 1025 tokens
+        LargeAttnParams lp{};
+        lp.tok_off = tok_off; lp.order = graph_order; lp.q = q; lp.k = k; lp.v = v; lp.qkv_stride = qkv_row_stride; lp.bias = bias;
+        lp.H = H; lp.T = T; lp.Tp = Tp; lp.scale = scale; lp.t_lo = kLargeT; lp.drop = make_attn_drop(drop_p, seed, seed_dev);
+        lp.out = out; lp.lse = lse;
+        rc = launch_large_attn_fwd<__nv_bfloat16, kAttD>(lp, B, t_max_host, static_cast<cudaStream_t>(stream));
+    }
     if (forked) cudaStreamWaitEvent(static_cast<cudaStream_t>(stream), fj.join, 0);   // join on every path
     return rc;
 }

@@ -61,4 +61,32 @@ struct SmallAttnParams {
 template <int kD> int32_t launch_small_attn_fwd(const SmallAttnParams &p, int B, cudaStream_t s);
 template <int kD> int32_t launch_small_attn_bwd(const SmallAttnParams &p, int B, cudaStream_t s);
 
+// Graphs of more than kLargeT tokens (up to MOBGT_MAX_MODEL_NODES + 1) are computed by the SIMT kernels of k3_attn_large.cu;
+// the tensor-core kernels skip them on the device and size their shared memory for at most kLargeT tokens.
+constexpr int kLargeT = MOBGT_MAX_NODES + 1;
+
+struct LargeAttnParams {
+    const int32_t *tok_off;
+    const int32_t *order;             // [B] graph ids in launch order or NULL
+    const void *q, *k, *v;            // TE [ntok, qkv_stride]
+    int64_t qkv_stride;
+    const void *bias;                 // TE [B,H,T,Tp]
+    int H, T, Tp;
+    float scale;
+    int t_lo;                         // graphs of more than t_lo tokens belong to these kernels
+    AttnDrop drop;
+    void *out;                        // TE [ntok, H*d]
+    float *lse;                       // [ntok, H]   (backward: input)
+    const void *o, *dout;             // TE [ntok, H*d]
+    void *dq, *dk, *dv;               // TE [ntok, dqkv_stride]
+    int64_t dqkv_stride;
+    void *dbias;                      // f32 (accumulate 0 / 1) or bf16 (accumulate 2) [B,H,T,Tp]
+    int accumulate;
+};
+
+// TE: __nv_bfloat16 (forward and backward) or float (backward); kD: 16 or 24; t_max: the largest token count of the batch.
+// Explicitly instantiated in k3_attn_large.cu.
+template <typename TE, int kD> int32_t launch_large_attn_fwd(const LargeAttnParams &p, int B, int t_max, cudaStream_t s);
+template <typename TE, int kD> int32_t launch_large_attn_bwd(const LargeAttnParams &p, int B, int t_max, cudaStream_t s);
+
 }  // namespace mobgt

@@ -53,6 +53,9 @@ def build_parser():
     d.add_argument("--seed", type=int, default=1)
     d.add_argument("--multi_hop_max_dist", type=int, default=5)
     d.add_argument("--rel_pos_max", type=int, default=1024)
+    d.add_argument("--max_node", type=int, default=512,
+                   help="largest trajectory graph (nodes) a batch takes; larger ones are left out of every epoch (collator.py:313). "
+                        "Up to 512 by default; 513..1024 turns on the collator's large_graphs mode (the reference: 30000, data.py)")
     s = parser.add_argument_group("synthetic data (stand-in for ../dataset/<name>) and run options of this implementation")
     s.add_argument("--synthetic", type=str, default=None, help="c1|c2|c4|tiny (default: by dataset_name)")
     s.add_argument("--train_graphs", type=int, default=2048)
@@ -72,7 +75,10 @@ def build_parser():
 
 
 def parse_args(argv=None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if not 1 <= args.max_node <= 1024:
+        parser.error(f"--max_node {args.max_node}: the model's kernels take graphs of 1 to 1024 nodes")
     args.max_steps = args.tot_updates + 1                               # entry.py:57
     return args
 
@@ -135,8 +141,9 @@ def cli_main(argv=None):
     def loader(items, shuffle, epoch, pad):
         # one batch ahead: host packing in --num_workers processes, H2D + K1 + poi_pos + sort plans on a side stream; training
         # batches are padded to size buckets so that the captured CUDA graphs replay across batches of different graphs
-        return collator.PackedLoader(item_batches(items, shuffle, epoch, pad), num_workers=args.num_workers, max_node=512,
-                                     bucket=shuffle and not args.no_cuda_graph and args.precision == 16, **ckw)
+        return collator.PackedLoader(item_batches(items, shuffle, epoch, pad), num_workers=args.num_workers, max_node=args.max_node,
+                                     bucket=shuffle and not args.no_cuda_graph and args.precision == 16,
+                                     large_graphs=args.max_node > _C.MAX_NODES, **ckw)
 
     model = Graphormer(
         n_layers=args.n_layers, num_heads=args.num_heads, hidden_dim=args.hidden_dim,
@@ -181,11 +188,13 @@ def cli_main(argv=None):
         t0 = time.time()
         limit = args.max_steps if args.limit_train_steps is None else min(args.max_steps, tr.step_count + args.limit_train_steps)
         loss = None
+        result["train_graphs"] = 0                                      # graphs trained on, summed over the epochs run
         for epoch in range(epoch0, args.max_epochs):
             ld = loader(train, True, epoch, pad=True)
             b = ld.current()
             while b is not None and tr.step_count < limit:
                 loss = tr.train_step(b)
+                result["train_graphs"] += int(b.B)
                 ld.advance()                                            # collate the next batch under this step's kernels
                 b = ld.current()
                 if rank == 0 and tr.step_count % max(1, args.progress_bar_refresh_rate) == 0:

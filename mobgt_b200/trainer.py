@@ -25,7 +25,7 @@ import sys
 import torch
 import torch.distributed as dist
 
-from . import graphs, ops, parallel
+from . import _C, graphs, ops, parallel
 
 
 def _signature(batch):
@@ -115,7 +115,9 @@ class Trainer:
 
     # ---------------------------------------------------------------------------------------- one step
     def _graph_for(self, batch):
-        if not self.use_graph:
+        # a batch holding a graph of more than 512 nodes (collator large_graphs mode, at most one such graph in a few thousand)
+        # runs eagerly: its bias and dS planes are ~40x those of an ordinary batch and would stay reserved in the graph pool
+        if not self.use_graph or int(batch.N) > _C.MAX_NODES:
             return None
         sig = _signature(batch)
         g = self._graphs.get(sig)
